@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the UNMODIFIED reference on the host cores
+    python bench.py ... --dump-outputs DIR                   # also save what the last timed step returned, to compare builds
 
 A "step" is one forward pass over one batch of synthetic noisy two-speaker mixtures
 (BASELINE.json configs[1]: config_with_vad.json, 256 x 4 s per GPU, filter_signals_by_smo_vad).
@@ -297,6 +298,29 @@ def pcie_ceiling(torch, dev, h2d_bytes, d2h_bytes, reps=10):
     return dt
 
 
+DUMP_BYTES = 60_000_000   # array data of --dump-outputs: with the .npy headers, under 64 MB in all
+
+
+def dump_outputs(out_dir, returned):
+    """Write the tensors a forward returned as float32 ``out_dir/<name>.npy`` (complex ones with a trailing (real, imag)
+    axis). If together they exceed DUMP_BYTES, every array keeps the same batch rows: a sample drawn with a fixed seed,
+    so that two runs with the same arguments write the same rows."""
+    import numpy as np
+    import torch
+    arrays = {k: torch.view_as_real(v) if v.is_complex() else v for k, v in returned.items() if torch.is_tensor(v)}
+    B = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(v[0].numel() * 4 for v in arrays.values())
+    rows = np.arange(B)
+    if B * row_bytes > DUMP_BYTES:
+        if row_bytes > DUMP_BYTES:
+            raise SystemExit(f"--dump-outputs: one batch row of the outputs alone is {row_bytes} bytes")
+        rows = np.sort(np.random.default_rng(0).choice(B, DUMP_BYTES // row_bytes, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v[torch.from_numpy(rows).to(v.device)].float().cpu().numpy())
+    print(f"bench.py: wrote {', '.join(arrays)} of batch rows {rows.tolist()} to {out_dir}", file=sys.stderr, flush=True)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -313,7 +337,14 @@ def main():
     ap.add_argument("--lean", action="store_true", help="skip the optional exports (est/mask/spectrum/logits)")
     ap.add_argument("--online-streams", type=int, default=1024, help="concurrent streams of the online leg (0 = skip)")
     ap.add_argument("--online-hops", type=int, default=12)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed forward returned (rank 0) as DIR/<name>.npy, "
+                         "float32; a fixed, seeded sample of the batch rows when all of it would exceed 64 MB")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's outputs; it cannot be combined with --impl reference")
 
     # NCCL logs (its version banner included, which WARN and VERSION both print) go to stdout by default and would
     # precede the JSON line: send them to stderr
@@ -375,14 +406,19 @@ def main():
     sampler = ClockSampler(local_rank) if rank == 0 else None
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
+    last = None
     for _ in range(a.steps):
-        step()
+        last = None       # release the previous step's outputs before the next forward allocates its own
+        last = step()
     e1.record()
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
     t_dev = gather_max_time(e0.elapsed_time(e1) * 1e-3)
     launches = model.last_launch_count * a.steps
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, dict(zip(("out", "output_vad", "estimated_stfts"), last)))
+    del last
 
     # ---- per-kernel-class timing (separate pass; events inside forward on the same stream)
     model.set_profile(True)

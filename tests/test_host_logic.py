@@ -146,27 +146,23 @@ def test_two_rank_gloo_sharding_and_metric_gather(tmp_path):
 
 
 def test_pit_helpers_equal_reference_functions():
-    """The re-written pairwise-loss / exhaustive-permutation helpers against the reference's own (imported through
-    oracle/ref_loader.py), 2 and 3 sources, including exact ties (-> identity, torch.min's first index)."""
-    from oracle import ref_loader
+    """The re-written pairwise-loss / exhaustive-permutation helpers against the reference's, 2 and 3 sources, including
+    exact ties (-> identity, torch.min's first index). The expected values are stored in tests/golden/reference_helpers.npz:
+    computed by the reference's own functions where it can be imported, otherwise by tests/golden/make_helper_golden.py's
+    restatement of their code, which shares nothing with septfa_b200 (``meta["source"]`` says which)."""
+    from conftest import load_golden
     from septfa_b200.pit import PITLossWrapper
-    ns = ref_loader.load()
-    RP = ns.pit_wrapper.PITLossWrapper
-    g = torch.Generator().manual_seed(5)
+    g, _ = load_golden("reference_helpers")
     for n_src in (2, 3):
-        pw = torch.rand(64, n_src, n_src, generator=g)
-        pw[::7] = 0.25                                     # all permutations tie
-        pw[1::9, 0, 0] = pw[1::9, 1, 0]                    # partial ties
-        pw[1::9, 1, 1] = pw[1::9, 0, 1]
+        pw = torch.from_numpy(g[f"pit_pw{n_src}"])       # rows of all-equal entries and rows with partial ties
         loss, idx = PITLossWrapper.find_best_perm_factorial(pw)
-        ref_loss, ref_idx = RP.find_best_perm_factorial(pw)
-        assert torch.equal(idx, ref_idx) and torch.allclose(loss, ref_loss, atol=1e-7)
-    est, tgt = torch.randn(3, 2, 500, generator=g), torch.randn(3, 2, 500, generator=g)
+        assert np.array_equal(idx.numpy(), g[f"pit_idx{n_src}"]) and np.allclose(loss.numpy(), g[f"pit_loss{n_src}"],
+                                                                                 rtol=0, atol=1e-7)
+    est, tgt = torch.from_numpy(g["pit_est"]), torch.from_numpy(g["pit_tgt"])
     l1 = torch.nn.L1Loss()
-    assert torch.equal(PITLossWrapper.get_pw_losses(l1, est, tgt), RP.get_pw_losses(l1, est, tgt))
-    mine, theirs = PITLossWrapper(l1, pit_from="pw_pt"), RP(l1, pit_from="pw_pt")
-    a, b = mine(est, tgt, return_incides=True), theirs(est, tgt, return_incides=True)
-    assert torch.equal(a[1], b[1]) and abs(a[0].item() - b[0].item()) < 1e-7
+    assert np.array_equal(PITLossWrapper.get_pw_losses(l1, est, tgt).numpy(), g["pit_pw_l1"])
+    loss, idx = PITLossWrapper(l1, pit_from="pw_pt")(est, tgt, return_incides=True)
+    assert np.array_equal(idx.numpy(), g["pit_wrapper_idx"]) and abs(loss.item() - g["pit_wrapper_loss"].item()) < 1e-7
 
 
 def test_reference_bytecode_build_matches_source(tmp_path):
