@@ -179,7 +179,7 @@ int septfa_graph_launch(septfa_graph* g, void* stream);
 int septfa_graph_num_nodes(const septfa_graph* g);
 void septfa_graph_destroy(septfa_graph* g);
 
-/* Number of GPU kernels launched by the last forward / online step on this handle. */
+/* Number of GPU kernels launched by the last forward / online step / live push on this handle (0 after a refused push). */
 int septfa_last_launch_count(const septfa_handle* h);
 
 /* Per-kernel-class device timing. With option "profile" = 1, forward records CUDA events on its
@@ -210,6 +210,39 @@ size_t septfa_online_workspace_bytes(const septfa_online* st);
 int septfa_online_step(septfa_online* st, const float* win, const septfa_infer_kw* kw, float* emitted,
                        int32_t* perm, void* workspace, size_t workspace_bytes, void* stream);
 int septfa_online_hops_done(const septfa_online* st);
+
+/* ---- live streaming sessions: OnlineSaving for streams that start and end independently ---------------------------
+ * A session has `capacity` slots (1 .. 32767); each slot hosts one stream at a time. A stream is a sequence of pushes
+ * of exactly one hop each (SEPTFA_LIVE_HOP float32 samples, already normalised by the caller). Push k (0-based) of a
+ * stream runs the forward on the 3 s window concat(zeros for k < 2, hops k-2 .. k) - the stream left-padded with 2 s of
+ * zeros, model/online_class_known_targets.py:92-93 - and returns
+ *   out  [2, 16000]           separated audio for the stream's samples [16000 k, 16000 (k + 1)): the window's last
+ *                             second, speakers permuted;
+ *   perm [2] (int32)          the permutation: the L1 PIT of online_class_unknown_targets.py:84-94 between the window and
+ *                             the last min(16000 k, 32000) emitted samples (ties -> identity); at k = 0 the window's
+ *                             [1 s, 2 s) is compared with its own [2 s, 3 s), like the reference's first window;
+ *   vad  [2, 63] (nullable)   out_vad of the window (probabilities, or the smoothed decisions with
+ *                             kw->return_smoothed_vad), frames 125 .. 187, speakers in the emitted order. Frame j is
+ *                             centred on stream sample 16000 k + 256 j; since 16000 = 62.5 x 256, the frame grids of
+ *                             consecutive hops are offset by half a frame. Needs a model with a VAD head.
+ * So the concatenated out of a stream of N pushes equals OnlineSaving.calc_online on that stream alone, left-padded with
+ * 32000 zeros. septfa_live_release ends the streams in the listed slots; the next push into such a slot starts a new
+ * stream at k = 0 and reads nothing of the old one.
+ * Slot lists are host arrays of n distinct slots, 1 <= n <= capacity; a bad list (slot out of range, a slot twice, n out
+ * of range) is refused with SEPTFA_E_INVALID before anything is launched. A push that returns an error leaves every slot
+ * unchanged. Per slot the session keeps on the device a hop counter, the last two input hops and the last two emitted
+ * hops (~384 KB per slot). Pushes and releases are stream-ordered and do not synchronise the host; issue all calls of a
+ * session on one stream. hops: device [n, 16000]; out: device [n, 2, 16000]; out_vad: device [n, 2, 63];
+ * perm: device int32 [n, 2]; the workspace is sized by septfa_live_workspace_bytes for pushes of up to n slots. */
+#define SEPTFA_LIVE_HOP 16000
+#define SEPTFA_LIVE_FRAMES_PER_HOP 63
+typedef struct septfa_live septfa_live;
+int septfa_live_create(septfa_handle* h, int capacity, septfa_live** out);
+void septfa_live_destroy(septfa_live* lv);
+size_t septfa_live_workspace_bytes(const septfa_live* lv, int n);
+int septfa_live_release(septfa_live* lv, const int32_t* slots_host, int n, void* stream);
+int septfa_live_push(septfa_live* lv, const int32_t* slots_host, int n, const float* hops, const septfa_infer_kw* kw,
+                     float* out, float* out_vad, int32_t* perm, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Stand-alone PIT for 2 sources (model/pit_wrapper.py:149-177,261-312): a[S,2,n], b[S,2,n] ->
  * perm[S,2] (int32), decided per stream; pw_sums (nullable, device double [S,4]) receives the

@@ -7,11 +7,11 @@ utilities (``synth``) work without torch or the CUDA library.
 """
 import importlib as _importlib
 
-__all__ = ["SeparationModel", "OnlineSaving", "OnlineSavingKnownTargets", "PITLossWrapper",
+__all__ = ["SeparationModel", "OnlineSaving", "OnlineSavingKnownTargets", "LiveSession", "PITLossWrapper",
            "reorder_source_mse", "calc_sisdr", "synth"]
 
 _LAZY = {
-    "SeparationModel": "model", "OnlineSaving": "online", "OnlineSavingKnownTargets": "online",
+    "SeparationModel": "model", "OnlineSaving": "online", "OnlineSavingKnownTargets": "online", "LiveSession": "live",
     "PITLossWrapper": "pit", "reorder_source_mse": "pit", "calc_sisdr": "pit",
 }
 
@@ -19,6 +19,6 @@ _LAZY = {
 def __getattr__(name):
     if name in _LAZY:
         return getattr(_importlib.import_module(f"{__name__}.{_LAZY[name]}"), name)
-    if name in ("synth", "model", "online", "pit", "lib", "shard", "inference", "evaluate"):
+    if name in ("synth", "model", "online", "live", "pit", "lib", "shard", "inference", "evaluate"):
         return _importlib.import_module(f"{__name__}.{name}")
     raise AttributeError(name)

@@ -114,6 +114,14 @@ struct septfa_online {
   double* acc = nullptr;
 };
 
+struct septfa_live {
+  septfa_handle* h = nullptr;
+  int capacity = 0;
+  int32_t* hops_done = nullptr;   // [capacity] hops pushed by the slot's current stream (0: no history is read)
+  float* in_ring = nullptr;       // [capacity][2][16000] the last two input hops, hop k at position k & 1
+  float* tail_ring = nullptr;     // [capacity][2][2][16000] the last two emitted hops (both speakers), the same way
+};
+
 namespace {
 
 constexpr int kFs = 16000, kWinLen = 48000, kHopLen = 16000, kTailCap = 32000;
@@ -1360,6 +1368,136 @@ int septfa_online_step(septfa_online* o, const float* win, const septfa_infer_kw
   o->cur ^= 1;
   o->tail_len = std::min(o->tail_len + kHopLen, kTailCap);
   o->hops += 1;
+  h->last_launches = launches + ctx().launches;
+  CUDA_TRY(h, cudaGetLastError());
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------ live sessions
+}  // extern "C"
+
+namespace {
+
+struct LiveWorkspace {
+  int32_t* slots;   // [n] device copy of the push's slot list
+  float* win;       // [n, 48000]
+  float* pred;      // [n, 2, 48000]
+  float* vad;       // [n, 2, 188]
+  void* fws;        // the forward's workspace
+  size_t fws_bytes;
+  size_t total;
+};
+
+LiveWorkspace live_carve(const septfa_handle* h, uintptr_t base, int n) {
+  auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+  LiveWorkspace w{};
+  size_t off = 0;
+  w.slots = reinterpret_cast<int32_t*>(base + off); off += al((size_t)n * sizeof(int32_t));
+  w.win = reinterpret_cast<float*>(base + off);     off += al((size_t)n * kWinLen * sizeof(float));
+  w.pred = reinterpret_cast<float*>(base + off);    off += al((size_t)n * 2 * kWinLen * sizeof(float));
+  w.vad = reinterpret_cast<float*>(base + off);     off += al((size_t)n * 2 * septfa_num_frames(kWinLen) * sizeof(float));
+  w.fws = reinterpret_cast<void*>(base + off);
+  w.fws_bytes = septfa_workspace_bytes(h, n, kWinLen);
+  w.total = off + w.fws_bytes;
+  return w;
+}
+
+// A slot list comes from the host: it is checked in full before anything is launched, since a bad entry would index the
+// per-slot state out of bounds on the device and a duplicate would make two CTAs race on one slot.
+int check_live_slots(septfa_live* lv, const int32_t* slots, int n) {
+  septfa_handle* h = lv->h;
+  if (!slots) return fail(h, SEPTFA_E_INVALID, "null slot list");
+  if (n < 1 || n > lv->capacity)
+    return fail(h, SEPTFA_E_INVALID, "n = " + std::to_string(n) + ": a slot list holds 1 .. capacity (" +
+                                         std::to_string(lv->capacity) + ") slots");
+  std::vector<uint8_t> seen(lv->capacity, 0);
+  for (int i = 0; i < n; ++i) {
+    const int32_t s = slots[i];
+    if (s < 0 || s >= lv->capacity)
+      return fail(h, SEPTFA_E_INVALID, "slot " + std::to_string(s) + " (entry " + std::to_string(i) + ") out of range 0 .. " +
+                                           std::to_string(lv->capacity - 1));
+    if (seen[s]) return fail(h, SEPTFA_E_INVALID, "slot " + std::to_string(s) + " listed twice (entry " + std::to_string(i) + ")");
+    seen[s] = 1;
+  }
+  return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int septfa_live_create(septfa_handle* h, int capacity, septfa_live** out) {
+  if (!h || !out || capacity < 1 || capacity > 32767)
+    return fail(h, SEPTFA_E_INVALID, "bad arguments (1 <= capacity <= 32767 slots per live session)");
+  *out = nullptr;
+  if (!h->committed) return fail(h, SEPTFA_E_STATE, "weights not committed");
+  CUDA_TRY(h, cudaSetDevice(h->device));
+  auto* lv = new septfa_live();
+  lv->h = h;
+  lv->capacity = capacity;
+  const size_t hop_b = (size_t)kHopLen * sizeof(float);
+  if (cudaMalloc(reinterpret_cast<void**>(&lv->hops_done), (size_t)capacity * sizeof(int32_t)) != cudaSuccess ||
+      cudaMalloc(reinterpret_cast<void**>(&lv->in_ring), (size_t)capacity * 2 * hop_b) != cudaSuccess ||
+      cudaMalloc(reinterpret_cast<void**>(&lv->tail_ring), (size_t)capacity * 4 * hop_b) != cudaSuccess ||
+      cudaMemset(lv->hops_done, 0, (size_t)capacity * sizeof(int32_t)) != cudaSuccess) {
+    cudaFree(lv->hops_done); cudaFree(lv->in_ring); cudaFree(lv->tail_ring);
+    delete lv;
+    return fail(h, SEPTFA_E_CUDA, "live session allocation failed");
+  }
+  *out = lv;
+  return 0;
+}
+
+void septfa_live_destroy(septfa_live* lv) {
+  if (!lv) return;
+  cudaSetDevice(lv->h->device);
+  cudaFree(lv->hops_done); cudaFree(lv->in_ring); cudaFree(lv->tail_ring);
+  delete lv;
+}
+
+size_t septfa_live_workspace_bytes(const septfa_live* lv, int n) {
+  if (!lv || n < 1 || n > lv->capacity) return 0;
+  return live_carve(lv->h, 0, n).total + 256;
+}
+
+int septfa_live_release(septfa_live* lv, const int32_t* slots_host, int n, void* stream) {
+  if (!lv) return SEPTFA_E_INVALID;
+  septfa_handle* h = lv->h;
+  if (int rc = check_live_slots(lv, slots_host, n)) return rc;
+  CUDA_TRY(h, cudaSetDevice(h->device));
+  bind_ctx(&h->lctx);
+  launch_live_release(slots_host, n, lv->hops_done, reinterpret_cast<cudaStream_t>(stream));
+  CUDA_TRY(h, cudaGetLastError());
+  return 0;
+}
+
+int septfa_live_push(septfa_live* lv, const int32_t* slots_host, int n, const float* hops, const septfa_infer_kw* kw,
+                     float* out, float* out_vad, int32_t* perm, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!lv) return SEPTFA_E_INVALID;
+  septfa_handle* h = lv->h;
+  // every check comes before the first launch: a push that fails leaves every slot as it was
+  h->last_launches = 0;
+  if (int rc = check_live_slots(lv, slots_host, n)) return rc;
+  if (!hops || !out || !perm || !workspace) return fail(h, SEPTFA_E_INVALID, "null hops / out / perm / workspace");
+  if (out_vad && !h->cfg.final_vad) return fail(h, SEPTFA_E_INVALID, "out_vad needs a model with a VAD head (final_vad)");
+  if (!h->committed) return fail(h, SEPTFA_E_STATE, "weights not committed");
+  if (workspace_bytes < septfa_live_workspace_bytes(lv, n)) return fail(h, SEPTFA_E_WORKSPACE, "live workspace too small");
+  CUDA_TRY(h, cudaSetDevice(h->device));
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const LiveWorkspace ws = live_carve(h, (reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255, n);
+  CUDA_TRY(h, cudaMemcpyAsync(ws.slots, slots_host, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  bind_ctx(&h->lctx);
+  ctx().launches = 0;
+  launch_live_window(ws.slots, n, lv->hops_done, lv->in_ring, hops, ws.win, st);
+  const int before = ctx().launches;
+  if (int rc = septfa_forward(h, ws.win, n, kWinLen, kw, ws.pred, ws.vad, nullptr, nullptr, nullptr, nullptr, ws.fws,
+                              ws.fws_bytes, st))
+    return rc;
+  const int launches = before + h->last_launches;
+  bind_ctx(&h->lctx);
+  ctx().launches = 0;
+  launch_live_pit_emit(ws.slots, n, lv->hops_done, ws.pred, ws.vad, (int)septfa_num_frames(kWinLen), lv->tail_ring, out,
+                       out_vad, perm, st);
   h->last_launches = launches + ctx().launches;
   CUDA_TRY(h, cudaGetLastError());
   return 0;

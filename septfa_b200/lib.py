@@ -97,6 +97,12 @@ _PROTOS = {
     "septfa_online_step": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(InferKw), C.c_void_p, C.c_void_p, C.c_void_p,
                                      C.c_size_t, C.c_void_p]),
     "septfa_online_hops_done": (C.c_int, [C.c_void_p]),
+    "septfa_live_create": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]),
+    "septfa_live_destroy": (None, [C.c_void_p]),
+    "septfa_live_workspace_bytes": (C.c_size_t, [C.c_void_p, C.c_int]),
+    "septfa_live_release": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    "septfa_live_push": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.POINTER(InferKw), C.c_void_p, C.c_void_p,
+                                   C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "septfa_minmax_normalize": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "septfa_sisdr": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "septfa_pit_l1": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p,

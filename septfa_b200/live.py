@@ -1,0 +1,109 @@
+"""Live streaming sessions: one 1 s hop per stream slot per push, streams that start and end independently, VAD per hop.
+
+``OnlineSaving.calc_online`` drives S streams in lockstep over whole recordings the caller already holds. A
+:class:`LiveSession` serves streams as they arrive: each slot hosts one stream at a time, every push carries one new
+hop for any subset of the slots, and the session keeps each stream's last two input hops and last two emitted hops on
+the device (``septfa_live_*`` in ``include/septfa.h``). Push k of a stream returns the stream's separated samples
+``[16000 k, 16000 (k + 1))``: the concatenated output of a stream of N pushes equals
+``OnlineSaving.calc_online(F.pad(x, (32000, 0)))`` on that stream alone (the windowing of
+``model/online_class_known_targets.py:92-93``, the stitch of ``model/online_class_unknown_targets.py:84-94``).
+"""
+from __future__ import annotations
+
+import ctypes as C
+
+import numpy as np
+import torch
+
+from . import lib as _lib
+
+HOP = 16000
+FRAMES_PER_HOP = 63
+
+
+def check_slots(slots, capacity):
+    """``slots`` as a contiguous int32 array of distinct slots in ``0 .. capacity - 1``, 1 <= len <= capacity;
+    ``ValueError`` otherwise."""
+    a = np.asarray(slots.cpu() if isinstance(slots, torch.Tensor) else slots)
+    if a.ndim != 1 or not (1 <= a.size <= capacity):
+        raise ValueError(f"a slot list is a 1-D list of 1 .. {capacity} slots, got shape {a.shape}")
+    if not np.issubdtype(a.dtype, np.integer):
+        raise ValueError(f"slots must be integers, got {a.dtype}")
+    if a.min() < 0 or a.max() >= capacity:
+        raise ValueError(f"slots must lie in 0 .. {capacity - 1}, got {a.min()} .. {a.max()}")
+    if np.unique(a).size != a.size:
+        raise ValueError("a slot may appear only once per call")
+    return np.ascontiguousarray(a, dtype=np.int32)
+
+
+class LiveSession:
+    """``capacity`` stream slots on one device, for a :class:`~septfa_b200.model.SeparationModel`.
+
+    ``push(slots, hops)`` takes one hop (16000 float32 samples, already normalised) for each listed slot and returns
+    ``(out [n, 2, 16000], vad [n, 2, 63] or None, perm [n, 2] int32)`` on the device, stream-ordered on the current
+    stream. ``vad`` holds frames 125 .. 187 of the window's VAD output (frame j centred on stream sample
+    ``16000 k + 256 j``), speakers in the emitted order; it is None for a model without a VAD head or with
+    ``vad=False``. ``release(slots)`` ends the streams in those slots: the next push into one starts a new stream.
+    ``inference_kw`` is the forward's (gating, smoothed VAD), fixed for the session.
+    """
+
+    def __init__(self, model, capacity, inference_kw=None, device=None):
+        self.model = model
+        self.capacity = int(capacity)
+        if not 1 <= self.capacity <= 32767:
+            raise ValueError("capacity must lie in 1 .. 32767")
+        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        if self.device.type != "cuda":
+            raise RuntimeError("septfa_b200.LiveSession runs on CUDA only (no CPU fallback)")
+        self._kw = _lib.InferKw.from_dict(inference_kw) if (inference_kw and model.final_vad) else None
+        self._lv = C.c_void_p()
+        with torch.cuda.device(self.device):
+            self._h = model._handle(self.device)
+            _lib.check(self._h.ptr, self._h.lib.septfa_live_create(self._h.ptr, self.capacity, C.byref(self._lv)))
+            need = self._h.lib.septfa_live_workspace_bytes(self._lv, self.capacity)
+            self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+        self.last_launch_count = 0
+
+    def _stream(self):
+        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def push(self, slots, hops, vad=True):
+        ids = check_slots(slots, self.capacity)
+        n = ids.size
+        if not (isinstance(hops, torch.Tensor) and hops.is_cuda and hops.dtype == torch.float32):
+            raise ValueError("hops must be a CUDA float32 tensor")
+        if tuple(hops.shape) != (n, HOP):
+            raise ValueError(f"hops must have shape ({n}, {HOP}), got {tuple(hops.shape)}")
+        if hops.device != self.device:
+            raise ValueError(f"hops are on {hops.device}, the session on {self.device}")
+        hops = hops.contiguous()
+        with torch.cuda.device(self.device):
+            h = self.model._handle(self.device)
+            out = torch.empty((n, 2, HOP), dtype=torch.float32, device=self.device)
+            v = torch.empty((n, 2, FRAMES_PER_HOP), dtype=torch.float32, device=self.device) \
+                if (vad and self.model.final_vad) else None
+            perm = torch.empty((n, 2), dtype=torch.int32, device=self.device)
+            rc = h.lib.septfa_live_push(self._lv, ids.ctypes.data_as(C.c_void_p), n, C.c_void_p(hops.data_ptr()),
+                                        C.byref(self._kw) if self._kw is not None else None, C.c_void_p(out.data_ptr()),
+                                        C.c_void_p(v.data_ptr()) if v is not None else None, C.c_void_p(perm.data_ptr()),
+                                        C.c_void_p(self._ws.data_ptr()), self._ws.numel(), self._stream())
+            _lib.check(h.ptr, rc)
+            self.last_launch_count = h.lib.septfa_last_launch_count(h.ptr)
+        return out, v, perm
+
+    def release(self, slots):
+        ids = check_slots(slots, self.capacity)
+        with torch.cuda.device(self.device):
+            _lib.check(self._h.ptr, self._h.lib.septfa_live_release(self._lv, ids.ctypes.data_as(C.c_void_p), ids.size,
+                                                                    self._stream()))
+
+    def close(self):
+        if self._lv:
+            self._h.lib.septfa_live_destroy(self._lv)
+            self._lv = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
