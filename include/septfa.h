@@ -179,7 +179,8 @@ int septfa_graph_launch(septfa_graph* g, void* stream);
 int septfa_graph_num_nodes(const septfa_graph* g);
 void septfa_graph_destroy(septfa_graph* g);
 
-/* Number of GPU kernels launched by the last forward / online step / live push on this handle (0 after a refused push). */
+/* Number of GPU kernels launched by the last forward / online step / live push on this handle (0 after a refused push
+ * or a create refused for its geometry). */
 int septfa_last_launch_count(const septfa_handle* h);
 
 /* Per-kernel-class device timing. With option "profile" = 1, forward records CUDA events on its
@@ -198,12 +199,18 @@ int septfa_last_launch_count(const septfa_handle* h);
 int septfa_profile_read(septfa_handle* h, double* ms, int* launches, int n, int reset);
 
 /* ---- online mode: OnlineSaving.calc_online, one hop for S independent streams -------------
- * State kept on the device per stream: the last <= 2 s of already-emitted (permutation-fixed)
- * signal. Each step takes the current 3 s windows win[S, 48000], runs forward, picks per stream
- * the speaker permutation that minimises the L1 distance between the window's overlap with the
- * emitted signal (PITLossWrapper pw_pt + L1Loss, n_src = 2, ties -> identity), reorders, and
- * emits the last 1 s: emitted[S, 2, 16000], perm[S, 2] (int32). */
+ * An online state has a window of W samples and a hop of H samples (OnlineSaving's max_len and
+ * save_sec times fs); septfa_online_create is septfa_online_create_win with W = 48000, H = 16000.
+ * Accepted: 256 <= H, 2 H <= W <= 160000, W and H multiples of 16 (1 ms); anything else is
+ * refused with SEPTFA_E_INVALID before anything is allocated.
+ * State kept on the device per stream: the last <= W - H samples of already-emitted
+ * (permutation-fixed) signal. Each step takes the current windows win[S, W], runs forward, picks
+ * per stream the speaker permutation that minimises the L1 distance between the window's overlap
+ * with the emitted signal (PITLossWrapper pw_pt + L1Loss, n_src = 2, ties -> identity; at the
+ * first step the window's [W - 2H, W - H) against its own [W - H, W)), reorders, and emits the
+ * last hop: emitted[S, 2, H], perm[S, 2] (int32). */
 int septfa_online_create(septfa_handle* h, int S, septfa_online** out);
+int septfa_online_create_win(septfa_handle* h, int S, int window, int hop, septfa_online** out);
 void septfa_online_destroy(septfa_online* st);
 int septfa_online_reset(septfa_online* st, void* stream);
 size_t septfa_online_workspace_bytes(const septfa_online* st);
@@ -212,33 +219,44 @@ int septfa_online_step(septfa_online* st, const float* win, const septfa_infer_k
 int septfa_online_hops_done(const septfa_online* st);
 
 /* ---- live streaming sessions: OnlineSaving for streams that start and end independently ---------------------------
- * A session has `capacity` slots (1 .. 32767); each slot hosts one stream at a time. A stream is a sequence of pushes
- * of exactly one hop each (SEPTFA_LIVE_HOP float32 samples, already normalised by the caller). Push k (0-based) of a
- * stream runs the forward on the 3 s window concat(zeros for k < 2, hops k-2 .. k) - the stream left-padded with 2 s of
- * zeros, model/online_class_known_targets.py:92-93 - and returns
- *   out  [2, 16000]           separated audio for the stream's samples [16000 k, 16000 (k + 1)): the window's last
- *                             second, speakers permuted;
- *   perm [2] (int32)          the permutation: the L1 PIT of online_class_unknown_targets.py:84-94 between the window and
- *                             the last min(16000 k, 32000) emitted samples (ties -> identity); at k = 0 the window's
- *                             [1 s, 2 s) is compared with its own [2 s, 3 s), like the reference's first window;
- *   vad  [2, 63] (nullable)   out_vad of the window (probabilities, or the smoothed decisions with
- *                             kw->return_smoothed_vad), frames 125 .. 187, speakers in the emitted order. Frame j is
- *                             centred on stream sample 16000 k + 256 j; since 16000 = 62.5 x 256, the frame grids of
- *                             consecutive hops are offset by half a frame. Needs a model with a VAD head.
- * So the concatenated out of a stream of N pushes equals OnlineSaving.calc_online on that stream alone, left-padded with
- * 32000 zeros. septfa_live_release ends the streams in the listed slots; the next push into such a slot starts a new
- * stream at k = 0 and reads nothing of the old one.
+ * A session has `capacity` slots (1 .. 32767); each slot hosts one stream at a time. Every stream of a session has a
+ * window of W samples and a hop of H samples, fixed by septfa_live_create_win (septfa_live_create: W = 48000,
+ * H = SEPTFA_LIVE_HOP = 16000). Accepted: 256 <= H, 2 H <= W <= 160000, W and H multiples of 16 (1 ms); W - H need not
+ * be a multiple of H. Anything else is refused with SEPTFA_E_INVALID before anything is allocated.
+ * A stream is a sequence of pushes of exactly one hop each (H float32 samples, already normalised by the caller). Push
+ * k (0-based) of a stream runs the forward on the window concat(the stream's last W - H samples, zeros before its first
+ * sample; the new hop) - the stream left-padded with W - H zeros, model/online_class_known_targets.py:92-93 - and returns
+ *   out  [2, H]               separated audio for the stream's samples [H k, H (k + 1)): the window's last H samples,
+ *                             speakers permuted;
+ *   perm [2] (int32)          the permutation: the L1 PIT of online_class_unknown_targets.py:84-94 between the window's
+ *                             [W - H - o, W - H) and the last o = min(H k, W - H) emitted samples (ties -> identity);
+ *                             at k = 0 the window's [W - 2H, W - H) is compared with its own [W - H, W), like the
+ *                             reference's first window;
+ *   vad  [2, F] (nullable)    out_vad of the window (probabilities, or the smoothed decisions with
+ *                             kw->return_smoothed_vad), the window frames j0 .. j0 + F - 1 whose centres 256 j lie in
+ *                             [W - H, W): j0 = ceil((W - H) / 256), F = ceil(W / 256) - j0 (septfa_live_vad_frames),
+ *                             speakers in the emitted order. Frame j is centred on stream sample H k - (W - H) + 256 j.
+ *                             When 256 divides H and W - H, F = H / 256 and the frames of consecutive hops tile one
+ *                             grid; otherwise consecutive grids are offset (at the default, 16000 = 62.5 x 256: by half
+ *                             a frame; j0 = 125, F = 63). Needs a model with a VAD head.
+ * So the concatenated out of a stream of N pushes equals OnlineSaving.calc_online (max_len = W / 16000, save_sec =
+ * H / 16000) on that stream alone, left-padded with W - H zeros. septfa_live_release ends the streams in the listed
+ * slots; the next push into such a slot starts a new stream at k = 0 and reads nothing of the old one.
  * Slot lists are host arrays of n distinct slots, 1 <= n <= capacity; a bad list (slot out of range, a slot twice, n out
  * of range) is refused with SEPTFA_E_INVALID before anything is launched. A push that returns an error leaves every slot
- * unchanged. Per slot the session keeps on the device a hop counter, the last two input hops and the last two emitted
- * hops (~384 KB per slot). Pushes and releases are stream-ordered and do not synchronise the host; issue all calls of a
- * session on one stream. hops: device [n, 16000]; out: device [n, 2, 16000]; out_vad: device [n, 2, 63];
- * perm: device int32 [n, 2]; the workspace is sized by septfa_live_workspace_bytes for pushes of up to n slots. */
+ * unchanged. Per slot the session keeps on the device a hop counter, the last W - H input samples and the last W - H
+ * emitted samples of both speakers (12 (W - H) + 4 bytes: ~384 KB at the default). Pushes and releases are
+ * stream-ordered and do not synchronise the host; issue all calls of a session on one stream. hops: device [n, H];
+ * out: device [n, 2, H]; out_vad: device [n, 2, F]; perm: device int32 [n, 2]; the workspace is sized by
+ * septfa_live_workspace_bytes for pushes of up to n slots. */
 #define SEPTFA_LIVE_HOP 16000
 #define SEPTFA_LIVE_FRAMES_PER_HOP 63
 typedef struct septfa_live septfa_live;
 int septfa_live_create(septfa_handle* h, int capacity, septfa_live** out);
+int septfa_live_create_win(septfa_handle* h, int capacity, int window, int hop, septfa_live** out);
 void septfa_live_destroy(septfa_live* lv);
+/* F, the VAD frames per push; *first_frame (nullable) receives j0. */
+int septfa_live_vad_frames(const septfa_live* lv, int* first_frame);
 size_t septfa_live_workspace_bytes(const septfa_live* lv, int n);
 int septfa_live_release(septfa_live* lv, const int32_t* slots_host, int n, void* stream);
 int septfa_live_push(septfa_live* lv, const int32_t* slots_host, int n, const float* hops, const septfa_infer_kw* kw,

@@ -239,14 +239,19 @@ void launch_pit(const float* a, int64_t a_bstride, int64_t a_sstride, const floa
 void launch_online_emit(const float* pred /*[S,2,Lw]*/, int64_t Lw, const int32_t* perm, int S, int hop, int tail_cap,
                         const float* tail_in /*[S,2,tail_cap]*/, int tail_len, float* tail_out, float* emitted /*[S,2,hop]*/,
                         cudaStream_t st);
-// live.cu: streaming sessions. Slots index the per-slot state: hops_done [capacity], in_ring [capacity][2][16000],
-// tail_ring [capacity][2][2][16000]; slots (device) [n] lists the slot of each entry of a push.
+// live.cu: streaming sessions with a window of W and a hop of H samples (R = W - H). Slots index the per-slot state:
+// hops_done [capacity], in_ring [capacity][R], tail_ring [capacity][2][R]; slots (device) [n] lists the slot of each
+// entry of a push. The caller has checked the geometry: 256 <= H, 2 H <= W, W and H multiples of 16.
+struct LiveGeom {
+  int win, hop;               // W, H
+  int vad_frame0, vad_frames; // j0 = ceil((W - H) / 256), F = ceil(W / 256) - j0
+};
 constexpr int kLiveReleaseChunk = 1000;   // slots per release launch (passed by value: 4 KB of kernel arguments)
-void launch_live_window(const int32_t* slots, int n, const int32_t* hops_done, float* in_ring, const float* hops /*[n,16000]*/,
-                        float* win /*[n,48000]*/, cudaStream_t st);
-void launch_live_pit_emit(const int32_t* slots, int n, int32_t* hops_done, const float* pred /*[n,2,48000]*/,
-                          const float* vad /*[n,2,T]*/, int T, float* tail_ring, float* out /*[n,2,16000]*/,
-                          float* out_vad /*[n,2,63] or null*/, int32_t* perm /*[n,2]*/, cudaStream_t st);
+void launch_live_window(const int32_t* slots, int n, const int32_t* hops_done, float* in_ring, const float* hops /*[n,H]*/,
+                        float* win /*[n,W]*/, LiveGeom g, cudaStream_t st);
+void launch_live_pit_emit(const int32_t* slots, int n, int32_t* hops_done, const float* pred /*[n,2,W]*/,
+                          const float* vad /*[n,2,T]*/, int T, float* tail_ring, float* out /*[n,2,H]*/,
+                          float* out_vad /*[n,2,F] or null*/, int32_t* perm /*[n,2]*/, LiveGeom g, cudaStream_t st);
 void launch_live_release(const int32_t* slots_host, int n, int32_t* hops_done, cudaStream_t st);
 
 // Per-handle launch state (septfa_handle owns one; every C-ABI entry binds it to the calling thread before launching).

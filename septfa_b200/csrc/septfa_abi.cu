@@ -107,6 +107,7 @@ struct septfa_graph {
 struct septfa_online {
   septfa_handle* h = nullptr;
   int S = 0;
+  int win = 0, hop = 0;   // W, H; the emitted tail keeps the last W - H samples
   int hops = 0;
   int tail_len = 0;
   int cur = 0;
@@ -117,20 +118,34 @@ struct septfa_online {
 struct septfa_live {
   septfa_handle* h = nullptr;
   int capacity = 0;
+  LiveGeom g{};                   // window W, hop H, VAD frames j0 .. j0 + F - 1
   int32_t* hops_done = nullptr;   // [capacity] hops pushed by the slot's current stream (0: no history is read)
-  float* in_ring = nullptr;       // [capacity][2][16000] the last two input hops, hop k at position k & 1
-  float* tail_ring = nullptr;     // [capacity][2][2][16000] the last two emitted hops (both speakers), the same way
+  float* in_ring = nullptr;       // [capacity][W - H] the last W - H input samples, sample s at position s mod (W - H)
+  float* tail_ring = nullptr;     // [capacity][2][W - H] the last W - H emitted samples of both speakers, the same way
 };
 
 namespace {
 
-constexpr int kFs = 16000, kWinLen = 48000, kHopLen = 16000, kTailCap = 32000;
+constexpr int kFs = 16000, kWinLen = 48000, kHopLen = 16000;
+constexpr int kMaxWinLen = 160000;   // 10 s
 constexpr int kHostChunksMax = 8;
 
 int fail(septfa_handle* h, int code, const std::string& msg) {
   if (h) h->err = msg; else g_create_error = msg;
   return code;
 }
+
+// Window W and hop H of an online state or a live session: 256 <= H, 2 H <= W <= 160000, both multiples of 16 (1 ms,
+// so that ring segments and float4 accesses stay aligned).
+int check_geometry(septfa_handle* h, int W, int H) {
+  const std::string g = "window " + std::to_string(W) + ", hop " + std::to_string(H) + ": ";
+  if (H < 256) return fail(h, SEPTFA_E_INVALID, g + "the hop must be >= 256 samples");
+  if (W < 2 * (int64_t)H) return fail(h, SEPTFA_E_INVALID, g + "the window must be >= 2 hops");
+  if (W > kMaxWinLen) return fail(h, SEPTFA_E_INVALID, g + "the window must be <= 160000 samples (10 s)");
+  if (W % 16 || H % 16) return fail(h, SEPTFA_E_INVALID, g + "window and hop must be multiples of 16 samples (1 ms)");
+  return 0;
+}
+
 #define CUDA_TRY(h, expr)                                                                     \
   do {                                                                                        \
     cudaError_t e_ = (expr);                                                                  \
@@ -1295,13 +1310,21 @@ void septfa_graph_destroy(septfa_graph* g) {
 
 // ------------------------------------------------------------------------------------------ online
 int septfa_online_create(septfa_handle* h, int S, septfa_online** out) {
+  return septfa_online_create_win(h, S, kWinLen, kHopLen, out);
+}
+
+int septfa_online_create_win(septfa_handle* h, int S, int window, int hop, septfa_online** out) {
   if (!h || !out || S < 1 || S > 32767) return fail(h, SEPTFA_E_INVALID, "bad arguments (1 <= S <= 32767 streams per online state)");
+  *out = nullptr;
+  if (int rc = check_geometry(h, window, hop)) { h->last_launches = 0; return rc; }
   if (!h->committed) return fail(h, SEPTFA_E_STATE, "weights not committed");
   CUDA_TRY(h, cudaSetDevice(h->device));
   auto* o = new septfa_online();
   o->h = h;
   o->S = S;
-  const size_t tb = (size_t)S * 2 * kTailCap * sizeof(float);
+  o->win = window;
+  o->hop = hop;
+  const size_t tb = (size_t)S * 2 * (window - hop) * sizeof(float);
   if (cudaMalloc(reinterpret_cast<void**>(&o->tail[0]), tb) != cudaSuccess ||
       cudaMalloc(reinterpret_cast<void**>(&o->tail[1]), tb) != cudaSuccess ||
       cudaMalloc(reinterpret_cast<void**>(&o->acc), (size_t)S * 4 * sizeof(double)) != cudaSuccess) {
@@ -1330,9 +1353,9 @@ int septfa_online_hops_done(const septfa_online* o) { return o ? o->hops : 0; }
 
 size_t septfa_online_workspace_bytes(const septfa_online* o) {
   if (!o) return 0;
-  const size_t pred = ((size_t)o->S * 2 * kWinLen * sizeof(float) + 255) & ~(size_t)255;
-  const size_t vad = ((size_t)o->S * 2 * septfa_num_frames(kWinLen) * sizeof(float) + 255) & ~(size_t)255;
-  return pred + vad + septfa_workspace_bytes(o->h, o->S, kWinLen) + 256;
+  const size_t pred = ((size_t)o->S * 2 * o->win * sizeof(float) + 255) & ~(size_t)255;
+  const size_t vad = ((size_t)o->S * 2 * septfa_num_frames(o->win) * sizeof(float) + 255) & ~(size_t)255;
+  return pred + vad + septfa_workspace_bytes(o->h, o->S, o->win) + 256;
 }
 
 int septfa_online_step(septfa_online* o, const float* win, const septfa_infer_kw* kw, float* emitted, int32_t* perm,
@@ -1342,31 +1365,32 @@ int septfa_online_step(septfa_online* o, const float* win, const septfa_infer_kw
   if (workspace_bytes < septfa_online_workspace_bytes(o)) return fail(h, SEPTFA_E_WORKSPACE, "online workspace too small");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
-  const size_t pred_b = ((size_t)o->S * 2 * kWinLen * sizeof(float) + 255) & ~(size_t)255;
-  const size_t vad_b = ((size_t)o->S * 2 * septfa_num_frames(kWinLen) * sizeof(float) + 255) & ~(size_t)255;
+  const size_t pred_b = ((size_t)o->S * 2 * o->win * sizeof(float) + 255) & ~(size_t)255;
+  const size_t vad_b = ((size_t)o->S * 2 * septfa_num_frames(o->win) * sizeof(float) + 255) & ~(size_t)255;
   float* pred = reinterpret_cast<float*>(base);
   float* vad = reinterpret_cast<float*>(base + pred_b);
   void* fws = base + pred_b + vad_b;
   // pred_separation, _, _ = self.model(truncated_signal_mix, inference_kw)   online_class_unknown_targets.py:84
-  if (int rc = septfa_forward(h, win, o->S, kWinLen, kw, pred, vad, nullptr, nullptr, nullptr, nullptr, fws,
+  if (int rc = septfa_forward(h, win, o->S, o->win, kw, pred, vad, nullptr, nullptr, nullptr, nullptr, fws,
                               workspace_bytes - pred_b - vad_b - 256, st))
     return rc;
   int launches = h->last_launches;
   bind_ctx(&h->lctx);
   ctx().launches = 0;
-  const int64_t Lw = kWinLen;
+  const int64_t Lw = o->win;
+  const int hop = o->hop, tail_cap = o->win - o->hop;
   if (o->hops == 0) {
-    // indx == 0: online_signal = pred[..., -fs:] (not yet reordered) is what the overlap is compared to (:85-88)
-    launch_pit(pred + (Lw - 2 * kHopLen), 2 * Lw, Lw, pred + (Lw - kHopLen), 2 * Lw, Lw, o->S, kHopLen, o->acc, perm, st);
+    // indx == 0: online_signal = pred[..., -hop:] (not yet reordered) is what the overlap is compared to (:85-88)
+    launch_pit(pred + (Lw - 2 * hop), 2 * Lw, Lw, pred + (Lw - hop), 2 * Lw, Lw, o->S, hop, o->acc, perm, st);
   } else {
-    const int n = o->tail_len;  // min(emitted so far, 2 s)
-    launch_pit(pred + (Lw - kHopLen - n), 2 * Lw, Lw, o->tail[o->cur], 2 * (int64_t)kTailCap, kTailCap, o->S, n, o->acc,
+    const int n = o->tail_len;  // min(emitted so far, W - H)
+    launch_pit(pred + (Lw - hop - n), 2 * Lw, Lw, o->tail[o->cur], 2 * (int64_t)tail_cap, tail_cap, o->S, n, o->acc,
                perm, st);
   }
-  // pred = reorder_source_mse(pred, perm); online_signal = cat(online_signal, pred[..., -fs:])   (:93-94)
-  launch_online_emit(pred, Lw, perm, o->S, kHopLen, kTailCap, o->tail[o->cur], o->tail_len, o->tail[o->cur ^ 1], emitted, st);
+  // pred = reorder_source_mse(pred, perm); online_signal = cat(online_signal, pred[..., -hop:])   (:93-94)
+  launch_online_emit(pred, Lw, perm, o->S, hop, tail_cap, o->tail[o->cur], o->tail_len, o->tail[o->cur ^ 1], emitted, st);
   o->cur ^= 1;
-  o->tail_len = std::min(o->tail_len + kHopLen, kTailCap);
+  o->tail_len = std::min(o->tail_len + hop, tail_cap);
   o->hops += 1;
   h->last_launches = launches + ctx().launches;
   CUDA_TRY(h, cudaGetLastError());
@@ -1380,24 +1404,25 @@ namespace {
 
 struct LiveWorkspace {
   int32_t* slots;   // [n] device copy of the push's slot list
-  float* win;       // [n, 48000]
-  float* pred;      // [n, 2, 48000]
-  float* vad;       // [n, 2, 188]
+  float* win;       // [n, W]
+  float* pred;      // [n, 2, W]
+  float* vad;       // [n, 2, T(W)]
   void* fws;        // the forward's workspace
   size_t fws_bytes;
   size_t total;
 };
 
-LiveWorkspace live_carve(const septfa_handle* h, uintptr_t base, int n) {
+LiveWorkspace live_carve(const septfa_live* lv, uintptr_t base, int n) {
   auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+  const int W = lv->g.win;
   LiveWorkspace w{};
   size_t off = 0;
   w.slots = reinterpret_cast<int32_t*>(base + off); off += al((size_t)n * sizeof(int32_t));
-  w.win = reinterpret_cast<float*>(base + off);     off += al((size_t)n * kWinLen * sizeof(float));
-  w.pred = reinterpret_cast<float*>(base + off);    off += al((size_t)n * 2 * kWinLen * sizeof(float));
-  w.vad = reinterpret_cast<float*>(base + off);     off += al((size_t)n * 2 * septfa_num_frames(kWinLen) * sizeof(float));
+  w.win = reinterpret_cast<float*>(base + off);     off += al((size_t)n * W * sizeof(float));
+  w.pred = reinterpret_cast<float*>(base + off);    off += al((size_t)n * 2 * W * sizeof(float));
+  w.vad = reinterpret_cast<float*>(base + off);     off += al((size_t)n * 2 * septfa_num_frames(W) * sizeof(float));
   w.fws = reinterpret_cast<void*>(base + off);
-  w.fws_bytes = septfa_workspace_bytes(h, n, kWinLen);
+  w.fws_bytes = septfa_workspace_bytes(lv->h, n, W);
   w.total = off + w.fws_bytes;
   return w;
 }
@@ -1427,18 +1452,25 @@ int check_live_slots(septfa_live* lv, const int32_t* slots, int n) {
 extern "C" {
 
 int septfa_live_create(septfa_handle* h, int capacity, septfa_live** out) {
+  return septfa_live_create_win(h, capacity, kWinLen, kHopLen, out);
+}
+
+int septfa_live_create_win(septfa_handle* h, int capacity, int window, int hop, septfa_live** out) {
   if (!h || !out || capacity < 1 || capacity > 32767)
     return fail(h, SEPTFA_E_INVALID, "bad arguments (1 <= capacity <= 32767 slots per live session)");
   *out = nullptr;
+  if (int rc = check_geometry(h, window, hop)) { h->last_launches = 0; return rc; }
   if (!h->committed) return fail(h, SEPTFA_E_STATE, "weights not committed");
   CUDA_TRY(h, cudaSetDevice(h->device));
   auto* lv = new septfa_live();
   lv->h = h;
   lv->capacity = capacity;
-  const size_t hop_b = (size_t)kHopLen * sizeof(float);
+  const int first = (window - hop + 255) / 256;   // the first window frame whose centre 256 j lies in [W - H, W)
+  lv->g = LiveGeom{window, hop, first, (window + 255) / 256 - first};
+  const size_t ring_b = (size_t)(window - hop) * sizeof(float);
   if (cudaMalloc(reinterpret_cast<void**>(&lv->hops_done), (size_t)capacity * sizeof(int32_t)) != cudaSuccess ||
-      cudaMalloc(reinterpret_cast<void**>(&lv->in_ring), (size_t)capacity * 2 * hop_b) != cudaSuccess ||
-      cudaMalloc(reinterpret_cast<void**>(&lv->tail_ring), (size_t)capacity * 4 * hop_b) != cudaSuccess ||
+      cudaMalloc(reinterpret_cast<void**>(&lv->in_ring), (size_t)capacity * ring_b) != cudaSuccess ||
+      cudaMalloc(reinterpret_cast<void**>(&lv->tail_ring), (size_t)capacity * 2 * ring_b) != cudaSuccess ||
       cudaMemset(lv->hops_done, 0, (size_t)capacity * sizeof(int32_t)) != cudaSuccess) {
     cudaFree(lv->hops_done); cudaFree(lv->in_ring); cudaFree(lv->tail_ring);
     delete lv;
@@ -1457,7 +1489,13 @@ void septfa_live_destroy(septfa_live* lv) {
 
 size_t septfa_live_workspace_bytes(const septfa_live* lv, int n) {
   if (!lv || n < 1 || n > lv->capacity) return 0;
-  return live_carve(lv->h, 0, n).total + 256;
+  return live_carve(lv, 0, n).total + 256;
+}
+
+int septfa_live_vad_frames(const septfa_live* lv, int* first_frame) {
+  if (!lv) return SEPTFA_E_INVALID;
+  if (first_frame) *first_frame = lv->g.vad_frame0;
+  return lv->g.vad_frames;
 }
 
 int septfa_live_release(septfa_live* lv, const int32_t* slots_host, int n, void* stream) {
@@ -1484,20 +1522,20 @@ int septfa_live_push(septfa_live* lv, const int32_t* slots_host, int n, const fl
   if (workspace_bytes < septfa_live_workspace_bytes(lv, n)) return fail(h, SEPTFA_E_WORKSPACE, "live workspace too small");
   CUDA_TRY(h, cudaSetDevice(h->device));
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const LiveWorkspace ws = live_carve(h, (reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255, n);
+  const LiveWorkspace ws = live_carve(lv, (reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255, n);
   CUDA_TRY(h, cudaMemcpyAsync(ws.slots, slots_host, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
   bind_ctx(&h->lctx);
   ctx().launches = 0;
-  launch_live_window(ws.slots, n, lv->hops_done, lv->in_ring, hops, ws.win, st);
+  launch_live_window(ws.slots, n, lv->hops_done, lv->in_ring, hops, ws.win, lv->g, st);
   const int before = ctx().launches;
-  if (int rc = septfa_forward(h, ws.win, n, kWinLen, kw, ws.pred, ws.vad, nullptr, nullptr, nullptr, nullptr, ws.fws,
+  if (int rc = septfa_forward(h, ws.win, n, lv->g.win, kw, ws.pred, ws.vad, nullptr, nullptr, nullptr, nullptr, ws.fws,
                               ws.fws_bytes, st))
     return rc;
   const int launches = before + h->last_launches;
   bind_ctx(&h->lctx);
   ctx().launches = 0;
-  launch_live_pit_emit(ws.slots, n, lv->hops_done, ws.pred, ws.vad, (int)septfa_num_frames(kWinLen), lv->tail_ring, out,
-                       out_vad, perm, st);
+  launch_live_pit_emit(ws.slots, n, lv->hops_done, ws.pred, ws.vad, (int)septfa_num_frames(lv->g.win), lv->tail_ring, out,
+                       out_vad, perm, lv->g, st);
   h->last_launches = launches + ctx().launches;
   CUDA_TRY(h, cudaGetLastError());
   return 0;

@@ -91,6 +91,7 @@ _PROTOS = {
     "septfa_graph_destroy": (None, [C.c_void_p]),
     "septfa_profile_read": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_int), C.c_int, C.c_int]),
     "septfa_online_create": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]),
+    "septfa_online_create_win": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "septfa_online_destroy": (None, [C.c_void_p]),
     "septfa_online_reset": (C.c_int, [C.c_void_p, C.c_void_p]),
     "septfa_online_workspace_bytes": (C.c_size_t, [C.c_void_p]),
@@ -98,7 +99,9 @@ _PROTOS = {
                                      C.c_size_t, C.c_void_p]),
     "septfa_online_hops_done": (C.c_int, [C.c_void_p]),
     "septfa_live_create": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]),
+    "septfa_live_create_win": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "septfa_live_destroy": (None, [C.c_void_p]),
+    "septfa_live_vad_frames": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "septfa_live_workspace_bytes": (C.c_size_t, [C.c_void_p, C.c_int]),
     "septfa_live_release": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "septfa_live_push": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.POINTER(InferKw), C.c_void_p, C.c_void_p,

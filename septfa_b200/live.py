@@ -1,12 +1,14 @@
-"""Live streaming sessions: one 1 s hop per stream slot per push, streams that start and end independently, VAD per hop.
+"""Live streaming sessions: one hop per stream slot per push, streams that start and end independently, VAD per hop.
 
 ``OnlineSaving.calc_online`` drives S streams in lockstep over whole recordings the caller already holds. A
 :class:`LiveSession` serves streams as they arrive: each slot hosts one stream at a time, every push carries one new
-hop for any subset of the slots, and the session keeps each stream's last two input hops and last two emitted hops on
-the device (``septfa_live_*`` in ``include/septfa.h``). Push k of a stream returns the stream's separated samples
-``[16000 k, 16000 (k + 1))``: the concatenated output of a stream of N pushes equals
-``OnlineSaving.calc_online(F.pad(x, (32000, 0)))`` on that stream alone (the windowing of
-``model/online_class_known_targets.py:92-93``, the stitch of ``model/online_class_unknown_targets.py:84-94``).
+hop for any subset of the slots, and the session keeps each stream's last ``window - hop`` input samples and emitted
+samples on the device (``septfa_live_*`` in ``include/septfa.h``). With a window of W and a hop of H samples (default
+48000 / 16000), push k of a stream returns the stream's separated samples ``[H k, H (k + 1))``: the concatenated output
+of a stream of N pushes equals ``OnlineSaving.calc_online(F.pad(x, (W - H, 0)))`` with ``max_len = W / 16000`` and
+``save_sec = H / 16000`` on that stream alone (the windowing of ``model/online_class_known_targets.py:92-93``, the
+stitch of ``model/online_class_unknown_targets.py:84-94``). The oldest sample of a hop comes back about H samples after
+it was taken, plus the push time: the hop sets the latency.
 """
 from __future__ import annotations
 
@@ -17,8 +19,27 @@ import torch
 
 from . import lib as _lib
 
-HOP = 16000
-FRAMES_PER_HOP = 63
+WINDOW = 48000
+HOP = 16000              # the default hop
+FRAMES_PER_HOP = 63      # VAD frames per push at the default geometry
+MAX_WINDOW = 160000      # 10 s
+
+
+def check_geometry(window, hop):
+    """``(window, hop)`` as ints if the library accepts them: 256 <= hop, 2 hop <= window <= 160000, both multiples of 16
+    samples (1 ms); ``ValueError`` otherwise."""
+    if not all(isinstance(v, (int, np.integer)) and not isinstance(v, bool) for v in (window, hop)):
+        raise ValueError(f"window and hop are integer sample counts, got {window!r}, {hop!r}")
+    window, hop = int(window), int(hop)
+    if hop < 256:
+        raise ValueError(f"hop = {hop}: must be >= 256 samples")
+    if window < 2 * hop:
+        raise ValueError(f"window = {window}, hop = {hop}: the window must be >= 2 hops")
+    if window > MAX_WINDOW:
+        raise ValueError(f"window = {window}: must be <= {MAX_WINDOW} samples (10 s)")
+    if window % 16 or hop % 16:
+        raise ValueError(f"window = {window}, hop = {hop}: both must be multiples of 16 samples (1 ms)")
+    return window, hop
 
 
 def check_slots(slots, capacity):
@@ -39,19 +60,22 @@ def check_slots(slots, capacity):
 class LiveSession:
     """``capacity`` stream slots on one device, for a :class:`~septfa_b200.model.SeparationModel`.
 
-    ``push(slots, hops)`` takes one hop (16000 float32 samples, already normalised) for each listed slot and returns
-    ``(out [n, 2, 16000], vad [n, 2, 63] or None, perm [n, 2] int32)`` on the device, stream-ordered on the current
-    stream. ``vad`` holds frames 125 .. 187 of the window's VAD output (frame j centred on stream sample
-    ``16000 k + 256 j``), speakers in the emitted order; it is None for a model without a VAD head or with
-    ``vad=False``. ``release(slots)`` ends the streams in those slots: the next push into one starts a new stream.
-    ``inference_kw`` is the forward's (gating, smoothed VAD), fixed for the session.
+    Every stream has a window of ``window`` and a hop of ``hop`` samples (see :func:`check_geometry`).
+    ``push(slots, hops)`` takes one hop (``hop`` float32 samples, already normalised) for each listed slot and returns
+    ``(out [n, 2, hop], vad [n, 2, frames_per_hop] or None, perm [n, 2] int32)`` on the device, stream-ordered on the
+    current stream. ``vad`` holds the window frames ``first_frame .. first_frame + frames_per_hop - 1`` of the window's
+    VAD output, those centred on the new hop (frame j centred on window sample ``256 j``; 125 .. 187 at the default),
+    speakers in the emitted order; it is None for a model without a VAD head or with ``vad=False``. ``release(slots)``
+    ends the streams in those slots: the next push into one starts a new stream. ``inference_kw`` is the forward's
+    (gating, smoothed VAD), fixed for the session.
     """
 
-    def __init__(self, model, capacity, inference_kw=None, device=None):
+    def __init__(self, model, capacity, inference_kw=None, device=None, window=WINDOW, hop=HOP):
         self.model = model
         self.capacity = int(capacity)
         if not 1 <= self.capacity <= 32767:
             raise ValueError("capacity must lie in 1 .. 32767")
+        self.window, self.hop = check_geometry(window, hop)
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         if self.device.type != "cuda":
             raise RuntimeError("septfa_b200.LiveSession runs on CUDA only (no CPU fallback)")
@@ -59,7 +83,11 @@ class LiveSession:
         self._lv = C.c_void_p()
         with torch.cuda.device(self.device):
             self._h = model._handle(self.device)
-            _lib.check(self._h.ptr, self._h.lib.septfa_live_create(self._h.ptr, self.capacity, C.byref(self._lv)))
+            _lib.check(self._h.ptr, self._h.lib.septfa_live_create_win(self._h.ptr, self.capacity, self.window, self.hop,
+                                                                       C.byref(self._lv)))
+            j0 = C.c_int()
+            self.frames_per_hop = self._h.lib.septfa_live_vad_frames(self._lv, C.byref(j0))
+            self.first_frame = j0.value
             need = self._h.lib.septfa_live_workspace_bytes(self._lv, self.capacity)
             self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
         self.last_launch_count = 0
@@ -72,15 +100,15 @@ class LiveSession:
         n = ids.size
         if not (isinstance(hops, torch.Tensor) and hops.is_cuda and hops.dtype == torch.float32):
             raise ValueError("hops must be a CUDA float32 tensor")
-        if tuple(hops.shape) != (n, HOP):
-            raise ValueError(f"hops must have shape ({n}, {HOP}), got {tuple(hops.shape)}")
+        if tuple(hops.shape) != (n, self.hop):
+            raise ValueError(f"hops must have shape ({n}, {self.hop}), got {tuple(hops.shape)}")
         if hops.device != self.device:
             raise ValueError(f"hops are on {hops.device}, the session on {self.device}")
         hops = hops.contiguous()
         with torch.cuda.device(self.device):
             h = self.model._handle(self.device)
-            out = torch.empty((n, 2, HOP), dtype=torch.float32, device=self.device)
-            v = torch.empty((n, 2, FRAMES_PER_HOP), dtype=torch.float32, device=self.device) \
+            out = torch.empty((n, 2, self.hop), dtype=torch.float32, device=self.device)
+            v = torch.empty((n, 2, self.frames_per_hop), dtype=torch.float32, device=self.device) \
                 if (vad and self.model.final_vad) else None
             perm = torch.empty((n, 2), dtype=torch.int32, device=self.device)
             rc = h.lib.septfa_live_push(self._lv, ids.ctypes.data_as(C.c_void_p), n, C.c_void_p(hops.data_ptr()),

@@ -1,4 +1,4 @@
-"""Sliding-window "online" drivers (3 s window, 1 s hop) on top of the CUDA forward.
+"""Sliding-window "online" drivers (3 s window, 1 s hop by default) on top of the CUDA forward.
 
 Reference: ``model/online_class_unknown_targets.py:9-105`` (``OnlineSaving``) and
 ``model/online_class_known_targets.py:9-154``. The reference re-runs the full non-causal model
@@ -21,6 +21,7 @@ import numpy as np
 import torch
 
 from . import lib as _lib
+from .live import check_geometry
 from .pit import PITLossWrapper, calc_sisdr, reorder_source_mse
 
 
@@ -64,7 +65,23 @@ class OnlineSaving:
 
     def get_truncated_signal(self, full_signal_mix):
         s = int(np.floor(self.fs * self.indx * self.save_sec))
-        return full_signal_mix[:, s: s + self.max_len * self.fs]  # :39-41
+        return full_signal_mix[:, s: s + self.geometry()[0]]  # :39-41
+
+    def geometry(self):
+        """(W, H) = (fs * max_len, fs * save_sec) in samples. The device stitch takes integer windows and hops that
+        ``live.check_geometry`` accepts (256 <= H, 2 H <= W <= 160000, multiples of 16); anything else raises
+        ``NotImplementedError``."""
+        wh = []
+        for name, sec in (("max_len", self.max_len), ("save_sec", self.save_sec)):
+            v = self.fs * sec
+            if abs(v - round(v)) > 1e-6:
+                raise NotImplementedError(f"septfa_b200.OnlineSaving: fs * {name} = {v} is not a whole number of samples")
+            wh.append(int(round(v)))
+        try:
+            return check_geometry(*wh)
+        except ValueError as e:
+            raise NotImplementedError(f"septfa_b200.OnlineSaving: max_len = {self.max_len}, save_sec = {self.save_sec}: "
+                                      f"{e}") from None
 
     # -- wav dumps (host I/O, batch item 0 like the reference) ------------------------------
     def save_audio(self, name_folder, separated_signals, mix):
@@ -89,18 +106,18 @@ class OnlineSaving:
         """model/online_class_unknown_targets.py:72-105. ``full_signal_mix`` [S, L] on a CUDA device."""
         if not full_signal_mix.is_cuda:
             raise RuntimeError("septfa_b200.OnlineSaving runs on CUDA only (no CPU fallback)")
+        win_len, hop = self.geometry()
         x = full_signal_mix.detach().float()
-        if x.shape[-1] < self.fs * self.max_len:                                              # :73-74
-            x = torch.nn.functional.pad(x, (0, self.fs * self.max_len - x.shape[-1]))
+        if x.shape[-1] < win_len:                                                             # :73-74
+            x = torch.nn.functional.pad(x, (0, win_len - x.shape[-1]))
         max_indx = np.floor((x.shape[-1] - self.fs * self.max_len) / (self.fs * self.save_sec))  # :77
         S = x.shape[0]
         dev = x.device
-        hop = int(np.floor(self.fs * self.save_sec))
         kw = _lib.InferKw.from_dict(inference_kw) if (inference_kw and self.model.final_vad) else None
         with torch.cuda.device(dev):
             h = self.model._handle(dev)
             st = C.c_void_p()
-            _lib.check(h.ptr, h.lib.septfa_online_create(h.ptr, S, C.byref(st)))
+            _lib.check(h.ptr, h.lib.septfa_online_create_win(h.ptr, S, win_len, hop, C.byref(st)))
             try:
                 need = h.lib.septfa_online_workspace_bytes(st)
                 ws = torch.empty(need, dtype=torch.uint8, device=dev)
@@ -118,9 +135,9 @@ class OnlineSaving:
                     online[:, :, self.indx * hop:(self.indx + 1) * hop] = emitted              # :94 (cat)
                     if sample_indx < self.num_save_samples:                                   # :95-96
                         # per-window dumps of batch item 0: the model's window output (first tensor of the online
-                        # workspace, [S, 2, 48000]) reordered by this hop's permutation, and the window of the mixture
+                        # workspace, [S, 2, W]) reordered by this hop's permutation, and the window of the mixture
                         base = (ws.data_ptr() + 255) // 256 * 256 - ws.data_ptr()
-                        pred0 = ws[base: base + 2 * self.max_len * self.fs * 4].view(torch.float32).view(1, 2, -1)
+                        pred0 = ws[base: base + 2 * win_len * 4].view(torch.float32).view(1, 2, -1)
                         pred0 = pred0[:, perms[self.indx][0].long()]
                         self.save_audio(name_folder, pred0, win)
                     self.increase_indx()

@@ -1,13 +1,16 @@
-"""Live-session push latency against the lockstep online step at the same number of streams.
+"""Live-session push latency against the lockstep online step at the same number of streams and the same geometry.
 
-Workload: a live session of --capacity slots (config_with_vad, seeded weights, filter_signals_by_smo_vad). Slot s starts
-its first stream at step s mod 7; every stream runs 3 .. 10 hops of a seeded synthetic mixture, then its slot releases
-and starts the next stream at the same step. Once all slots have started, every step pushes every slot (n = capacity),
-with some slots at k = 0 .. 2 (zero-padded windows) and the rest in steady state. The lockstep leg is
-septfa_online_step on the same number of streams with resident 3 s windows (the online leg of bench.py). The two legs
-alternate step by step; each call is timed with CUDA events between two device synchronisations, on its own.
+Workload: a live session of --capacity slots with a window of --window and a hop of --hop samples (config_with_vad,
+seeded weights, filter_signals_by_smo_vad). With c = window / (3 hop) (1 at the default 48000 / 16000), slot s starts
+its first stream at step s mod 7c; every stream runs 3c .. 10c hops of a seeded synthetic mixture, then its slot
+releases and starts the next stream at the same step. Once all slots have started, every step pushes every slot
+(n = capacity), with some slots in their zero-padded first pushes and the rest in steady state. The lockstep leg is
+septfa_online_step on the same number of streams with resident windows of the same geometry (the online leg of
+bench.py at the default). The two legs alternate step by step; each call is timed with CUDA events between two device
+synchronisations, on its own. realtime_streams = capacity * (hop / 16000) / push p99: the streams one GPU keeps up
+with when it does nothing but push.
 
-    python tools/live_bench.py [--capacity 1024 --steps 60 --warmup 10] --out profiles/live_bench_n1024.json
+    python tools/live_bench.py [--capacity 1024 --steps 60 --warmup 10c --window 48000 --hop 16000] --out FILE.json
 """
 import argparse
 import contextlib
@@ -26,7 +29,7 @@ from septfa_b200 import lib as _lib  # noqa: E402
 from septfa_b200 import synth  # noqa: E402
 from septfa_b200.model import SeparationModel  # noqa: E402
 
-HOP = 16000
+FS = 16000
 
 
 def gpu_info(index):
@@ -45,9 +48,18 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--capacity", type=int, default=1024)
     ap.add_argument("--steps", type=int, default=60, help="timed steps per leg")
-    ap.add_argument("--warmup", type=int, default=10, help="untimed steps first (>= 7: every slot has started)")
+    ap.add_argument("--warmup", type=int, default=None, help="untimed steps first (default 10c; >= 7c: every slot has started)")
+    ap.add_argument("--window", type=int, default=48000, help="window W in samples")
+    ap.add_argument("--hop", type=int, default=16000, help="hop H in samples")
     ap.add_argument("--out", default=None, help="write the JSON record here too")
     a = ap.parse_args()
+    W, H = a.window, a.hop
+    c = W / (3 * H)                                  # hop counts scale with W / H
+    period, max_hops = max(1, round(7 * c)), round(10 * c)
+    if a.warmup is None:
+        a.warmup = round(10 * c)
+    if a.warmup < period:
+        raise SystemExit(f"--warmup must be >= {period}: every slot must have started before the timed steps")
     if not torch.cuda.is_available():
         raise SystemExit("live_bench measures on a CUDA device; none found")
     dev = torch.device("cuda", 0)
@@ -63,24 +75,25 @@ def main():
     n = a.capacity
     stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
 
-    # 32 distinct mixtures of 10 hops; stream j of slot s plays mixture (s + 7 j) % 32 for 3 + (s + j) % 8 hops
-    mixes = torch.from_numpy(synth.make_mixtures(32, 10 * HOP, 4321)).to(dev).view(32, 10, HOP)
-    start = np.arange(n) % 7
+    # 32 distinct mixtures of 10c hops; stream j of slot s plays mixture (s + 7 j) % 32 for (3 + (s + j) % 8) c hops
+    mixes = torch.from_numpy(synth.make_mixtures(32, max_hops * H, 4321)).to(dev).view(32, max_hops, H)
+    start = np.arange(n) % period
     gen = np.zeros(n, dtype=np.int64)          # streams finished per slot
     k = np.zeros(n, dtype=np.int64)            # hops pushed by the slot's current stream
 
     lv = C.c_void_p()
-    _lib.check(h.ptr, lib.septfa_live_create(h.ptr, n, C.byref(lv)))
+    _lib.check(h.ptr, lib.septfa_live_create_win(h.ptr, n, W, H, C.byref(lv)))
+    n_vad = lib.septfa_live_vad_frames(lv, None)
     ws = torch.empty(lib.septfa_live_workspace_bytes(lv, n), dtype=torch.uint8, device=dev)
-    out = torch.empty((n, 2, HOP), device=dev)
-    vad = torch.empty((n, 2, 63), device=dev)
+    out = torch.empty((n, 2, H), device=dev)
+    vad = torch.empty((n, 2, n_vad), device=dev)
     perm = torch.empty((n, 2), dtype=torch.int32, device=dev)
 
     st = C.c_void_p()
-    _lib.check(h.ptr, lib.septfa_online_create(h.ptr, n, C.byref(st)))
+    _lib.check(h.ptr, lib.septfa_online_create_win(h.ptr, n, W, H, C.byref(st)))
     ws_on = torch.empty(lib.septfa_online_workspace_bytes(st), dtype=torch.uint8, device=dev)
-    win = torch.from_numpy(np.tile(synth.make_mixtures(16, 48000, 4321), ((n + 15) // 16, 1))[:n]).to(dev)
-    emitted = torch.empty((n, 2, HOP), device=dev)
+    win = torch.from_numpy(np.tile(synth.make_mixtures(16, W, 4321), ((n + 15) // 16, 1))[:n]).to(dev)
+    emitted = torch.empty((n, 2, H), device=dev)
     perm_on = torch.empty((n, 2), dtype=torch.int32, device=dev)
 
     def timed(fn):
@@ -94,7 +107,7 @@ def main():
 
     push_ms, step_ms, ns, restarts, launches = [], [], [], [], 0
     for t in range(a.warmup + a.steps):
-        length = 3 + (np.arange(n) + gen) % 8
+        length = np.round((3 + (np.arange(n) + gen) % 8) * c).astype(np.int64)
         ended = np.nonzero((k == length) & (start <= t))[0].astype(np.int32)
         if ended.size:
             _lib.check(h.ptr, lib.septfa_live_release(lv, ended.ctypes.data_as(C.c_void_p), ended.size, stream))
@@ -129,16 +142,19 @@ def main():
     lib.septfa_live_destroy(lv)
     lib.septfa_online_destroy(st)
 
-    p50p, p50s = pct(push_ms, 0.5), pct(step_ms, 0.5)
+    p50p, p50s, p99p = pct(push_ms, 0.5), pct(step_ms, 0.5), pct(push_ms, 0.99)
     rec = {"bench": "live_push_vs_lockstep_online_step", **gpu_info(0),
-           "config": "config_with_vad, seeded weights, filter_signals_by_smo_vad, 3 s windows / 1 s hops",
+           "config": "config_with_vad, seeded weights, filter_signals_by_smo_vad",
+           "window": W, "hop": H, "frames": _lib.num_frames(W), "vad_frames_per_push": n_vad,
            "streams": n, "timed_steps": len(push_ms), "warmup_steps": a.warmup,
+           "stream_hops": [int(round(3 * c)), max_hops], "start_period_steps": period,
            "releases_per_step_mean": float(np.mean(restarts)),
-           "push": {"p50_ms": p50p, "p99_ms": pct(push_ms, 0.99), "min_ms": min(push_ms), "launches": launches},
+           "push": {"p50_ms": p50p, "p99_ms": p99p, "min_ms": min(push_ms), "launches": launches},
            "lockstep_step": {"p50_ms": p50s, "p99_ms": pct(step_ms, 0.99), "min_ms": min(step_ms)},
            "push_over_step_p50": p50p / p50s,
+           "realtime_streams_at_push_p99": n * (H / FS) / (p99p / 1000.0),
            "timing": "CUDA events around one call between device synchronisations; legs alternate step by step",
-           "state_bytes_per_slot": 4 + 6 * HOP * 4}
+           "state_bytes_per_slot": 4 + 12 * (W - H)}
     line = json.dumps(rec)
     print(line, flush=True)
     if a.out:
