@@ -105,12 +105,14 @@ int64_t septfa_key_numel(const septfa_handle* h, int i);
  * batch chunks septfa_forward_host pipelines over its two stream lanes); kernel-selection switches for
  * cross-checks (default 1): "fused_resid" (cluster-resident gate + residual kernel), "conv1_persist"
  * (persistent warp-specialised conv1 kernel), "pdl" (programmatic dependent launch of the kernel chain),
- * "dconv_mma" (tensor-core depthwise + res_out kernel), "dconv_pair" (... on CTA pairs, cta_group::2, weights resident),
- * "conv1_pair" (TF32 CTA-pair conv1 fed by TMA from the fp32 stream; blocks 1 .. n-1 of the recursive-LN wiring),
- * "conv1_wres" (resident weights in the persistent conv1 kernel), "l2_discard" (the hand-off buffers inside a block are
- * dropped from the L2 once they have been read);
+ * "dconv_mma" (tensor-core depthwise + res_out kernel on CTA pairs, cta_group::2, weights resident),
+ * "conv1_pair" (TF32 CTA-pair conv1 fed by TMA from the fp32 stream; blocks 1 .. n-1 of the recursive-LN wiring;
+ * 2 = at any batch size), "l2_discard" (the hand-off buffers inside a block are dropped from the L2 once they have been read);
  * "stream_half" (default 0): opt-in mode that stores the residual stream between blocks as fp16 - 11 % faster, but the
- * stream's rounding accumulates over all blocks (VAD probabilities within 2e-3 of the reference instead of 1e-3). */
+ * stream's rounding accumulates over all blocks (VAD probabilities within 2e-3 of the reference instead of 1e-3).
+ * Any other name is refused with SEPTFA_E_INVALID ("unknown option"), among them the retired switches that selected a
+ * kernel slower on every measured workload (the single-CTA depthwise kernel and its bring-up variants, the streamed-weight
+ * form of the persistent conv1 kernel). */
 /* "precision": arithmetic of the two block contractions (conv1d 256->256, res_out 512->256) on the tensor cores.
  *   SEPTFA_PRECISION_FAST      fp16 operands, one tcgen05 pass, fp16 storage of the tensors between them
  *   SEPTFA_PRECISION_ACCURATE  2-term fp16 split of both operands (three passes, fp32-accurate), fp32 storage

@@ -1,13 +1,28 @@
-// Two-SM (cta_group::2) variant of the tensor-core depthwise + res_out kernel of dconv_mma.cu (model/model.py:136/142,144):
+// Persistent, warp-specialised tcgen05 kernel for the second half of a TCN block (model/model.py:136/142,144), on CTA pairs:
 //   q = PReLU(depthwise dilated k3 conv(GN1(p))),  racc = (W3 diag(g2)) q,  statistics of q, row / column sums of racc
-// The arithmetic, the plane layout of p, the block-diagonal mini-GEMMs, the register transform with q written back to
-// tensor memory (A-from-TMEM res_out MMA) and the exact edge corrections are those of dconv_mma.cu. What changes is who
-// holds the weights: the CTAs run as PAIRS (clusters of two on one TPC) and every MMA is a tcgen05.mma.cta_group::2 of
-// M = 256 (128 frames per CTA) issued by the pair's leader; the B operand of such an MMA is split along N between the two
-// CTAs, so each CTA needs only HALF of the res_out weight image (128 of its 256 output rows: 128 KB) and half of every
-// tap matrix (24 KB) - and those fit in shared memory for the whole persistent kernel. dconv_mma.cu re-streams the 256 KB
-// image for every 128-frame tile, which bounds it at one SM's TMA ingress (~20 B/clk: 1.95 k cycles per 64-channel chunk
-// against 0.6 k cycles of MMA work); here the only per-tile traffic into an SM is its own 68 KB of p.
+// with BOTH contractions on the tensor cores. The depthwise convolution is block-diagonal (output channel o reads input
+// channel o/2), so for a group of 16 input channels and one tap k it is a tiny GEMM
+//   D1[frames x 32 outputs] += P_k[frames x 16] * B_k[16 x 32],   P_k = the p tile shifted by (k-1)*dilation frames,
+// whose A operand needs no data movement at all: p is stored by conv1 as per-K-group planes [32][rows][8 channels]
+// (16 bytes per frame and plane), one TMA bulk copy brings a plane's 136 frames (tile + halo) into shared memory already
+// in the canonical no-swizzle K-major core-matrix layout (8 frames x 16 B), and a shift by s frames is the same buffer
+// addressed 16*s bytes further on. GroupNorm reg1 is folded into the taps (w' = w * gamma, fp16) and into a per-row affine
+//   x = rstd * conv + (c2f - rstd * mean * sw),   q = PReLU(x)      (sw = sum of the fp16 taps, c2f = b2 + beta / gamma * sw)
+// applied to the fp32 accumulator on its way from tensor memory to the fp16 A operand of the res_out GEMM, which takes it
+// from tensor memory: q never touches shared memory. That is 9 SASS instructions per PAIR of q values (FFMA2 pipe) instead
+// of ~34 for the CUDA-core depthwise producer of gemm_tc.cu (MODE 1), which bounded that kernel at 20 % of the tensor
+// roofline.
+// Zero padding of the NORMALISED signal (the reference pads h1, not p): the tensor-core convolution reads whatever
+// neighbours the shifted view holds; the <= 2*dil rows per utterance whose tap falls outside are corrected exactly,
+//   x_true = x_mma - w'_k * (rstd * (p_wrong - mean) + beta / gamma),
+// with the same fp16 weight and fp16 input the tensor core multiplied.
+//
+// The CTAs run as PAIRS (clusters of two on one TPC) and every MMA is a tcgen05.mma.cta_group::2 of M = 256 (128 frames
+// per CTA) issued by the pair's leader; the B operand of such an MMA is split along N between the two CTAs, so each CTA
+// needs only HALF of the res_out weight image (128 of its 256 output rows: 128 KB) and half of every tap matrix (24 KB) -
+// and those fit in shared memory for the whole persistent kernel. The per-tile traffic into an SM is its own 68 KB of p.
+// (A single-CTA form has to re-stream the 256 KB image for every 128-frame tile, which bounds it at one SM's TMA ingress:
+// ~20 B/clk, 1.95 k cycles per 64-channel chunk against 0.6 k cycles of MMA work.)
 // Roles per CTA (16 warps):
 //   warp 0        p loader   : 4 bulk copies (K-group planes) per 32-channel chunk, ring of 4
 //   warp 1        static loader (prologue), then EDGE warp: the exact zero-padding corrections of the <= 8 rows of a tile whose
@@ -21,7 +36,8 @@
 //                 128-byte-swizzled boxes -> one TMA tensor store per box (UTMASTG), per-utterance column sums, row sums
 // Tensor memory (per CTA, allocated with cta_group::2): D2 = columns 0-255; ring of 4 x 64 columns at 256-511 (D1, then q).
 // Synchronisation: mbarriers only; barriers the leader's MMA thread waits on receive remote (cluster-scope) arrivals from
-// the peer, MMA completion is multicast to both CTAs. Requires T >= 128 and the plane layout of p.
+// the peer, MMA completion is multicast to both CTAs. Requires T >= 128 (a tile touches at most two utterances) and the
+// plane layout of p (conv1's persistent kernels write it); otherwise the forward uses launch_tc_dconv's kernel.
 #include <algorithm>
 #include <cuda.h>
 #include "kernels.h"
@@ -92,7 +108,8 @@ __device__ __forceinline__ void umma2_f16(uint32_t d_tmem, uint64_t a_desc, uint
       "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate), "r"(0u)
       : "memory");
 }
-// ... with the A operand in each CTA's tensor memory
+// ... with the A operand in each CTA's tensor memory (its 128 rows = 128 lanes, 16-bit elements packed two per 32-bit
+// column: element k of row m lives in lane m, column k / 2, low half for even k)
 __device__ __forceinline__ void umma2_f16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
   asm volatile(
       "{\n\t.reg .pred p;\n\t"

@@ -39,7 +39,7 @@ constexpr int kOffEpi = kOffW + kWStages * kWBytes;
 constexpr int kOffBias = kOffEpi + 4 * kEpiWarpBytes;   // [256] fp32 bias (broadcast LDS instead of 8 uniform LDG per 32 columns)
 constexpr int kOffBar = kOffBias + 1024;
 constexpr int kSmemBytes = kOffBar + 256;
-// Resident-weight variant (PLANES: the epilogue needs no staging buffer): the whole W1 image (4 chunks, 128 KB) is loaded
+// PLANES keeps the weights resident (its epilogue needs no staging buffer): the whole W1 image (4 chunks, 128 KB) is loaded
 // once per CTA and stays in shared memory for every tile, so the per-tile traffic into the SM is the A rows only.
 constexpr int kAStagesR = 4;
 constexpr int kOffWR = kAStagesR * kABytes;                   // 64 KB of A stages, then 128 KB of weights
@@ -61,15 +61,15 @@ struct PersistParams {
 };
 
 // PLANES: p is stored as K-group planes (kernels.h, DconvMmaParams): a lane = a row, so the 32 lanes of a warp write 512
-// contiguous bytes per plane straight from registers (full sectors: no staging, no bulk store).
-template <bool AMAX, bool PLANES, bool WRES>
+// contiguous bytes per plane straight from registers (full sectors: no staging, no bulk store), and the resident weights
+// take the staging buffer's place.
+template <bool AMAX, bool PLANES>
 __global__ void __launch_bounds__(kThreadsP, 1) k_conv1_persist(PersistParams p) {
-  static_assert(!WRES || PLANES, "resident weights take the staging buffer's place");
-  constexpr int kAStages = WRES ? kAStagesR : septfa::kAStages;
-  constexpr int kWStages = WRES ? kNCH : septfa::kWStages;
-  constexpr int kOffW = WRES ? kOffWR : septfa::kOffW;
+  constexpr int kAStages = PLANES ? kAStagesR : septfa::kAStages;
+  constexpr int kWStages = PLANES ? kNCH : septfa::kWStages;
+  constexpr int kOffW = PLANES ? kOffWR : septfa::kOffW;
   extern __shared__ __align__(1024) uint8_t smem[];
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (WRES ? kOffBarR : kOffBar));
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (PLANES ? kOffBarR : kOffBar));
   uint64_t* a_full = bars;                    // [kAStages] 256 producer arrivals
   uint64_t* a_empty = bars + 4;               // [kAStages] MMA commit
   uint64_t* w_full = bars + 8;                // [kWStages] bulk copy bytes
@@ -77,7 +77,7 @@ __global__ void __launch_bounds__(kThreadsP, 1) k_conv1_persist(PersistParams p)
   uint64_t* acc_full = bars + 14;             // [2] MMA commit
   uint64_t* acc_empty = bars + 16;            // [2] 128 epilogue arrivals
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 18);
-  float* bias_s = reinterpret_cast<float*>(smem + (WRES ? kOffBiasR : kOffBias));
+  float* bias_s = reinterpret_cast<float*>(smem + (PLANES ? kOffBiasR : kOffBias));
   constexpr uint32_t IDESC = make_idesc_f16(kTileM, 256);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -87,7 +87,7 @@ __global__ void __launch_bounds__(kThreadsP, 1) k_conv1_persist(PersistParams p)
     for (int s = 0; s < kWStages; ++s) mbar_init(w_full + s, 1);
     for (int s = 0; s < 2; ++s) { mbar_init(w_empty + s, 1); mbar_init(acc_full + s, 1); mbar_init(acc_empty + s, 128); }
     fence_mbar_init();
-    if constexpr (WRES) {   // static weights: the whole image, once, before the dependency wait
+    if constexpr (PLANES) {   // static weights: the whole image, once, before the dependency wait
       for (int j = 0; j < kNCH; ++j) {
         mbar_expect_tx(w_full + j, kWBytes);
         bulk_copy_g2s(smem + kOffW + j * kWBytes, reinterpret_cast<const uint8_t*>(p.w_img) + (size_t)j * kWBytes, kWBytes, w_full + j);
@@ -241,7 +241,7 @@ __global__ void __launch_bounds__(kThreadsP, 1) k_conv1_persist(PersistParams p)
     if constexpr (!PLANES) bulk_wait_read_all();
   } else if (warp == 12) {
     // ------------------------------------------------------------ weight loader
-    if (!WRES && lane == 0) {
+    if (!PLANES && lane == 0) {
       int g = 0;
       for (int tile = first; tile < p.ntiles; tile += stride) {
         for (int j = 0; j < kNCH; ++j, ++g) {
@@ -261,8 +261,8 @@ __global__ void __launch_bounds__(kThreadsP, 1) k_conv1_persist(PersistParams p)
         const int buf = lt & 1, ub = lt >> 1;
         if (ub > 0) { mbar_wait(acc_empty + buf, (ub - 1) & 1, 600); tc_fence_after(); }
         for (int j = 0; j < kNCH; ++j, ++ga, ++gw) {
-          const int sa = ga % kAStages, ua = ga / kAStages, sw = WRES ? j : gw % kWStages, uw = WRES ? 0 : gw / kWStages;
-          if (!WRES || lt == 0) mbar_wait(w_full + sw, uw & 1, 200 + j);
+          const int sa = ga % kAStages, ua = ga / kAStages, sw = PLANES ? j : gw % kWStages, uw = PLANES ? 0 : gw / kWStages;
+          if (!PLANES || lt == 0) mbar_wait(w_full + sw, uw & 1, 200 + j);
           mbar_wait(a_full + sa, ua & 1, 300 + j);
           tc_fence_after();
           const uint64_t a_desc = make_sw128_desc(smem_u32(smem + kOffA + sa * kABytes));
@@ -271,7 +271,7 @@ __global__ void __launch_bounds__(kThreadsP, 1) k_conv1_persist(PersistParams p)
           for (int kk = 0; kk < 4; ++kk)
             umma_f16(tmem_base + (uint32_t)(buf * 256), a_desc + (uint64_t)(kk * 2), b_desc + (uint64_t)(kk * 2), IDESC, (j | kk) != 0);
           umma_commit(a_empty + sa);
-          if constexpr (!WRES) umma_commit(w_empty + sw);
+          if constexpr (!PLANES) umma_commit(w_empty + sw);
         }
         umma_commit(acc_full + buf);
       }
@@ -292,12 +292,10 @@ cudaError_t conv1_persist_setup() {
   int dev = 0;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&g_sm_count, cudaDevAttrMultiProcessorCount, dev);
-  cudaError_t e = cudaFuncSetAttribute(k_conv1_persist<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_conv1_persist<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_conv1_persist<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_conv1_persist<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_conv1_persist<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytesR);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_conv1_persist<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytesR);
+  cudaError_t e = cudaFuncSetAttribute(k_conv1_persist<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_conv1_persist<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_conv1_persist<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytesR);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_conv1_persist<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytesR);
   return e;
 }
 
@@ -309,15 +307,12 @@ bool launch_conv1_persist(const Conv1Params& c, cudaStream_t st) {
   p.w_img = c.w_img; p.in = c.w_in; p.norm = c.norm; p.bias = c.bias_f; p.slope = c.slope;
   p.out = reinterpret_cast<__half*>(c.p_out); p.st_out = c.st_p; p.Mp = c.Mp;
   const dim3 grid(std::min(g_sm_count, p.ntiles));
-  if (c.planes && ctx().conv1_wres) {
-    if (c.slope <= 1.f) launch_k(k_conv1_persist<true, true, true>, grid, dim3(kThreadsP), kSmemBytesR, st, true, p);
-    else launch_k(k_conv1_persist<false, true, true>, grid, dim3(kThreadsP), kSmemBytesR, st, true, p);
-  } else if (c.planes) {
-    if (c.slope <= 1.f) launch_k(k_conv1_persist<true, true, false>, grid, dim3(kThreadsP), kSmemBytes, st, true, p);
-    else launch_k(k_conv1_persist<false, true, false>, grid, dim3(kThreadsP), kSmemBytes, st, true, p);
+  if (c.planes) {
+    if (c.slope <= 1.f) launch_k(k_conv1_persist<true, true>, grid, dim3(kThreadsP), kSmemBytesR, st, true, p);
+    else launch_k(k_conv1_persist<false, true>, grid, dim3(kThreadsP), kSmemBytesR, st, true, p);
   } else {
-    if (c.slope <= 1.f) launch_k(k_conv1_persist<true, false, false>, grid, dim3(kThreadsP), kSmemBytes, st, true, p);
-    else launch_k(k_conv1_persist<false, false, false>, grid, dim3(kThreadsP), kSmemBytes, st, true, p);
+    if (c.slope <= 1.f) launch_k(k_conv1_persist<true, false>, grid, dim3(kThreadsP), kSmemBytes, st, true, p);
+    else launch_k(k_conv1_persist<false, false>, grid, dim3(kThreadsP), kSmemBytes, st, true, p);
   }
   return true;
 }

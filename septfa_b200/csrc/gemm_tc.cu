@@ -30,7 +30,6 @@ constexpr int kStgPitch = 36;               // floats per staged row (32 + 4 pad
 
 struct TcParams {
   int M, T, B;
-  int late_trigger;            // MODE 1: let the dependent grid (a persistent kernel) launch only when this CTA's main loop is done
   const __half* w_img;
   const __half* w_img_lo;   // MODE 2 / SPLIT: low part of the fp16 split of the weights
   const void* in;           // [M,256] fp32 (MODE 0/2, and MODE 1 when !H16) or fp16 (MODE 1 with H16)
@@ -146,7 +145,9 @@ __global__ void __launch_bounds__(kThreads, SPLIT ? 1 : 2) k_tc_gemm(TcParams p)
     fence_mbar_init();
   }
   if (warp == 9) tmem_alloc(tmem_slot, 256);
-  if (!(MODE == 1 && p.late_trigger)) pdl_launch_dependents();
+  // MODE 1 (dconv) does not trigger its dependents: its successor is a persistent grid, which must not take SM slots
+  // this grid's second wave still needs (resid_fused.cu)
+  if (MODE != 1) pdl_launch_dependents();
   if (MODE == 1) {
     // folded depthwise taps (static weights): staged before waiting for the previous kernel; the global image already
     // has the shared-memory layout (consecutive c8 = consecutive 16 B: conflict-free LDS.128 across a warp)
@@ -685,8 +686,6 @@ void launch_mode(const TcParams& p, int ntiles_n, cudaStream_t st) {
 
 }  // namespace
 
-// The dconv kernel's successor is a persistent grid: it may become resident only when every dconv CTA is past its main
-// loop (trigger at the start of the epilogue), otherwise it takes SM slots from the dconv grid's second wave.
 #ifdef SEPTFA_TIMELINE
 long long* g_tl_conv1 = nullptr;  // bring-up timeline of one conv1 launch
 #endif
@@ -762,7 +761,6 @@ void launch_tc_dconv(const DconvParams& c, cudaStream_t st) {
   p.slope2 = c.slope2; p.dil = c.dil; p.st_q = c.st_q;
   p.out = c.racc; p.out_stride = kC; p.rowsum = c.rowsum; p.colsum = c.colsum;
   p.dbg = c.dbg;
-  p.late_trigger = ctx().dconv_late_trigger;
   if (c.split) {   // split-precision operands, fp32 p and racc
     if (c.slope2 <= 1.f) launch_mode<1, false, true, true>(p, 1, st); else launch_mode<1, false, false, true>(p, 1, st);
   } else if (c.slope2 <= 1.f) {

@@ -399,7 +399,7 @@ __global__ void __launch_bounds__(kPersistThreads, 4) k_resid_persist(FusedParam
 }  // namespace
 
 // Programmatic early launch of the persistent cluster kernel: only safe because its predecessor (the dconv kernel)
-// triggers its dependents late, at the start of each CTA's epilogue. With the usual trigger at kernel entry the
+// does not trigger its dependents, so they launch as its CTAs exit. With the usual trigger at kernel entry the
 // persistent grid became resident while the dconv grid's second wave still needed the SM slots (5.86 vs 5.09 ms per
 // step); with the late trigger the early launch hides the launch latency instead (3.75 -> 3.70 ms).
 
@@ -481,7 +481,7 @@ static void launch_cluster(K kernel, const FusedParams& p, int nclusters, int cs
   at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
-  cfg.numAttrs = (ctx().use_pdl && ctx().fused_pdl && ctx().dconv_late_trigger) ? 2 : 1;
+  cfg.numAttrs = ctx().use_pdl ? 2 : 1;
   cudaLaunchKernelEx(&cfg, kernel, p);
   ++ctx().launches;
 }

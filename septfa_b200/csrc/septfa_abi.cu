@@ -32,9 +32,7 @@ struct DevBlock {
   const __half* w1_img; const __half* w1_img_lo; const __half* w3_img_lo; const float* w1_t; const float* b1; const float* b1f; float a1; const float* g1; const float* be1;
   const float4* w2b; const float4* w2f; const float* c2f; float a2; int dil;
   const float4* wtab; const float* bog;   // tcgen05 dconv producer: pair-ordered tap table, beta1 / gamma1
-  const uint8_t* tap_img2;   // dconv_mma2.cu: per-rank halves of the tap matrices
-  const uint8_t* tap_img; const float4* swc; const float* w16; bool mma_ok;   // tensor-core depthwise kernel (dconv_mma.cu)
-  alignas(64) CUtensorMap w3_tmap; bool tmap_ok;   // res_out weight image as a TMA tensor
+  const uint8_t* tap_img2; const float4* swc; const float* w16; bool mma_ok;   // tensor-core depthwise kernel (dconv_mma2.cu)
   const __half* w3_img; const float* w3_t; const float* s3_tc; const float* s3_ref; const float* c03;
   TfParams tf;
   const float* lf_g; const float* lf_b; const float* ls_g; const float* ls_b;  // recursive
@@ -264,31 +262,6 @@ std::vector<double> split_lo(const std::vector<double>& w) {
   return lo;
 }
 
-// CUtensorMap over a pre-swizzled weight image of `rows` x 64 halves (128-byte rows): box = 256 rows = one 32 KB K-chunk,
-// copied verbatim (no TMA swizzle: the image already has the operand layout). The encoder comes from the driver through
-// the runtime's entry-point query, so nothing links against libcuda.
-bool make_weight_tmap(CUtensorMap* out, const void* gptr, int rows) {
-  typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                               const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                               CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-  static EncodeFn fn = nullptr;
-  if (!fn) {
-    void* sym = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &sym, cudaEnableDefault, &qres) != cudaSuccess || sym == nullptr) {
-      cudaGetLastError();
-      return false;
-    }
-    fn = reinterpret_cast<EncodeFn>(sym);
-  }
-  const cuuint64_t dims[2] = {64, (cuuint64_t)rows};
-  const cuuint64_t strides[1] = {128};
-  const cuuint32_t box[2] = {64, 256};
-  const cuuint32_t estr[2] = {1, 1};
-  return fn(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(gptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 // CUtensorMap over the fp16 residual stream [rows][256]: box = 64 halves x 128 rows with the 128-byte swizzle, i.e. one
 // K-chunk of a 128-frame tile lands in shared memory as a K-major SWIZZLE_128B tcgen05 operand (rows past `rows`: zeros).
 bool make_stream_tmap(CUtensorMap* out, const void* gptr, int64_t rows, int box_rows = 128, bool f32 = false) {
@@ -423,15 +396,6 @@ int septfa_create(septfa_handle** out, const septfa_config* cfg, int device) {
   h->nblk = c.layer * c.stack;
   h->ln_mode = c.apply_recursive_ln ? LN_RECURSIVE : (c.apply_residual_ln ? LN_RESIDUAL : LN_NONE);  // model.py:347-352
   build_keys(h);
-  // environment overrides of the kernel-selection switches, read once per handle (same names as septfa_set_option)
-  if (const char* e = getenv("SEPTFA_PDL")) h->lctx.use_pdl = atoi(e) ? 1 : 0;
-  if (const char* e = getenv("SEPTFA_FUSED_RESID")) h->fused_resid = atoi(e) ? 1 : 0;
-  if (const char* e = getenv("SEPTFA_CONV1_PERSIST")) h->lctx.conv1_persist = atoi(e) ? 1 : 0;
-  if (const char* e = getenv("SEPTFA_DCONV_LATE_TRIGGER")) h->lctx.dconv_late_trigger = atoi(e) ? 1 : 0;
-  if (const char* e = getenv("SEPTFA_FUSED_PDL")) h->lctx.fused_pdl = atoi(e) ? 1 : 0;
-  if (const char* e = getenv("SEPTFA_DCONV_MMA")) h->lctx.dconv_mma = atoi(e) ? 1 : 0;
-  if (const char* e = getenv("SEPTFA_DCONV_CLUSTER")) h->lctx.dconv_cluster = atoi(e) == 2 ? 2 : 1;
-  if (const char* e = getenv("SEPTFA_DCONV_DESC_SWAP")) h->lctx.dconv_desc_swap = atoi(e) ? 1 : 0;
   if (cudaSetDevice(device) != cudaSuccess) { delete h; return fail(nullptr, SEPTFA_E_CUDA, "cudaSetDevice failed"); }
   cudaDeviceGetAttribute(&h->sm_count, cudaDevAttrMultiProcessorCount, device);
   cudaError_t e = tc_gemm_setup();
@@ -440,7 +404,6 @@ int septfa_create(septfa_handle** out, const septfa_config* cfg, int device) {
   if (e == cudaSuccess) e = conv1_tma_setup();
   if (e == cudaSuccess) e = conv1_pair_setup();
   if (e == cudaSuccess) e = dconv_mma2_setup();
-  if (e == cudaSuccess) e = dconv_mma_setup();
   if (e != cudaSuccess) { delete h; return fail(nullptr, SEPTFA_E_CUDA, std::string("tc_gemm_setup: ") + cudaGetErrorString(e)); }
   *out = h;
   return 0;
@@ -514,10 +477,6 @@ int septfa_set_option(septfa_handle* h, const char* name, int value) {
     h->lctx.stream_half = value ? 1 : 0;
     return 0;
   }
-  if (std::strcmp(name, "conv1_wres") == 0) {
-    h->lctx.conv1_wres = value ? 1 : 0;
-    return 0;
-  }
   if (std::strcmp(name, "fused_resid") == 0) {
     h->fused_resid = value ? 1 : 0;
     return 0;
@@ -532,22 +491,6 @@ int septfa_set_option(septfa_handle* h, const char* name, int value) {
   }
   if (std::strcmp(name, "l2_discard") == 0) {
     h->lctx.l2_discard = value ? 1 : 0;
-    return 0;
-  }
-  if (std::strcmp(name, "dconv_pair") == 0) {
-    h->lctx.dconv_pair = value ? 1 : 0;
-    return 0;
-  }
-  if (std::strcmp(name, "dconv_w_tmap") == 0) {
-    h->lctx.dconv_w_tmap = value ? 1 : 0;
-    return 0;
-  }
-  if (std::strcmp(name, "dconv_cluster") == 0) {
-    h->lctx.dconv_cluster = value == 2 ? 2 : 1;
-    return 0;
-  }
-  if (std::strcmp(name, "dconv_desc_swap") == 0) {   // bring-up switch of dconv_mma.cu
-    h->lctx.dconv_desc_swap = value ? 1 : 0;
     return 0;
   }
   if (std::strcmp(name, "precision") == 0) {
@@ -714,13 +657,14 @@ int septfa_commit_weights(septfa_handle* h) {
         if (upload(h, tab, &tptr) || upload(h, bog, &d.bog)) return SEPTFA_E_CUDA;
         d.wtab = reinterpret_cast<const float4*>(tptr);
       }
-      // dconv_mma.cu: the depthwise conv as block-diagonal tensor-core GEMMs. Group gi = input channels 16 gi .. +15 ->
-      // outputs 32 gi .. +31; per tap k a B operand [32 outputs][16 inputs] (fp16, K-major, no swizzle: core matrices of
-      // 8 rows x 16 B, the two K halves 512 B apart) with B[n][n / 2] = fp16(w[o][k] * gamma1[o / 2]) and zeros elsewhere.
+      // dconv_mma2.cu: the depthwise conv as block-diagonal tensor-core GEMMs. Group gi = input channels 16 gi .. +15 ->
+      // outputs 32 gi .. +31; per tap k a B operand [32 outputs][16 inputs] with B[n][n / 2] = fp16(w[o][k] * gamma1[o / 2])
+      // and zeros elsewhere, split along the outputs into the halves the two CTAs of a pair hold: per rank [16 outputs][16
+      // inputs] (fp16, K-major, no swizzle: core matrices of 8 rows x 16 B, the two K halves 256 B apart).
       // The kernel's affine uses the SAME rounded taps (sw = their sum, c2f = b2 + beta / gamma * sw), so the result is
       // an exact depthwise conv with the effective weights fp16(w gamma) / gamma.
       {
-        std::vector<uint8_t> img(kDconvTapBytes, 0), img2(kDconvTapBytes, 0);
+        std::vector<uint8_t> img2(kDconvTapBytes, 0);
         std::vector<float> swc(4 * 256), w16(3 * kH);
         bool ok = true;
         for (int cch = 0; cch < kC; ++cch) ok = ok && std::isfinite(g1v[cch]) && std::fabs(g1v[cch]) >= 1e-3f;
@@ -734,8 +678,6 @@ int septfa_commit_weights(septfa_handle* h) {
             w16[k * kH + o] = fq;
             sw += (double)fq;
             const int gi = o / 32, n = o % 32, kk = (o / 2) % 16;
-            const size_t byte = (size_t)((gi * 3 + k) * 1024) + (size_t)(kk / 8) * 512 + (size_t)n * 16 + (size_t)(kk % 8) * 2;
-            std::memcpy(img.data() + byte, &hq, 2);
             // pair layout: [rank = n / 16][group][tap][K half][16 outputs][8 inputs]
             const size_t byte2 = (size_t)(n / 16) * (kDconvTapBytes / 2) + (size_t)((gi * 3 + k) * 512) + (size_t)(kk / 8) * 256 +
                                  (size_t)(n % 16) * 16 + (size_t)(kk % 8) * 2;
@@ -746,7 +688,7 @@ int septfa_commit_weights(septfa_handle* h) {
           swc[(o / 2) * 4 + 2 + (o & 1)] = (float)((double)b2[o] + bogv * sw);
         }
         const float* sp = nullptr;
-        if (upload(h, img2, &d.tap_img2) || upload(h, img, &d.tap_img) || upload(h, swc, &sp) || upload(h, w16, &d.w16)) return SEPTFA_E_CUDA;
+        if (upload(h, img2, &d.tap_img2) || upload(h, swc, &sp) || upload(h, w16, &d.w16)) return SEPTFA_E_CUDA;
         d.swc = reinterpret_cast<const float4*>(sp);
         d.mma_ok = ok;
       }
@@ -777,7 +719,6 @@ int septfa_commit_weights(septfa_handle* h) {
           upload(h, wt, &d.w3_t) || upload(h, s3_tc, &d.s3_tc) ||
           upload(h, s3_ref, &d.s3_ref) || upload(h, c03, &d.c03))
         return SEPTFA_E_CUDA;
-      d.tmap_ok = make_weight_tmap(&d.w3_tmap, d.w3_img, 8 * 256);
     }
     d.tf.enabled = c.tf_attention;
     if (c.tf_attention) {
@@ -903,9 +844,9 @@ int septfa_forward(septfa_handle* h, const float* x, int B, int64_t L, const sep
   launch_frontend(x, B, L, T, h->win_fwd, h->twiddle, c.activity_input_bool, h->act_k, h->act_b, h->act_a, ws.S, ws.w,
                   ws.dcg, ws.st0, spectrum, st);   // (the optional spectrum export leaves from the front end's own rows)
 
-  // Tensor-core depthwise kernel (dconv_mma.cu): p travels as K-group planes; its halo slots must read as zeros.
+  // Tensor-core depthwise kernel (dconv_mma2.cu): p travels as K-group planes; its halo slots must read as zeros.
   const bool planes = half_io && T >= 128 && h->lctx.conv1_persist && h->lctx.dconv_mma && h->all_mma_ok;
-  const int Mp = (M + 255) / 256 * 256 + 2 * kPlaneHalo;   // whole tile PAIRS (dconv_mma.cu walks its tiles in pairs)
+  const int Mp = (M + 255) / 256 * 256 + 2 * kPlaneHalo;   // whole tile PAIRS (dconv_mma2.cu walks its tiles in pairs)
   if (planes) {
     uint8_t* pb = reinterpret_cast<uint8_t*>(ws.p);
     CUDA_TRY(h, cudaMemset2DAsync(pb, (size_t)Mp * 16, 0, (size_t)kPlaneHalo * 16, 32, st));
@@ -919,8 +860,6 @@ int septfa_forward(septfa_handle* h, const float* x, int B, int64_t L, const sep
   const bool stream_half = planes && h->lctx.stream_half && h->ln_mode == LN_RECURSIVE && h->fused_resid && resid_fused_cluster_size(T) > 0 && h->nblk > 1;
   alignas(64) CUtensorMap wh_tmap;
   if (stream_half && !make_stream_tmap(&wh_tmap, ws.wh, M)) return fail(h, SEPTFA_E_CUDA, "cuTensorMapEncodeTiled failed for the fp16 stream");
-  // CTA-pair dconv kernel (dconv_mma2.cu): cta_group::2 MMAs, res_out weights resident in shared memory
-  const bool pair = planes && h->lctx.dconv_pair;
   // TF32 CTA-pair conv1 (gemm_conv1_pair.cu) for blocks 1 .. n-1: the fp32 stream is its A operand, fetched by TMA
   // (from ~2.5 tiles per SM on: each of its CTAs first loads 128 KB of weights, which 1-2 tiles do not pay back - measured
   // at 64 / 128 / 256 x 4 s: +0.06 / +0.03 / -0.055 ms per forward against the persistent producer kernel; option value 2
@@ -930,7 +869,7 @@ int septfa_forward(septfa_handle* h, const float* x, int B, int64_t L, const sep
   alignas(64) CUtensorMap w32_tmap;
   if (c1pair && !make_stream_tmap(&w32_tmap, ws.w, M, 128, true)) return fail(h, SEPTFA_E_CUDA, "cuTensorMapEncodeTiled failed for the fp32 stream");
   alignas(64) CUtensorMap racc_tmap;   // the pair kernel's epilogue stores racc with TMA tensor stores (boxes of 32 rows x 64 columns)
-  if (pair && !make_stream_tmap(&racc_tmap, ws.racc, M, 32)) return fail(h, SEPTFA_E_CUDA, "cuTensorMapEncodeTiled failed for racc");
+  if (planes && !make_stream_tmap(&racc_tmap, ws.racc, M, 32)) return fail(h, SEPTFA_E_CUDA, "cuTensorMapEncodeTiled failed for racc");
   const double inv_n = 1.0 / ((double)kC * T);
   StreamNorm norm{ws.st0, h->ln_g, h->ln_b, 1e-8f, inv_n};  // TCN.LN, model.py:333
   for (int i = 0; i < h->nblk; ++i) {
@@ -969,11 +908,9 @@ int septfa_forward(septfa_handle* h, const float* x, int B, int64_t L, const sep
     }
 #endif
     if (planes) {
-      DconvMmaParams dm{reinterpret_cast<const __half*>(ws.p), Mp, st_p, d.tap_img, d.tap_img2, d.swc, d.w16, d.bog, d.a2, d.dil, M, T, B, d.w3_img, d.tmap_ok ? &d.w3_tmap : nullptr,
-                        reinterpret_cast<__half*>(ws.racc), ws.rowsum, colsum, st_q};
-      dm.racc_tmap = pair ? &racc_tmap : nullptr;
-      dm.discard = h->lctx.l2_discard;
-      if (pair) launch_dconv_mma2(dm, st); else launch_dconv_mma(dm, st);
+      DconvMmaParams dm{reinterpret_cast<const __half*>(ws.p), Mp, st_p, d.tap_img2, d.swc, d.w16, d.bog, d.a2, d.dil, M, T, B, d.w3_img,
+                        reinterpret_cast<__half*>(ws.racc), ws.rowsum, colsum, st_q, &racc_tmap, h->lctx.l2_discard};
+      launch_dconv_mma2(dm, st);
     } else if (tc_dconv) {
       launch_tc_dconv(dc, st);
     } else {

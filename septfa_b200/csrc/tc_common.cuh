@@ -59,19 +59,11 @@ __device__ __forceinline__ void bulk_copy_g2s(void* dst, const void* src, uint32
                : "memory");
 }
 
-// Thread-block clusters: rank of this CTA, cluster-wide barrier, multicast forms of the bulk copy and the MMA commit.
+// Thread-block clusters: rank of this CTA, cluster-wide barrier.
 __device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
 __device__ __forceinline__ void cluster_sync_all() {
   asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
   asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// One L2 read, delivered to the same shared-memory offset of every CTA in `mask`; each destination CTA's mbarrier at the
-// same offset receives the byte count (every CTA arms its own barrier with mbar_expect_tx).
-__device__ __forceinline__ void bulk_copy_g2s_mc(void* dst, const void* src, uint32_t bytes, uint64_t* bar, uint16_t mask) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::"r"(
-                   smem_u32(dst)),
-               "l"(src), "r"(bytes), "r"(smem_u32(bar)), "h"(mask)
-               : "memory");
 }
 
 // TMA bulk copy shared -> global (SASS: UBLKCP ... .S2G), tracked by the thread's bulk async-group.
@@ -103,26 +95,6 @@ __device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t a_desc, uint6
       "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-// D[tmem] (+)= A[tmem] * B[smem]^T: the A operand (M = 128 rows = 128 lanes, 16-bit elements packed two per 32-bit
-// column: element k of row m lives in lane m, column k / 2, low half for even k) comes from tensor memory.
-__device__ __forceinline__ void umma_f16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, {%5, %5, %5, %5}, p;\n\t}" ::"r"(d_tmem),
-      "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate), "r"(0u)
-      : "memory");
-}
-// 32 lanes x 16 consecutive 32-bit columns: thread i of the warp writes lane (base_lane + i).
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};" ::"r"(taddr),
-      "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]), "r"(r[10]),
-      "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
-      : "memory");
-  asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-}
 // tcgen05.ld without the wait: lets the caller keep two loads in flight (follow with tmem_ld_wait()).
 __device__ __forceinline__ void tmem_ld32_nowait(uint32_t taddr, uint32_t (&r)[32]) {
   asm volatile(
@@ -141,12 +113,6 @@ __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.
 // Arrive on an mbarrier when all previously issued tcgen05 ops of this thread have completed.
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
-}
-// The same, arriving on the mbarrier at this offset in every CTA of `mask`.
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
-               "h"(mask)
                : "memory");
 }
 // 32 lanes x 32 consecutive fp32 columns: thread i of the warp gets lane (base_lane + i).

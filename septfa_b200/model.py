@@ -118,7 +118,11 @@ class SeparationModel(nn.Module):
         self.engine = int(engine)
 
     def set_option(self, name, value):
-        """Forwarded to septfa_set_option (e.g. "dconv_persistent", "host_chunks")."""
+        """Forwarded to septfa_set_option (e.g. "precision", "host_chunks", "dconv_mma"; include/septfa.h lists them).
+        A name or value the library refuses raises SeptfaError (at once, or at the first call on a device without a
+        handle yet) and is not kept, so the model stays usable."""
+        for h in self._handles.values():
+            _lib.check(h.ptr, h.lib.septfa_set_option(h.ptr, name.encode(), int(value)))
         if not hasattr(self, "_options"):
             self._options = {}
         self._options[name] = int(value)
@@ -153,8 +157,11 @@ class SeparationModel(nn.Module):
             h.version = self._weights_version
         _lib.check(h.ptr, h.lib.septfa_set_option(h.ptr, b"engine", self.engine))
         _lib.check(h.ptr, h.lib.septfa_set_option(h.ptr, b"profile", int(getattr(self, "_profile", False))))
-        for name, value in getattr(self, "_options", {}).items():
-            _lib.check(h.ptr, h.lib.septfa_set_option(h.ptr, name.encode(), int(value)))
+        for name, value in list(getattr(self, "_options", {}).items()):
+            rc = h.lib.septfa_set_option(h.ptr, name.encode(), int(value))
+            if rc != 0:
+                del self._options[name]
+                _lib.check(h.ptr, rc)
         return h
 
     # -- forward ---------------------------------------------------------------------------

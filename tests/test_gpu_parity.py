@@ -562,11 +562,12 @@ def test_precision_modes(cuda_models):
     m.set_option("precision", 0)
 
 
-@pytest.mark.parametrize("B,L", [(3, 64000), (2, 40000), (1, 200000), (5, 33000)])
+@pytest.mark.parametrize("B,L", [(3, 64000), (2, 40000), (1, 200000), (5, 33000), (1, 33024), (7, 48000)])
 def test_tensor_core_depthwise_kernel_equals_cuda_core_producer(cuda_models, B, L):
-    """dconv_mma.cu (depthwise conv as block-diagonal tcgen05 GEMMs on the plane layout of p, edge rows corrected) against
-    gemm_tc.cu MODE 1 (depthwise conv on the CUDA cores) on the same buffers: same network up to the fp16 rounding of
-    the folded taps; run-to-run bit-reproducible; and both within the band of the oracle."""
+    """dconv_mma2.cu (depthwise conv as block-diagonal tcgen05 GEMMs on the plane layout of p, edge rows corrected; CTA
+    pairs with the res_out weights resident) against gemm_tc.cu MODE 1 (depthwise conv on the CUDA cores) on the same
+    buffers: same network up to the fp16 rounding of the folded taps; even and odd tile counts, utterance boundaries
+    inside tiles, a tile pair with an empty tile; run-to-run bit-reproducible; and both within the band of the oracle."""
     from oracle import septfa_oracle as O
     args = synth.CONFIG_WITH_VAD
     m = cuda_models(args, 34, 0)
@@ -589,32 +590,22 @@ def test_tensor_core_depthwise_kernel_equals_cuda_core_producer(cuda_models, B, 
     assert np.abs(v1.cpu().numpy() - ref_vad).max() < 1e-3
 
 
-@pytest.mark.parametrize("B,L", [(3, 64000), (2, 40000), (1, 200000), (5, 33000), (1, 33024), (7, 48000)])
-def test_pair_dconv_kernel_equals_single_cta_kernel(cuda_models, B, L):
-    """dconv_mma2.cu (CTA pairs, cta_group::2 MMAs, res_out weights resident in shared memory, edge warp, TMA tensor stores)
-    against dconv_mma.cu (one CTA per tile, weight stream) on the same buffers: same arithmetic up to the association of the
-    edge corrections and the fp16 partial sums of the column means; even and odd tile counts, utterance boundaries inside
-    tiles, a tile pair with an empty tile; run-to-run bit-reproducible; both within the band of the oracle."""
-    from oracle import septfa_oracle as O
-    args = synth.CONFIG_WITH_VAD
-    m = cuda_models(args, 34, 0)
-    xh = synth.make_mixtures(B, L, 781)
-    x = torch.from_numpy(xh).cuda()
-    try:
-        m.set_option("dconv_pair", 0)
-        o0, v0, _ = m(x, {})
-        m.set_option("dconv_pair", 1)
-        o1, v1, _ = m(x, {})
-        o2, v2, _ = m(x, {})
-    finally:
-        m.set_option("dconv_pair", 1)
-    tail = (L % 256) if (L % 256) > 200 else 0     # samples only the last frame covers: overlap-add envelope ~1e-8 (SURVEY A.10)
-    assert (o1 - o0)[..., :L - tail].abs().max().item() < 5e-4
-    assert (v1 - v0).abs().max().item() < 1e-3
-    assert torch.equal(o1, o2) and torch.equal(v1, v2)
-    W = O.OracleWeights(synth.make_state_dict_numpy(args, 34), args, np.float64)
-    _, ref_vad, _, _ = O.forward(xh, W, {})
-    assert np.abs(v1.cpu().numpy() - ref_vad).max() < 1e-3
+def test_retired_kernel_switches_are_refused():
+    """Kernel-selection switches that only selected a path slower on every measured workload are gone:
+    septfa_set_option refuses their names as unknown options (SEPTFA_E_INVALID), the model does not keep a refused
+    name, and its forward is unchanged afterwards."""
+    from conftest import build_cuda_model
+    from septfa_b200.lib import SeptfaError
+    m = build_cuda_model(synth.CONFIG_WITH_VAD, 34)   # not the shared cache: the options below go to this model only
+    x = torch.from_numpy(synth.make_mixtures(2, 64000, 785)).cuda()
+    o0, v0, _ = m(x, {})
+    for name in ("dconv_pair", "dconv_w_tmap", "dconv_cluster", "dconv_desc_swap", "conv1_wres", "dconv_late_trigger",
+                 "fused_pdl"):
+        for value in (0, 1, 2):
+            with pytest.raises(SeptfaError, match=f"^septfa error -1: unknown option {name}$"):
+                m.set_option(name, value)
+    o1, v1, _ = m(x, {})
+    assert torch.equal(o0, o1) and torch.equal(v0, v1)
 
 
 @pytest.mark.parametrize("B,L", [(3, 64000), (1, 200000), (5, 33000)])

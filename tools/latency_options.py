@@ -23,7 +23,7 @@ def p50(x):
         ts.append(e0.elapsed_time(e1))
     return sorted(ts)[20]
 
-opts = [("default", None, None)] + [(f"{n}={v}", n, v) for n, v in (("dconv_pair", 0), ("dconv_mma", 0), ("conv1_pair", 2), ("conv1_wres", 0), ("fused_resid", 0))]
+opts = [("default", None, None)] + [(f"{n}={v}", n, v) for n, v in (("dconv_mma", 0), ("conv1_pair", 2), ("fused_resid", 0))]
 for B in (1, 8, 32):
     x = torch.from_numpy(synth.make_mixtures(B, 64000, 1)).cuda()
     line = []

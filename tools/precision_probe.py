@@ -16,8 +16,8 @@ for wseed in (0, 9):
         x = synth.make_mixtures(2, 64000, xseed)
         ref_out, ref_vad, _, _ = O.forward(x, W, dict(kw))
         xt = torch.from_numpy(x).cuda()
-        for opts in ({}, {"dconv_pair": 0}, {"dconv_mma": 0}, {"precision": 2}, {"engine": 7}):
-            for k, v in {"dconv_pair": 1, "dconv_mma": 1, "precision": 0}.items(): m.set_option(k, v)
+        for opts in ({}, {"dconv_mma": 0}, {"precision": 2}, {"engine": 7}):
+            for k, v in {"dconv_mma": 1, "precision": 0}.items(): m.set_option(k, v)
             m.engine = 0
             for k, v in opts.items():
                 if k == "engine": m.engine = v
