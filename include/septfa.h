@@ -248,7 +248,8 @@ int septfa_online_hops_done(const septfa_online* st);
  * of range) is refused with SEPTFA_E_INVALID before anything is launched. A push that returns an error leaves every slot
  * unchanged. Per slot the session keeps on the device a hop counter, the last W - H input samples and the last W - H
  * emitted samples of both speakers (12 (W - H) + 4 bytes: ~384 KB at the default). Pushes and releases are
- * stream-ordered and do not synchronise the host; issue all calls of a session on one stream. hops: device [n, H];
+ * stream-ordered and do not synchronise the host; issue all calls of a session on one stream. hops: device [n, Hn] (Hn = H
+ * at 16 kHz, see septfa_live_create_rate);
  * out: device [n, 2, H]; out_vad: device [n, 2, F]; perm: device int32 [n, 2]; the workspace is sized by
  * septfa_live_workspace_bytes for pushes of up to n slots. */
 #define SEPTFA_LIVE_HOP 16000
@@ -256,6 +257,18 @@ int septfa_online_hops_done(const septfa_online* st);
 typedef struct septfa_live septfa_live;
 int septfa_live_create(septfa_handle* h, int capacity, septfa_live** out);
 int septfa_live_create_win(septfa_handle* h, int capacity, int window, int hop, septfa_live** out);
+/* A session whose streams arrive at `rate` Hz (septfa_resample_geometry's rates; septfa_live_create_win is this with
+ * rate 16000). Push k of a stream carries Hn = H rate / 16000 native samples (septfa_live_input_hop); the hop H must be a
+ * multiple of the rate's hop_multiple. The session resamples each stream on the device, carrying the history from push
+ * to push, and then serves the 16 kHz stream u = concat(D zeros, septfa_resample(stream)) exactly as a 16 kHz session
+ * would: push k returns u[H k, H (k + 1)), its permutation and VAD frames. D (0 at 16000) is the delay of the streaming
+ * resampler: the outputs of a push before (k + 1) H - D need no native sample after the hop. So the output lags the
+ * input by D extra samples (6 .. 12 at the rates in the table of septfa_resample_geometry); a caller aligning output with
+ * input shifts by D. Per slot the session keeps 2 x (at most 2 width + orig) more floats; a new stream reads none of
+ * them. At 16000 nothing is added and a push launches what it launched before. */
+int septfa_live_create_rate(septfa_handle* h, int capacity, int window, int hop, int rate, septfa_live** out);
+/* Hn, the native samples per push; *delay (nullable) receives D. */
+int septfa_live_input_hop(const septfa_live* lv, int* delay);
 void septfa_live_destroy(septfa_live* lv);
 /* F, the VAD frames per push; *first_frame (nullable) receives j0. */
 int septfa_live_vad_frames(const septfa_live* lv, int* first_frame);
@@ -275,6 +288,22 @@ int septfa_pit_l1(septfa_handle* h, const float* a, const float* b, int S, int64
  * to numpy; a constant signal gives NaN like the reference). x, out: device [B, L]; lengths (nullable, device int64 [B]):
  * valid samples per utterance for ragged batches - extrema over the valid part, zeros written behind it. */
 int septfa_minmax_normalize(septfa_handle* h, const float* x, int B, int64_t L, const int64_t* lengths, float* out, void* stream);
+
+/* Resampling to 16 kHz: torchaudio.functional.resample(x, rate, 16000) with its defaults (sinc_interp_hann,
+ * lowpass_filter_width 6, rolloff 0.99), what read_mixture applies through transforms.Resample (only_inference.py:68-79).
+ * Accepted rates: integers in [8000, 192000] Hz; anything else is refused with SEPTFA_E_INVALID. With g = gcd(rate,
+ * 16000), orig = rate / g, new = 16000 / g, output m = b new + p is the fp32 FMA chain over the taps of phase p of a
+ * polyphase bank computed in double on the host and stored as fp32, keeping only the taps whose scaled time |t| < 6
+ * (torchaudio's taps beyond are ~1e-20 or smaller): within ~4e-7 of float64 torchaudio on inputs in [-0.9, 0.9].
+ * septfa_resample_geometry needs no handle and no device: *delay (nullable) receives D, the delay in 16 kHz samples of
+ * a streaming resampler fed in hops (septfa_live_create_rate), and *hop_multiple (nullable) receives `new`, which a live
+ * hop must be a multiple of. D is 12 at 8000 Hz, 8 at 11025 and 12000 Hz and 6 at 22050 .. 192000 Hz. */
+int septfa_resample_geometry(int rate, int* delay, int* hop_multiple);
+/* x: device [B, L] at `rate` Hz, x_fmt SEPTFA_FMT_F32 (float32) or SEPTFA_FMT_PCM16 (int16 PCM, converted as
+ * astype(float32), only_inference.py:69: no scaling); out: device float32 [B, ceil(16000 L / rate)]. Rate 16000 is the
+ * identity. The first call at a rate builds its bank, uploads it and waits for the upload; later calls at that rate are
+ * stream-ordered and do not synchronise the host. */
+int septfa_resample(septfa_handle* h, const void* x, int x_fmt, int B, int64_t L, int rate, float* out, void* stream);
 
 /* calc_sisdr (model/combined_loss.py:16-56): SI-SDR in dB of `rows` pairs preds[rows, n] / target[rows, n] (device,
  * float32, contiguous) in one pass; out_db device [rows]; scratch: device, rows * 5 doubles; rows <= 65535. Runs on the

@@ -9,7 +9,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libseptfa.so")
-SOURCES = ["frontend.cu", "tcn.cu", "gemm_tc.cu", "gemm_conv1_persist.cu", "gemm_conv1_tma.cu", "gemm_conv1_pair.cu", "dconv_mma2.cu", "resid_fused.cu", "backend.cu", "preproc.cu", "online.cu", "live.cu", "septfa_abi.cu"]
+SOURCES = ["frontend.cu", "tcn.cu", "gemm_tc.cu", "gemm_conv1_persist.cu", "gemm_conv1_tma.cu", "gemm_conv1_pair.cu", "dconv_mma2.cu", "resid_fused.cu", "backend.cu", "preproc.cu", "online.cu", "live.cu", "resample.cu", "septfa_abi.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--use_fast_math=false"]
 

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <cuda_fp16.h>
 #include <stdint.h>
+#include <vector>
 #include "common.cuh"
 
 namespace septfa {
@@ -248,6 +249,32 @@ void launch_live_pit_emit(const int32_t* slots, int n, int32_t* hops_done, const
                           const float* vad /*[n,2,T]*/, int T, float* tail_ring, float* out /*[n,2,H]*/,
                           float* out_vad /*[n,2,F] or null*/, int32_t* perm /*[n,2]*/, LiveGeom g, cudaStream_t st);
 void launch_live_release(const int32_t* slots_host, int n, int32_t* hops_done, cudaStream_t st);
+
+// ---- resampling to 16 kHz (resample.cu)
+constexpr int kResampleRate = 16000;
+constexpr int kResampleMinRate = 8000, kResampleMaxRate = 192000;
+constexpr int kResampleTile = 512;   // outputs per CTA
+// What a rate needs, computed on the host from the bank's effective support.
+struct ResamplePlan {
+  int orig, nw;        // rate / g, 16000 / g with g = gcd(rate, 16000)
+  int ntaps;           // taps stored per phase (the longest effective run; shorter ones are zero-padded)
+  int delay;           // D: 16 kHz samples a live stream lags by
+  int hist;            // native samples a live push reads from before its hop
+  int tile_span;       // native samples one tile of kResampleTile outputs reads (shared memory floats)
+};
+struct ResampleBank {
+  const float* taps;   // [ntaps][nw] fp32, tap i of phase p at i * nw + p
+  const int2* span;    // [nw] {first j - width, tap count} of each phase
+  int orig, nw, delay, hist, tile_span;
+};
+// false for a rate outside [8000, 192000]; taps / spans (nullable) receive the bank
+bool resample_plan(int rate, ResamplePlan* plan, std::vector<float>* taps, std::vector<int2>* spans);
+int64_t resample_out_len(int rate, int64_t L);
+void launch_resample(const void* x, bool pcm16, int B, int64_t L, int64_t L16, float* out, const ResampleBank& bk,
+                     cudaStream_t st);
+void launch_live_resample(const int32_t* slots, int n, const int32_t* hops_done, float* hist /*[cap][2][hist]*/,
+                          const float* hops /*[n,Hn]*/, float* u /*[n,H]*/, const ResampleBank& bk, int H, int Hn,
+                          cudaStream_t st);
 
 // Per-handle launch state (septfa_handle owns one; every C-ABI entry binds it to the calling thread before launching).
 struct LaunchCtx {

@@ -93,6 +93,10 @@ struct septfa_handle {
   int ev_used = 0;
   double prof_ms[SEPTFA_PROF_NCAT] = {0};
   int prof_launches[SEPTFA_PROF_NCAT] = {0};
+  // resampling filter banks by input rate, and their device memory: kept apart from `allocs`, which a weight commit
+  // frees, since live sessions and later calls hold the bank pointers until septfa_destroy
+  std::map<int, ResampleBank> banks;
+  std::vector<void*> bank_allocs;
 };
 
 struct septfa_graph {
@@ -120,6 +124,10 @@ struct septfa_live {
   int32_t* hops_done = nullptr;   // [capacity] hops pushed by the slot's current stream (0: no history is read)
   float* in_ring = nullptr;       // [capacity][W - H] the last W - H input samples, sample s at position s mod (W - H)
   float* tail_ring = nullptr;     // [capacity][2][W - H] the last W - H emitted samples of both speakers, the same way
+  int rate = kResampleRate;       // input rate; other than 16000: each push is resampled first
+  int in_hop = 0;                 // Hn = H rate / 16000 native samples per push
+  ResampleBank bank{};            // the handle's bank for `rate`
+  float* hist = nullptr;          // [capacity][2][bank.hist] native history, double-buffered by hop parity
 };
 
 namespace {
@@ -141,6 +149,13 @@ int check_geometry(septfa_handle* h, int W, int H) {
   if (W < 2 * (int64_t)H) return fail(h, SEPTFA_E_INVALID, g + "the window must be >= 2 hops");
   if (W > kMaxWinLen) return fail(h, SEPTFA_E_INVALID, g + "the window must be <= 160000 samples (10 s)");
   if (W % 16 || H % 16) return fail(h, SEPTFA_E_INVALID, g + "window and hop must be multiples of 16 samples (1 ms)");
+  return 0;
+}
+
+// An input rate the resampler accepts: an integer in [8000, 192000] Hz.
+int check_rate(septfa_handle* h, int rate, ResamplePlan* plan) {
+  if (!resample_plan(rate, plan, nullptr, nullptr))
+    return fail(h, SEPTFA_E_INVALID, "rate " + std::to_string(rate) + ": the input rate must lie in 8000 .. 192000 Hz");
   return 0;
 }
 
@@ -232,6 +247,30 @@ int upload(septfa_handle* h, const std::vector<T>& src, const T** dst) {
   h->allocs.push_back(d);
   CUDA_TRY(h, cudaMemcpy(d, src.data(), src.size() * sizeof(T), cudaMemcpyHostToDevice));
   *dst = reinterpret_cast<const T*>(d);
+  return 0;
+}
+
+// The handle's bank for `rate` (checked by the caller), built and uploaded at the first call for that rate. The upload
+// is waited for, so the bank can be used on any stream afterwards; later calls find it in the cache.
+int get_bank(septfa_handle* h, int rate, cudaStream_t st, ResampleBank* out) {
+  auto it = h->banks.find(rate);
+  if (it != h->banks.end()) { *out = it->second; return 0; }
+  ResamplePlan pl{};
+  std::vector<float> taps;
+  std::vector<int2> spans;
+  resample_plan(rate, &pl, &taps, &spans);
+  float* dt = nullptr;
+  int2* ds = nullptr;
+  CUDA_TRY(h, cudaMalloc(reinterpret_cast<void**>(&dt), taps.size() * sizeof(float)));
+  h->bank_allocs.push_back(dt);
+  CUDA_TRY(h, cudaMalloc(reinterpret_cast<void**>(&ds), spans.size() * sizeof(int2)));
+  h->bank_allocs.push_back(ds);
+  CUDA_TRY(h, cudaMemcpyAsync(dt, taps.data(), taps.size() * sizeof(float), cudaMemcpyHostToDevice, st));
+  CUDA_TRY(h, cudaMemcpyAsync(ds, spans.data(), spans.size() * sizeof(int2), cudaMemcpyHostToDevice, st));
+  CUDA_TRY(h, cudaStreamSynchronize(st));
+  const ResampleBank bk{dt, ds, pl.orig, pl.nw, pl.delay, pl.hist, pl.tile_span};
+  h->banks[rate] = bk;
+  *out = bk;
   return 0;
 }
 
@@ -414,6 +453,7 @@ void septfa_destroy(septfa_handle* h) {
   bind_ctx(nullptr);
   cudaSetDevice(h->device);
   for (void* p : h->allocs) cudaFree(p);
+  for (void* p : h->bank_allocs) cudaFree(p);
   cudaFree(h->norm_ext);
   cudaFree(h->hx_dev); cudaFree(h->hout_dev); cudaFree(h->hvad_dev); cudaFree(h->hws); cudaFree(h->hws_b); cudaFree(h->pit_acc);
   if (h->slot_compute) { cudaStreamSynchronize(h->slot_compute); cudaStreamDestroy(h->slot_compute); }
@@ -1344,6 +1384,7 @@ struct LiveWorkspace {
   float* win;       // [n, W]
   float* pred;      // [n, 2, W]
   float* vad;       // [n, 2, T(W)]
+  float* u;         // [n, H] the resampled hops (sessions at a rate other than 16000)
   void* fws;        // the forward's workspace
   size_t fws_bytes;
   size_t total;
@@ -1358,6 +1399,7 @@ LiveWorkspace live_carve(const septfa_live* lv, uintptr_t base, int n) {
   w.win = reinterpret_cast<float*>(base + off);     off += al((size_t)n * W * sizeof(float));
   w.pred = reinterpret_cast<float*>(base + off);    off += al((size_t)n * 2 * W * sizeof(float));
   w.vad = reinterpret_cast<float*>(base + off);     off += al((size_t)n * 2 * septfa_num_frames(W) * sizeof(float));
+  if (lv->rate != kResampleRate) { w.u = reinterpret_cast<float*>(base + off); off += al((size_t)n * lv->g.hop * sizeof(float)); }
   w.fws = reinterpret_cast<void*>(base + off);
   w.fws_bytes = septfa_workspace_bytes(lv->h, n, W);
   w.total = off + w.fws_bytes;
@@ -1393,23 +1435,48 @@ int septfa_live_create(septfa_handle* h, int capacity, septfa_live** out) {
 }
 
 int septfa_live_create_win(septfa_handle* h, int capacity, int window, int hop, septfa_live** out) {
+  return septfa_live_create_rate(h, capacity, window, hop, kResampleRate, out);
+}
+
+int septfa_live_create_rate(septfa_handle* h, int capacity, int window, int hop, int rate, septfa_live** out) {
   if (!h || !out || capacity < 1 || capacity > 32767)
     return fail(h, SEPTFA_E_INVALID, "bad arguments (1 <= capacity <= 32767 slots per live session)");
   *out = nullptr;
   if (int rc = check_geometry(h, window, hop)) { h->last_launches = 0; return rc; }
+  ResamplePlan pl{};
+  if (int rc = check_rate(h, rate, &pl)) { h->last_launches = 0; return rc; }
+  if (hop % pl.nw) {   // a push must carry a whole number of native samples
+    h->last_launches = 0;
+    return fail(h, SEPTFA_E_INVALID, "rate " + std::to_string(rate) + ", hop " + std::to_string(hop) +
+                                         ": the hop must be a multiple of " + std::to_string(pl.nw) + " samples at this rate");
+  }
+  const int in_hop = (int)((int64_t)hop * pl.orig / pl.nw);
+  if (pl.hist > in_hop) {
+    h->last_launches = 0;
+    return fail(h, SEPTFA_E_INVALID, "rate " + std::to_string(rate) + ", hop " + std::to_string(hop) +
+                                         ": the resampler's history exceeds one hop");
+  }
   if (!h->committed) return fail(h, SEPTFA_E_STATE, "weights not committed");
   CUDA_TRY(h, cudaSetDevice(h->device));
+  ResampleBank bank{};
+  if (rate != kResampleRate)
+    if (int rc = get_bank(h, rate, nullptr, &bank)) return rc;
   auto* lv = new septfa_live();
   lv->h = h;
   lv->capacity = capacity;
+  lv->rate = rate;
+  lv->in_hop = in_hop;
+  lv->bank = bank;
   const int first = (window - hop + 255) / 256;   // the first window frame whose centre 256 j lies in [W - H, W)
   lv->g = LiveGeom{window, hop, first, (window + 255) / 256 - first};
   const size_t ring_b = (size_t)(window - hop) * sizeof(float);
+  const size_t hist_b = (size_t)capacity * 2 * std::max(bank.hist, 1) * sizeof(float);
   if (cudaMalloc(reinterpret_cast<void**>(&lv->hops_done), (size_t)capacity * sizeof(int32_t)) != cudaSuccess ||
       cudaMalloc(reinterpret_cast<void**>(&lv->in_ring), (size_t)capacity * ring_b) != cudaSuccess ||
       cudaMalloc(reinterpret_cast<void**>(&lv->tail_ring), (size_t)capacity * 2 * ring_b) != cudaSuccess ||
+      (rate != kResampleRate && cudaMalloc(reinterpret_cast<void**>(&lv->hist), hist_b) != cudaSuccess) ||
       cudaMemset(lv->hops_done, 0, (size_t)capacity * sizeof(int32_t)) != cudaSuccess) {
-    cudaFree(lv->hops_done); cudaFree(lv->in_ring); cudaFree(lv->tail_ring);
+    cudaFree(lv->hops_done); cudaFree(lv->in_ring); cudaFree(lv->tail_ring); cudaFree(lv->hist);
     delete lv;
     return fail(h, SEPTFA_E_CUDA, "live session allocation failed");
   }
@@ -1420,8 +1487,14 @@ int septfa_live_create_win(septfa_handle* h, int capacity, int window, int hop, 
 void septfa_live_destroy(septfa_live* lv) {
   if (!lv) return;
   cudaSetDevice(lv->h->device);
-  cudaFree(lv->hops_done); cudaFree(lv->in_ring); cudaFree(lv->tail_ring);
+  cudaFree(lv->hops_done); cudaFree(lv->in_ring); cudaFree(lv->tail_ring); cudaFree(lv->hist);
   delete lv;
+}
+
+int septfa_live_input_hop(const septfa_live* lv, int* delay) {
+  if (!lv) return SEPTFA_E_INVALID;
+  if (delay) *delay = lv->rate == kResampleRate ? 0 : lv->bank.delay;
+  return lv->in_hop;
 }
 
 size_t septfa_live_workspace_bytes(const septfa_live* lv, int n) {
@@ -1463,6 +1536,10 @@ int septfa_live_push(septfa_live* lv, const int32_t* slots_host, int n, const fl
   CUDA_TRY(h, cudaMemcpyAsync(ws.slots, slots_host, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
   bind_ctx(&h->lctx);
   ctx().launches = 0;
+  if (lv->rate != kResampleRate) {
+    launch_live_resample(ws.slots, n, lv->hops_done, lv->hist, hops, ws.u, lv->bank, lv->g.hop, lv->in_hop, st);
+    hops = ws.u;
+  }
   launch_live_window(ws.slots, n, lv->hops_done, lv->in_ring, hops, ws.win, lv->g, st);
   const int before = ctx().launches;
   if (int rc = septfa_forward(h, ws.win, n, lv->g.win, kw, ws.pred, ws.vad, nullptr, nullptr, nullptr, nullptr, ws.fws,
@@ -1506,6 +1583,39 @@ int septfa_minmax_normalize(septfa_handle* h, const float* x, int B, int64_t L, 
   bind_ctx(&h->lctx);
   launch_minmax_normalize(x, B, L, lengths, h->norm_ext, out, reinterpret_cast<cudaStream_t>(stream));
   h->last_launches = 3;
+  CUDA_TRY(h, cudaGetLastError());
+  return 0;
+}
+
+int septfa_resample_geometry(int rate, int* delay, int* hop_multiple) {
+  ResamplePlan pl{};
+  if (int rc = check_rate(nullptr, rate, &pl)) return rc;
+  if (delay) *delay = pl.delay;
+  if (hop_multiple) *hop_multiple = pl.nw;
+  return 0;
+}
+
+int septfa_resample(septfa_handle* h, const void* x, int x_fmt, int B, int64_t L, int rate, float* out, void* stream) {
+  if (!h) return SEPTFA_E_INVALID;
+  h->last_launches = 0;
+  if (!x || !out || B < 1 || B > 65535 || L < 1) return fail(h, SEPTFA_E_INVALID, "bad arguments (1 <= B <= 65535, L >= 1)");
+  if (x_fmt != SEPTFA_FMT_F32 && x_fmt != SEPTFA_FMT_PCM16)
+    return fail(h, SEPTFA_E_INVALID, "x_fmt must be SEPTFA_FMT_F32 or SEPTFA_FMT_PCM16");
+  ResamplePlan pl{};
+  if (int rc = check_rate(h, rate, &pl)) return rc;
+  CUDA_TRY(h, cudaSetDevice(h->device));
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const int64_t L16 = resample_out_len(rate, L);
+  if (rate == kResampleRate && x_fmt == SEPTFA_FMT_F32) {
+    CUDA_TRY(h, cudaMemcpyAsync(out, x, (size_t)B * L * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    return 0;
+  }
+  ResampleBank bk{};
+  if (int rc = get_bank(h, rate, st, &bk)) return rc;
+  bind_ctx(&h->lctx);
+  ctx().launches = 0;
+  launch_resample(x, x_fmt == SEPTFA_FMT_PCM16, B, L, L16, out, bk, st);
+  h->last_launches = ctx().launches;
   CUDA_TRY(h, cudaGetLastError());
   return 0;
 }

@@ -128,22 +128,39 @@ def save_vad(vad_output, save_path):
             plt.close()
 
 
+def _first_channel(audio):
+    """read_mixture's channel choice (only_inference.py:70-72)."""
+    return audio[0] if audio.shape[1] > audio.shape[0] else audio[:, 0]
+
+
 def separate_files(model, paths, save_dir, inference_kw=None, precision_save=32, device=0, batch=64):
-    """The file loop either side of the forward (SURVEY.md section 8(f) rank 1), batched: 16-bit mono 16 kHz wav files of
-    EQUAL length are grouped into batches; each batch travels to the device as int16 PCM, is converted and min-max
-    normalised there (only_inference.py:69,81, bit-identical to numpy), separated, and comes back as float32 or - for
-    ``precision_save=16`` - float16, three batches in flight (forward_host_stream). Other files (stereo, other rates or
-    sample formats) take the single-file path of :func:`read_mixture`. Writes ``<stem>_Speaker_{0,1}.wav`` into
-    ``save_dir`` (float32 wav, or 16-bit PCM for precision 16) and returns ``{path: vad [2, T]}``."""
+    """The file loop either side of the forward (SURVEY.md section 8(f) rank 1), batched: 16-bit wav files of EQUAL
+    length and rate are grouped into batches. 16 kHz mono batches travel to the device as int16 PCM, are converted and
+    min-max normalised there (only_inference.py:69,81, bit-identical to numpy), separated, and come back as float32 or -
+    for ``precision_save=16`` - float16, three batches in flight (forward_host_stream). 16-bit files at another rate in
+    8 .. 192 kHz, and 16-bit stereo files at 16 kHz, are batched on the device in the reference's order: astype, resample
+    to 16 kHz (SeparationModel.resample; the identity at 16 kHz), normalise, forward. Stereo files are reduced to the first
+    channel as read_mixture does. These files do not go through read_mixture, so its notes on stereo and resampled input
+    are not printed for them. Other files (float wav, rates outside that range) take the single-file path of
+    :func:`read_mixture`. Writes ``<stem>_Speaker_{0,1}.wav`` into ``save_dir`` (float32 wav, or 16-bit PCM for precision
+    16) and returns ``{path: vad [2, T]}``."""
+    from .lib import RESAMPLE_MAX_RATE, RESAMPLE_MIN_RATE
     from scipy.io.wavfile import read, write
     Path(save_dir).mkdir(parents=True, exist_ok=True)
     kw = copy.deepcopy(DEFAULT_INFERENCE_KW)
     kw.update(inference_kw or {})
-    groups, singles = {}, []
+    groups, rate_groups, singles = {}, {}, []
     for pth in paths:
         sr, audio = read(pth)
         if sr == 16000 and audio.ndim == 1 and audio.dtype == np.int16 and len(audio) >= 257:
             groups.setdefault(len(audio), []).append((pth, audio))
+        elif (RESAMPLE_MIN_RATE <= sr <= RESAMPLE_MAX_RATE and audio.dtype == np.int16 and audio.ndim in (1, 2)
+              and audio.size):
+            a = np.ascontiguousarray(audio if audio.ndim == 1 else _first_channel(audio))
+            if -(-16000 * len(a) // sr) >= 257:
+                rate_groups.setdefault((sr, len(a)), []).append((pth, a))
+            else:
+                singles.append(pth)
         else:
             singles.append(pth)
     out_dtype = torch.float16 if precision_save == 16 else torch.float32
@@ -164,6 +181,17 @@ def separate_files(model, paths, save_dir, inference_kw=None, precision_save=32,
         for ch, (out, vad) in zip(chunks, model.forward_host_stream(batches, kw, device=device, out_dtype=out_dtype, reuse_outputs=True)):
             for i, (pth, _) in enumerate(ch):
                 emit(pth, out[i], vad[i].clone() if torch.is_tensor(vad) else None)
+    dev = torch.device("cuda", device)
+    for (sr, _), items in sorted(rate_groups.items()):
+        for i in range(0, len(items), batch):
+            ch = items[i:i + batch]
+            x = torch.from_numpy(np.stack([a for _, a in ch])).to(dev)
+            with torch.no_grad():
+                out, vad, _ = model(model.minmax_normalize(model.resample(x, sr)), kw)
+            out = out.to(out_dtype).cpu()
+            vad = vad.cpu() if torch.is_tensor(vad) else None
+            for j, (pth, _) in enumerate(ch):
+                emit(pth, out[j], vad[j].clone() if vad is not None else None)
     for pth in singles:
         x = read_mixture(pth).to(torch.device("cuda", device))
         with torch.no_grad():

@@ -100,12 +100,16 @@ _PROTOS = {
     "septfa_online_hops_done": (C.c_int, [C.c_void_p]),
     "septfa_live_create": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]),
     "septfa_live_create_win": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
+    "septfa_live_create_rate": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
+    "septfa_live_input_hop": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "septfa_live_destroy": (None, [C.c_void_p]),
     "septfa_live_vad_frames": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "septfa_live_workspace_bytes": (C.c_size_t, [C.c_void_p, C.c_int]),
     "septfa_live_release": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "septfa_live_push": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.POINTER(InferKw), C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "septfa_resample_geometry": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "septfa_resample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_void_p, C.c_void_p]),
     "septfa_minmax_normalize": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "septfa_sisdr": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "septfa_pit_l1": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p,
@@ -143,3 +147,17 @@ PROF_NAMES = ("frontend", "conv1", "dconv", "gate", "resid", "outconv", "vad", "
 
 def num_frames(L):
     return 1 + int(L) // 256
+
+
+RESAMPLE_MIN_RATE, RESAMPLE_MAX_RATE = 8000, 192000   # input rates septfa_resample accepts
+
+
+def resample_geometry(rate):
+    """``(delay, hop_multiple)`` of ``rate`` from septfa_resample_geometry (no device needed): the delay D in 16 kHz
+    samples of a streaming resampler, and the number a live hop at that rate must be a multiple of. Raises SeptfaError
+    for a rate the library refuses."""
+    lib = load()
+    d, m = C.c_int(), C.c_int()
+    rc = lib.septfa_resample_geometry(int(rate), C.byref(d), C.byref(m))
+    check(None, rc)
+    return d.value, m.value

@@ -9,28 +9,42 @@ of a stream of N pushes equals ``OnlineSaving.calc_online(F.pad(x, (W - H, 0)))`
 ``save_sec = H / 16000`` on that stream alone (the windowing of ``model/online_class_known_targets.py:92-93``, the
 stitch of ``model/online_class_unknown_targets.py:84-94``). The oldest sample of a hop comes back about H samples after
 it was taken, plus the push time: the hop sets the latency.
+
+A session at another input ``rate`` (8 .. 192 kHz) takes ``input_hop = hop * rate / 16000`` native samples per push and
+resamples each stream on the device (``septfa_live_create_rate``), carrying the resampler's history from push to push.
+It then serves the 16 kHz stream ``u = concat(delay zeros, resample(x))``: the output lags the input by ``delay``
+samples (6 .. 12, see ``septfa_resample_geometry``) on top of the hop.
 """
 from __future__ import annotations
 
 import ctypes as C
+import math
 
 import numpy as np
 import torch
 
 from . import lib as _lib
 
+RATE = 16000             # the model's rate, and the default input rate
 WINDOW = 48000
 HOP = 16000              # the default hop
 FRAMES_PER_HOP = 63      # VAD frames per push at the default geometry
 MAX_WINDOW = 160000      # 10 s
 
 
-def check_geometry(window, hop):
+def check_geometry(window, hop, rate=RATE):
     """``(window, hop)`` as ints if the library accepts them: 256 <= hop, 2 hop <= window <= 160000, both multiples of 16
-    samples (1 ms); ``ValueError`` otherwise."""
-    if not all(isinstance(v, (int, np.integer)) and not isinstance(v, bool) for v in (window, hop)):
-        raise ValueError(f"window and hop are integer sample counts, got {window!r}, {hop!r}")
-    window, hop = int(window), int(hop)
+    samples (1 ms); ``rate`` an integer in 8000 .. 192000 Hz, and the hop a multiple of ``16000 / gcd(rate, 16000)`` so
+    that a push carries a whole number of native samples (160 at 44.1 kHz, any hop at 48 kHz). ``ValueError``
+    otherwise."""
+    if not all(isinstance(v, (int, np.integer)) and not isinstance(v, bool) for v in (window, hop, rate)):
+        raise ValueError(f"window, hop and rate are integers, got {window!r}, {hop!r}, {rate!r}")
+    window, hop, rate = int(window), int(hop), int(rate)
+    if not _lib.RESAMPLE_MIN_RATE <= rate <= _lib.RESAMPLE_MAX_RATE:
+        raise ValueError(f"rate = {rate}: must lie in {_lib.RESAMPLE_MIN_RATE} .. {_lib.RESAMPLE_MAX_RATE} Hz")
+    step = RATE // math.gcd(rate, RATE)
+    if hop % step:
+        raise ValueError(f"rate = {rate}, hop = {hop}: the hop must be a multiple of {step} samples at this rate")
     if hop < 256:
         raise ValueError(f"hop = {hop}: must be >= 256 samples")
     if window < 2 * hop:
@@ -60,22 +74,25 @@ def check_slots(slots, capacity):
 class LiveSession:
     """``capacity`` stream slots on one device, for a :class:`~septfa_b200.model.SeparationModel`.
 
-    Every stream has a window of ``window`` and a hop of ``hop`` samples (see :func:`check_geometry`).
-    ``push(slots, hops)`` takes one hop (``hop`` float32 samples, already normalised) for each listed slot and returns
+    Every stream has a window of ``window`` and a hop of ``hop`` samples at 16 kHz and arrives at ``rate`` Hz (see
+    :func:`check_geometry`). ``push(slots, hops)`` takes one hop (``input_hop`` float32 samples at ``rate``, already
+    normalised) for each listed slot and returns
     ``(out [n, 2, hop], vad [n, 2, frames_per_hop] or None, perm [n, 2] int32)`` on the device, stream-ordered on the
     current stream. ``vad`` holds the window frames ``first_frame .. first_frame + frames_per_hop - 1`` of the window's
     VAD output, those centred on the new hop (frame j centred on window sample ``256 j``; 125 .. 187 at the default),
     speakers in the emitted order; it is None for a model without a VAD head or with ``vad=False``. ``release(slots)``
     ends the streams in those slots: the next push into one starts a new stream. ``inference_kw`` is the forward's
-    (gating, smoothed VAD), fixed for the session.
+    (gating, smoothed VAD), fixed for the session. At a rate other than 16000 the outputs are those of a 16 kHz session
+    fed ``concat(delay zeros, model.resample(stream))``; ``delay`` is 0 at 16000.
     """
 
-    def __init__(self, model, capacity, inference_kw=None, device=None, window=WINDOW, hop=HOP):
+    def __init__(self, model, capacity, inference_kw=None, device=None, window=WINDOW, hop=HOP, rate=RATE):
         self.model = model
         self.capacity = int(capacity)
         if not 1 <= self.capacity <= 32767:
             raise ValueError("capacity must lie in 1 .. 32767")
-        self.window, self.hop = check_geometry(window, hop)
+        self.window, self.hop = check_geometry(window, hop, rate)
+        self.rate = int(rate)
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         if self.device.type != "cuda":
             raise RuntimeError("septfa_b200.LiveSession runs on CUDA only (no CPU fallback)")
@@ -83,8 +100,11 @@ class LiveSession:
         self._lv = C.c_void_p()
         with torch.cuda.device(self.device):
             self._h = model._handle(self.device)
-            _lib.check(self._h.ptr, self._h.lib.septfa_live_create_win(self._h.ptr, self.capacity, self.window, self.hop,
-                                                                       C.byref(self._lv)))
+            _lib.check(self._h.ptr, self._h.lib.septfa_live_create_rate(self._h.ptr, self.capacity, self.window, self.hop,
+                                                                        self.rate, C.byref(self._lv)))
+            delay = C.c_int()
+            self.input_hop = self._h.lib.septfa_live_input_hop(self._lv, C.byref(delay))
+            self.delay = delay.value
             j0 = C.c_int()
             self.frames_per_hop = self._h.lib.septfa_live_vad_frames(self._lv, C.byref(j0))
             self.first_frame = j0.value
@@ -100,8 +120,8 @@ class LiveSession:
         n = ids.size
         if not (isinstance(hops, torch.Tensor) and hops.is_cuda and hops.dtype == torch.float32):
             raise ValueError("hops must be a CUDA float32 tensor")
-        if tuple(hops.shape) != (n, self.hop):
-            raise ValueError(f"hops must have shape ({n}, {self.hop}), got {tuple(hops.shape)}")
+        if tuple(hops.shape) != (n, self.input_hop):
+            raise ValueError(f"hops must have shape ({n}, {self.input_hop}), got {tuple(hops.shape)}")
         if hops.device != self.device:
             raise ValueError(f"hops are on {hops.device}, the session on {self.device}")
         hops = hops.contiguous()

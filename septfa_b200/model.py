@@ -272,6 +272,26 @@ class SeparationModel(nn.Module):
             _lib.check(h.ptr, rc)
         return out
 
+    def resample(self, x: torch.Tensor, rate):
+        """torchaudio.functional.resample(x, rate, 16000) on the device (septfa_resample), batched: ``x [B, L]`` is a CUDA
+        float32 tensor, or int16 PCM converted as ``astype(float32)`` (no scaling); returns float32
+        ``[B, ceil(16000 L / rate)]``. ``rate``: an integer in 8000 .. 192000 Hz; 16000 returns the input values."""
+        assert x.ndim == 2 and x.is_cuda and x.dtype in (torch.float32, torch.int16)
+        if isinstance(rate, bool) or int(rate) != rate:
+            raise ValueError(f"rate must be an integer number of Hz, got {rate!r}")
+        rate = int(rate)
+        x = x.contiguous()
+        B, L = x.shape
+        x_fmt = _lib.FMT_PCM16 if x.dtype == torch.int16 else _lib.FMT_F32
+        out = torch.empty((B, max(-(-16000 * L // rate), 0) if rate > 0 else 0), dtype=torch.float32, device=x.device)
+        with torch.cuda.device(x.device):
+            h = self._handle(x.device)
+            rc = h.lib.septfa_resample(h.ptr, C.c_void_p(x.data_ptr()), x_fmt, B, L, rate, C.c_void_p(out.data_ptr()),
+                                       C.c_void_p(torch.cuda.current_stream(x.device).cuda_stream))
+            _lib.check(h.ptr, rc)
+            self.last_launch_count = h.lib.septfa_last_launch_count(h.ptr)
+        return out
+
     def forward_host_submit(self, x_host: torch.Tensor, inference_kw={}, device=0, slot=0, out=None, vad=None,
                             out_dtype=torch.float32):
         """Asynchronous half of :meth:`forward_host` (septfa_forward_host_submit_fmt): enqueue copy-in, forward and

@@ -10,7 +10,12 @@ bench.py at the default). The two legs alternate step by step; each call is time
 synchronisations, on its own. realtime_streams = capacity * (hop / 16000) / push p99: the streams one GPU keeps up
 with when it does nothing but push.
 
-    python tools/live_bench.py [--capacity 1024 --steps 60 --warmup 10c --window 48000 --hop 16000] --out FILE.json
+With --rate R (other than 16000) a third leg pushes the same schedule into a session at R Hz (septfa_live_create_rate):
+every hop carries hop * R / 16000 native samples of seeded mixtures, which the session resamples on the device before
+the same window / forward / emit. The three legs alternate step by step; the record adds the rate leg's push times and
+its overhead over the 16 kHz push.
+
+    python tools/live_bench.py [--capacity 1024 --steps 60 --warmup 10c --window 48000 --hop 16000 --rate 48000] --out FILE.json
 """
 import argparse
 import contextlib
@@ -51,6 +56,7 @@ def main():
     ap.add_argument("--warmup", type=int, default=None, help="untimed steps first (default 10c; >= 7c: every slot has started)")
     ap.add_argument("--window", type=int, default=48000, help="window W in samples")
     ap.add_argument("--hop", type=int, default=16000, help="hop H in samples")
+    ap.add_argument("--rate", type=int, default=16000, help="input rate of a third leg (16000: no third leg)")
     ap.add_argument("--out", default=None, help="write the JSON record here too")
     a = ap.parse_args()
     W, H = a.window, a.hop
@@ -89,6 +95,14 @@ def main():
     vad = torch.empty((n, 2, n_vad), device=dev)
     perm = torch.empty((n, 2), dtype=torch.int32, device=dev)
 
+    lv_r = C.c_void_p()
+    if a.rate != FS:
+        _lib.check(h.ptr, lib.septfa_live_create_rate(h.ptr, n, W, H, a.rate, C.byref(lv_r)))
+        delay = C.c_int()
+        Hn = lib.septfa_live_input_hop(lv_r, C.byref(delay))
+        ws_r = torch.empty(lib.septfa_live_workspace_bytes(lv_r, n), dtype=torch.uint8, device=dev)
+        mixes_r = torch.from_numpy(synth.make_mixtures(32, max_hops * Hn, 4322)).to(dev).view(32, max_hops, Hn)
+
     st = C.c_void_p()
     _lib.check(h.ptr, lib.septfa_online_create_win(h.ptr, n, W, H, C.byref(st)))
     ws_on = torch.empty(lib.septfa_online_workspace_bytes(st), dtype=torch.uint8, device=dev)
@@ -106,11 +120,14 @@ def main():
         return e0.elapsed_time(e1)
 
     push_ms, step_ms, ns, restarts, launches = [], [], [], [], 0
+    push_r_ms, launches_r = [], 0
     for t in range(a.warmup + a.steps):
         length = np.round((3 + (np.arange(n) + gen) % 8) * c).astype(np.int64)
         ended = np.nonzero((k == length) & (start <= t))[0].astype(np.int32)
         if ended.size:
             _lib.check(h.ptr, lib.septfa_live_release(lv, ended.ctypes.data_as(C.c_void_p), ended.size, stream))
+            if lv_r:
+                _lib.check(h.ptr, lib.septfa_live_release(lv_r, ended.ctypes.data_as(C.c_void_p), ended.size, stream))
             gen[ended] += 1
             k[ended] = 0
         slots = np.nonzero(start <= t)[0].astype(np.int32)
@@ -131,15 +148,29 @@ def main():
                                                      stream))
         tp = timed(push)
         launches = lib.septfa_last_launch_count(h.ptr)
+        if lv_r:
+            hops_r = mixes_r[mix, torch.from_numpy(k[slots]).to(dev)].contiguous()
+
+            def push_r():
+                _lib.check(h.ptr, lib.septfa_live_push(lv_r, sl, slots.size, C.c_void_p(hops_r.data_ptr()), C.byref(ikw),
+                                                       C.c_void_p(out.data_ptr()), C.c_void_p(vad.data_ptr()),
+                                                       C.c_void_p(perm.data_ptr()), C.c_void_p(ws_r.data_ptr()), ws_r.numel(),
+                                                       stream))
+            tr = timed(push_r)
+            launches_r = lib.septfa_last_launch_count(h.ptr)
         ts = timed(step)
         k[slots] += 1
         if t >= a.warmup:
             assert slots.size == n, "timed steps must push every slot"
             push_ms.append(tp)
+            if lv_r:
+                push_r_ms.append(tr)
             step_ms.append(ts)
             ns.append(int(slots.size))
             restarts.append(int(ended.size))
     lib.septfa_live_destroy(lv)
+    if lv_r:
+        lib.septfa_live_destroy(lv_r)
     lib.septfa_online_destroy(st)
 
     p50p, p50s, p99p = pct(push_ms, 0.5), pct(step_ms, 0.5), pct(push_ms, 0.99)
@@ -155,6 +186,12 @@ def main():
            "realtime_streams_at_push_p99": n * (H / FS) / (p99p / 1000.0),
            "timing": "CUDA events around one call between device synchronisations; legs alternate step by step",
            "state_bytes_per_slot": 4 + 12 * (W - H)}
+    if lv_r:
+        p50r, p99r = pct(push_r_ms, 0.5), pct(push_r_ms, 0.99)
+        rec["rate_leg"] = {"rate": a.rate, "input_hop": Hn, "delay_samples": delay.value,
+                           "push": {"p50_ms": p50r, "p99_ms": p99r, "min_ms": min(push_r_ms), "launches": launches_r},
+                           "overhead_p50_ms": p50r - p50p, "overhead_p99_ms": p99r - p99p,
+                           "realtime_streams_at_push_p99": n * (H / FS) / (p99r / 1000.0)}
     line = json.dumps(rec)
     print(line, flush=True)
     if a.out:
