@@ -195,8 +195,8 @@ int septfa_last_launch_count(const septfa_handle* h);
 #define SEPTFA_PROF_RESID 4    /* post-block GroupNorm residual kernels */
 #define SEPTFA_PROF_OUTCONV 5  /* output statistics + tcgen05 GEMM 256->514 */
 #define SEPTFA_PROF_VAD 6      /* VAD head + smoothing */
-#define SEPTFA_PROF_ISTFT 7    /* mask + inverse STFT overlap-add */
-#define SEPTFA_PROF_EXPORT 8   /* optional torch-layout exports */
+#define SEPTFA_PROF_ISTFT 7    /* mask + inverse STFT overlap-add + the optional est / mask / logits exports */
+#define SEPTFA_PROF_EXPORT 8   /* reads 0: the exports are written by the ISTFT class's kernel */
 #define SEPTFA_PROF_NCAT 9
 int septfa_profile_read(septfa_handle* h, double* ms, int* launches, int n, int reset);
 

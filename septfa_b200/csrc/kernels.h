@@ -225,10 +225,13 @@ struct VadParams {
   int do_smooth;
 };
 void launch_vad(const VadParams& p, cudaStream_t st);
+cudaError_t backend_setup();   // opt-in shared memory of the mask / iSTFT / export kernel; call once per device
 void launch_mask_istft(const float2* S, const float* logits, const float* gate /*[B,2,T] or null*/, const float* window,
                        const float2* twiddle, int B, int64_t L, int T, float* out, cudaStream_t st);
-void launch_export(const float2* S, const float* logits, const float* gate, const float* z0, const float* dc_gated,
-                   int B, int T, float2* est, float* mask, float* spectrum, float* logits_out, cudaStream_t st);
+// waveform [B,2,L]; the exports est [B,2,257,T] complex, mask [B,2,257,T], logits_out [B,514,T] are each nullable
+void launch_mask_istft_export(const float2* S, const float* logits, const float* gate /*[B,2,T] or null*/, const float* window,
+                              const float2* twiddle, int B, int64_t L, int T, float* out, float2* est, float* mask,
+                              float* logits_out, cudaStream_t st);
 // online.cu
 void launch_pit(const float* a, int64_t a_bstride, int64_t a_sstride, const float* b, int64_t b_bstride, int64_t b_sstride,
                 int S, int64_t n, double* acc /*[S,4] zeroed*/, int32_t* perm, cudaStream_t st);

@@ -443,6 +443,7 @@ int septfa_create(septfa_handle** out, const septfa_config* cfg, int device) {
   if (e == cudaSuccess) e = conv1_tma_setup();
   if (e == cudaSuccess) e = conv1_pair_setup();
   if (e == cudaSuccess) e = dconv_mma2_setup();
+  if (e == cudaSuccess) e = backend_setup();
   if (e != cudaSuccess) { delete h; return fail(nullptr, SEPTFA_E_CUDA, std::string("tc_gemm_setup: ") + cudaGetErrorString(e)); }
   *out = h;
   return 0;
@@ -1001,9 +1002,13 @@ int septfa_forward(septfa_handle* h, const float* x, int B, int64_t L, const sep
     CUDA_TRY(h, cudaMemcpyAsync(out_vad, vsrc, (size_t)M * 2 * sizeof(float), cudaMemcpyDeviceToDevice, st));
   }
   prof_mark(h, SEPTFA_PROF_ISTFT, st);
-  launch_mask_istft(ws.S, ws.logits, gate, h->win_inv, h->twiddle, B, L, T, out_wav, st);
-  prof_mark(h, SEPTFA_PROF_EXPORT, st);
-  launch_export(ws.S, ws.logits, gate, ws.w, ws.dcg, B, T, reinterpret_cast<float2*>(est_stft), mask, nullptr, logits_out, st);
+  // With any of the est / mask / logits exports, one kernel writes them and the waveform from one read of S and the logits;
+  // without them the register-prefetch kernel (3 CTAs per SM against 2) is slightly faster end to end (DESIGN.md section 3).
+  if (est_stft != nullptr || mask != nullptr || logits_out != nullptr)
+    launch_mask_istft_export(ws.S, ws.logits, gate, h->win_inv, h->twiddle, B, L, T, out_wav, reinterpret_cast<float2*>(est_stft),
+                             mask, logits_out, st);
+  else
+    launch_mask_istft(ws.S, ws.logits, gate, h->win_inv, h->twiddle, B, L, T, out_wav, st);
   prof_mark(h, -1, st);
 #ifdef SEPTFA_TIMELINE
   if (getenv("SEPTFA_FUSED_TL")) resid_fused_dump_timeline();

@@ -19,6 +19,6 @@ ncu --set full --clock-control none --import-source on -k regex:"k_frontend|k_co
 ncu --set full --clock-control none --import-source on -k regex:"k_tc_gemm" -s 3 -c 1 \
     -o $OUT/prof_outconv_${TAG} -f $PY > $OUT/ncu_outconv_${TAG}.log 2>&1
 #    back-end kernels of the 4th forward
-ncu --set full --clock-control none --import-source on -k regex:"k_out_stats|k_vad_final|k_mask_istft|k_export" -s 12 -c 4 \
+ncu --set full --clock-control none --import-source on -k regex:"k_out_stats|k_vad_final|k_mask_istft_export" -s 9 -c 3 \
     -o $OUT/prof_ends_${TAG} -f $PY > $OUT/ncu_ends_${TAG}.log 2>&1
 for f in block outconv ends; do tail -n 2 $OUT/ncu_${f}_${TAG}.log; done
