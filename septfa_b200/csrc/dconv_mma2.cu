@@ -187,14 +187,6 @@ __device__ __forceinline__ uint64_t make_ns_desc(uint32_t saddr, uint32_t lbo, u
   return d;
 }
 
-// Bring-up timeline (clock64 stamps of CTA 0's roles), compiled in only with -DSEPTFA_DM_TIMELINE.
-#ifdef SEPTFA_DM_TIMELINE
-__device__ long long g_dm2_tl[10][64];
-#define DTL(role, idx) do { if (blockIdx.x == 0 && (idx) < 64) g_dm2_tl[role][idx] = clock64(); } while (0)
-#else
-#define DTL(role, idx) do { } while (0)
-#endif
-
 template <bool AMAX>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsD, 1) k_dconv_mma2(const __grid_constant__ DmParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -257,7 +249,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsD, 1) k_dcon
   cluster_sync_all();   // (also a CTA barrier) both CTAs' mbarriers are initialised and their tensor memory is allocated
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  if (threadIdx.x == 0) DTL(9, 0);
   // the pair walks tile pairs: cluster c takes pairs c, c + nclusters, ...; rank r the tile 2 * pair + r. Both CTAs run
   // the same number of tiles (the last pair of an odd tile count has an empty tile: no valid rows, nothing stored).
   const int npairs = (p.ntiles + 1) / 2;
@@ -296,7 +287,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsD, 1) k_dcon
             discard_chunk(g - kPStages);
           }
           if (lane == 0) {
-            DTL(0, g);
             mbar_expect_tx(p_full + s, kPChunkBytes);
 #pragma unroll
             for (int kg = 0; kg < 4; ++kg)   // frames r0 - 4 .. r0 + 131 = slots r0 .. r0 + 135
@@ -419,7 +409,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsD, 1) k_dcon
         mbar_wait(p_peer + sp, up & 1, 205 + j);
         if (ub > 0) mbar_wait(d1_empty + b, (ub - 1) & 1, 210 + j);
         tc_fence_after();
-        if (lane == 0) DTL(2, gi);
         const uint32_t slab = smem_u32(smem + kOffP + sp * kPChunkBytes);
         if (elect_one()) {
 #pragma unroll
@@ -449,7 +438,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsD, 1) k_dcon
         if (lt == 0) { mbar_wait(w_full + j, 0, 230 + j); mbar_wait(w_peer + j, 0, 235 + j); }
         mbar_wait(a2_full + ba, ua & 1, 240 + j);
         tc_fence_after();
-        if (lane == 0) DTL(3, gm);
         const uint32_t a_tmem = tmem_base + 256u + (uint32_t)(ba * 64);   // q: K 0..31 at +0..15, K 32..63 at +32..47
         const uint64_t b_desc = make_sw128_desc(smem_u32(smem + kOffW + j * kWHalfBytes));
         if (elect_one()) {
@@ -531,7 +519,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsD, 1) k_dcon
         tmem_ld32_nowait(t_addr(gg, 0), va);
         tmem_ld32_nowait(t_addr(gg, 1), vb);
         tmem_ld_wait();
-        if (warp == 4 && lane == 0) DTL(4, gg);
         if (cslot >= 0) {
           // zero padding of the normalised signal: take back what the out-of-utterance tap contributed (edge warp's table)
           mbar_wait(corr_full + sp, (gg / kPStages) & 1, 310 + j);
@@ -553,12 +540,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsD, 1) k_dcon
         if (lane == 0) mbar_arrive(p_empty + sp);
         half_chunk(va, j, gg, 0);
         half_chunk(vb, j, gg, 1);
-        if (warp == 4 && lane == 0 && gg < 32) DTL(7, 32 + gg);
         tmem_st_wait();
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive_cl(a2_full + (gg % kD1Bufs), 0);   // one arrival per warp, on the leader's barrier
-        if (warp == 4 && lane == 0) DTL(5, gg);
       }
       g += 8;
       // statistics of q of this warp's 32 rows x 256 columns, per utterance: fixed-order shuffle trees, double atomics
@@ -603,7 +588,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsD, 1) k_dcon
       const int n0_w = max(0, min(nv_w, e1 - (r0 + q4 * 32)));         // ... that belong to the tile's first utterance
       mbar_wait(d2_full, lt & 1, 500);
       tc_fence_after();
-      if (warp == 12 && lane == 0) DTL(6, lt * 4);
       float2 racc2 = make_float2(0.f, 0.f);
       const uint32_t t_row = tmem_base + ((uint32_t)(q4 * 32) << 16);
       auto pack_store = [&](const uint32_t (&u)[32], int cc) {   // cc: 32-column piece within the staged half row
@@ -738,7 +722,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsD, 1) k_dcon
         keep(vb, 3);
       }
       store_half(0);   // the staged half (two boxes) leaves with one tensor store per box
-      if (warp == 12 && lane == 0) DTL(6, lt * 4 + 1);
       colsum_half(0);
       if (lane == 0) bulk_wait_read_all();   // the first half's boxes have left the staging buffer
       __syncwarp();
@@ -753,7 +736,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsD, 1) k_dcon
       store_half(1);
       colsum_half(1);
       if (valid) p.rowsum[row] = racc2.x + racc2.y;
-      if (warp == 12 && lane == 0) DTL(6, lt * 4 + 2);
     }
     if (lane == 0) bulk_wait_read_all();
     __syncwarp();
@@ -764,21 +746,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsD, 1) k_dcon
   if (warp == 2) tmem_dealloc2(tmem_base, 512);
 }
 
-int g_dm2_sm_count = 0;
-
 }  // namespace
 
-#ifdef SEPTFA_DM_TIMELINE
-extern "C" int septfa_debug_dm2_timeline(long long* out) {   // [10][64] clock64 stamps of CTA 0 of the last launch
-  cudaDeviceSynchronize();
-  return cudaMemcpyFromSymbol(out, g_dm2_tl, sizeof(long long) * 640) == cudaSuccess ? 0 : -1;
-}
-#endif
-
 cudaError_t dconv_mma2_setup() {
-  int dev = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&g_dm2_sm_count, cudaDevAttrMultiProcessorCount, dev);
   cudaError_t e = cudaFuncSetAttribute(k_dconv_mma2<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
   if (e != cudaSuccess) return e;
   return cudaFuncSetAttribute(k_dconv_mma2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
@@ -791,19 +761,9 @@ void launch_dconv_mma2(const DconvMmaParams& c, cudaStream_t st) {
   p.w_img = c.w_img; p.racc = c.racc; p.rowsum = c.rowsum; p.colsum = c.colsum; p.st_q = c.st_q;
   p.racc_tmap = *reinterpret_cast<const CUtensorMap*>(c.racc_tmap);
   const int npairs = (p.ntiles + 1) / 2;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(2 * std::min(g_dm2_sm_count / 2, npairs));
-  cfg.blockDim = dim3(kThreadsD);
-  cfg.dynamicSmemBytes = kSmemBytes;
-  cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = ctx().use_pdl ? 1 : 0;
-  if (c.slope2 <= 1.f) cudaLaunchKernelEx(&cfg, k_dconv_mma2<true>, p);
-  else cudaLaunchKernelEx(&cfg, k_dconv_mma2<false>, p);
-  ++ctx().launches;
+  const dim3 grid(2 * std::min(ctx().sm_count / 2, npairs));
+  if (c.slope2 <= 1.f) launch_k(k_dconv_mma2<true>, grid, dim3(kThreadsD), kSmemBytes, st, true, p);
+  else launch_k(k_dconv_mma2<false>, grid, dim3(kThreadsD), kSmemBytes, st, true, p);
 }
 
 }  // namespace septfa

@@ -7,8 +7,8 @@
 
 namespace septfa {
 
-// Launch context of the calling thread: every C-ABI entry binds its handle's context (kernels.h), so options such as
-// "pdl" or "conv1_persist" and the launch counter are per handle, not process-wide.
+// Launch context of the calling thread: every C-ABI entry binds its handle's context (kernels.h), so the "pdl" option,
+// the SM count and the launch counter are per handle, not process-wide.
 namespace { LaunchCtx g_default_ctx; thread_local LaunchCtx* t_ctx = nullptr; }
 LaunchCtx& ctx() { return t_ctx ? *t_ctx : g_default_ctx; }
 void bind_ctx(LaunchCtx* c) { t_ctx = c; }

@@ -291,14 +291,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsC, 1) k_conv
   if (warp == 1) tmem_dealloc2(tmem_base, 512);
 }
 
-int g_sm_count_c = 0;
-
 }  // namespace
 
 cudaError_t conv1_pair_setup() {
-  int dev = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&g_sm_count_c, cudaDevAttrMultiProcessorCount, dev);
   cudaError_t e = cudaFuncSetAttribute(k_conv1_pair<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(k_conv1_pair<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
   return e;
@@ -311,19 +306,9 @@ void launch_conv1_pair(const Conv1PairParams& c, cudaStream_t st) {
   p.w_img = c.w_img; p.sb = c.sb; p.st_in = c.norm.gamma ? c.norm.st : nullptr; p.inv_n = c.norm.inv_n; p.eps = c.norm.eps;
   p.slope = c.slope; p.out = c.p_planes; p.st_out = c.st_p;
   const int npairs = (p.ntiles + 1) / 2;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(2 * std::min(g_sm_count_c / 2, npairs));
-  cfg.blockDim = dim3(kThreadsC);
-  cfg.dynamicSmemBytes = kSmemBytes;
-  cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = ctx().use_pdl ? 1 : 0;
-  if (c.slope <= 1.f) cudaLaunchKernelEx(&cfg, k_conv1_pair<true>, p);
-  else cudaLaunchKernelEx(&cfg, k_conv1_pair<false>, p);
-  ++ctx().launches;
+  const dim3 grid(2 * std::min(ctx().sm_count / 2, npairs));
+  if (c.slope <= 1.f) launch_k(k_conv1_pair<true>, grid, dim3(kThreadsC), kSmemBytes, st, true, p);
+  else launch_k(k_conv1_pair<false>, grid, dim3(kThreadsC), kSmemBytes, st, true, p);
 }
 
 }  // namespace septfa

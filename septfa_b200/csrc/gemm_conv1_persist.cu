@@ -284,14 +284,9 @@ __global__ void __launch_bounds__(kThreadsP, 1) k_conv1_persist(PersistParams p)
   if (warp == 13) tmem_dealloc(tmem_base, 512);
 }
 
-int g_sm_count = 0;
-
 }  // namespace
 
 cudaError_t conv1_persist_setup() {
-  int dev = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&g_sm_count, cudaDevAttrMultiProcessorCount, dev);
   cudaError_t e = cudaFuncSetAttribute(k_conv1_persist<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(k_conv1_persist<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(k_conv1_persist<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytesR);
@@ -299,14 +294,12 @@ cudaError_t conv1_persist_setup() {
   return e;
 }
 
-// Returns false when the persistent kernel does not apply (caller uses the one-tile-per-CTA kernel).
-bool launch_conv1_persist(const Conv1Params& c, cudaStream_t st) {
-  if (!ctx().conv1_persist || !c.half_io || c.T < kTileM || g_sm_count <= 0) return false;
+void launch_conv1_persist(const Conv1Params& c, cudaStream_t st) {
   PersistParams p{};
   p.M = c.M; p.T = c.T; p.ntiles = (c.M + kTileM - 1) / kTileM;
   p.w_img = c.w_img; p.in = c.w_in; p.norm = c.norm; p.bias = c.bias_f; p.slope = c.slope;
   p.out = reinterpret_cast<__half*>(c.p_out); p.st_out = c.st_p; p.Mp = c.Mp;
-  const dim3 grid(std::min(g_sm_count, p.ntiles));
+  const dim3 grid(std::min(ctx().sm_count, p.ntiles));
   if (c.planes) {
     if (c.slope <= 1.f) launch_k(k_conv1_persist<true, true>, grid, dim3(kThreadsP), kSmemBytesR, st, true, p);
     else launch_k(k_conv1_persist<false, true>, grid, dim3(kThreadsP), kSmemBytesR, st, true, p);
@@ -314,7 +307,6 @@ bool launch_conv1_persist(const Conv1Params& c, cudaStream_t st) {
     if (c.slope <= 1.f) launch_k(k_conv1_persist<true, false>, grid, dim3(kThreadsP), kSmemBytes, st, true, p);
     else launch_k(k_conv1_persist<false, false>, grid, dim3(kThreadsP), kSmemBytes, st, true, p);
   }
-  return true;
 }
 
 }  // namespace septfa

@@ -58,15 +58,6 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* tmap, 
                : "memory");
 }
 
-// Bring-up timeline (globaltimer stamps, ns, of CTA 0 and the last CTA), compiled in only with -DSEPTFA_C1_TIMELINE.
-#ifdef SEPTFA_C1_TIMELINE
-__device__ unsigned long long g_c1_tl[2][64];
-__device__ __forceinline__ unsigned long long gtimer() { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }
-#define CTL(idx) do { if ((blockIdx.x == 0 || blockIdx.x == gridDim.x - 1) && (idx) < 64) g_c1_tl[blockIdx.x ? 1 : 0][idx] = gtimer(); } while (0)
-#else
-#define CTL(idx) do { } while (0)
-#endif
-
 template <bool AMAX>
 __global__ void __launch_bounds__(kThreadsT, 1) k_conv1_tma(const __grid_constant__ TmaParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -82,7 +73,6 @@ __global__ void __launch_bounds__(kThreadsT, 1) k_conv1_tma(const __grid_constan
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (threadIdx.x == 0) {
-    CTL(0);
     if ((smem_u32(smem) & 1023u) != 0u) __trap();
     for (int s = 0; s < kAStages; ++s) { mbar_init(a_full + s, 1); mbar_init(a_empty + s, 1); }
     for (int j = 0; j < kNCH; ++j) mbar_init(w_full + j, 1);
@@ -97,15 +87,12 @@ __global__ void __launch_bounds__(kThreadsT, 1) k_conv1_tma(const __grid_constan
   if (warp == 1) tmem_alloc(tmem_slot, 512);
   if (threadIdx.x < 128) reinterpret_cast<float4*>(smem + kOffSb)[threadIdx.x] = __ldg(p.sb + threadIdx.x);
   pdl_launch_dependents();
-  if (threadIdx.x == 0) CTL(1);
   pdl_wait();
-  if (threadIdx.x == 0) CTL(2);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   const int first = blockIdx.x, stride = gridDim.x;
-  if (threadIdx.x == 0) CTL(3);
 
   if (warp == 0) {
     // ------------------------------------------------------------ TMA producer (rows past M read as zeros)
@@ -130,10 +117,9 @@ __global__ void __launch_bounds__(kThreadsT, 1) k_conv1_tma(const __grid_constan
         if (ub > 0) { mbar_wait(acc_empty + buf, (ub - 1) & 1, 600); tc_fence_after(); }
         for (int j = 0; j < kNCH; ++j, ++g) {
           const int sa = g % kAStages, ua = g / kAStages;
-          if (lt == 0) { mbar_wait(w_full + j, 0, 200 + j); CTL(4 + j); }
+          if (lt == 0) mbar_wait(w_full + j, 0, 200 + j);
           mbar_wait(a_full + sa, ua & 1, 300 + j);
           tc_fence_after();
-          CTL(8 + g);
           const uint64_t a_desc = make_sw128_desc(smem_u32(smem + kOffA + sa * kABytes));
           const uint64_t b_desc = make_sw128_desc(smem_u32(smem + kOffW + j * kWBytes));
 #pragma unroll
@@ -175,7 +161,6 @@ __global__ void __launch_bounds__(kThreadsT, 1) k_conv1_tma(const __grid_constan
       const float2 rs2 = make_float2(rstd, rstd), nr2 = make_float2(-mean * rstd, -mean * rstd);
       mbar_wait(acc_full + buf, (lt >> 1) & 1, 500);
       tc_fence_after();
-      if (warp == 4 && lane == 0) CTL(32 + 2 * lt);
       float2 s2 = make_float2(0.f, 0.f), q2 = make_float2(0.f, 0.f);
       const uint32_t t_row = tmem_base + (uint32_t)(buf * 256) + ((uint32_t)(lq * 32) << 16) + (uint32_t)(ch * kEpiCols);
       auto process = [&](const uint32_t (&u)[32], int c) {
@@ -224,7 +209,6 @@ __global__ void __launch_bounds__(kThreadsT, 1) k_conv1_tma(const __grid_constan
       const float sv = valid ? s2.x + s2.y : 0.f, qv = valid ? q2.x + q2.y : 0.f;
       const float a0 = warp_sum(second ? 0.f : sv), c0 = warp_sum(second ? 0.f : qv);
       const float a1 = warp_sum(second ? sv : 0.f), c1 = warp_sum(second ? qv : 0.f);
-      if (warp == 4 && lane == 0) CTL(33 + 2 * lt);
       if (lane == 0) {
         atomicAdd(&p.st_out[b_first].s, (double)a0);
         atomicAdd(&p.st_out[b_first].ss, (double)c0);
@@ -238,25 +222,12 @@ __global__ void __launch_bounds__(kThreadsT, 1) k_conv1_tma(const __grid_constan
 
   tc_fence_before();
   __syncthreads();
-  if (threadIdx.x == 0) CTL(48);
   if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
-int g_sm_count_t = 0;
-
 }  // namespace
 
-#ifdef SEPTFA_C1_TIMELINE
-extern "C" int septfa_debug_c1_timeline(unsigned long long* out) {   // [2][64] globaltimer stamps of the last launch
-  cudaDeviceSynchronize();
-  return cudaMemcpyFromSymbol(out, g_c1_tl, sizeof(unsigned long long) * 128) == cudaSuccess ? 0 : -1;
-}
-#endif
-
 cudaError_t conv1_tma_setup() {
-  int dev = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&g_sm_count_t, cudaDevAttrMultiProcessorCount, dev);
   cudaError_t e = cudaFuncSetAttribute(k_conv1_tma<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(k_conv1_tma<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
   return e;
@@ -268,7 +239,7 @@ void launch_conv1_tma(const Conv1TmaParams& c, cudaStream_t st) {
   p.M = c.M; p.T = c.T; p.ntiles = (c.M + kTileM - 1) / kTileM; p.Mp = c.Mp;
   p.w_img = c.w_img; p.sb = c.sb; p.st_in = c.norm.gamma ? c.norm.st : nullptr; p.inv_n = c.norm.inv_n; p.eps = c.norm.eps;
   p.slope = c.slope; p.out = c.p_planes; p.st_out = c.st_p;
-  const dim3 grid(std::min(g_sm_count_t, p.ntiles));
+  const dim3 grid(std::min(ctx().sm_count, p.ntiles));
   if (c.slope <= 1.f) launch_k(k_conv1_tma<true>, grid, dim3(kThreadsT), kSmemBytes, st, true, p);
   else launch_k(k_conv1_tma<false>, grid, dim3(kThreadsT), kSmemBytes, st, true, p);
 }

@@ -44,21 +44,9 @@ struct TcParams {
   void* out; int out_stride;  // fp32, or fp16 for MODE 0/1 with H16
   Stat2* st_out;
   float* rowsum; double* colsum;
-  long long* dbg;   // optional timeline buffer (bring-up only)
 };
 
 using namespace tc;
-
-// Bring-up timeline (clock64 stamps of one CTA), compiled in only with -DSEPTFA_TIMELINE.
-#ifdef SEPTFA_TIMELINE
-__device__ unsigned long long g_cta_tl[1024 * 8];
-__device__ __forceinline__ unsigned long long gtimer_ns() { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
-#define CTL(k) do { if (MODE == 1 && threadIdx.x == 0 && blockIdx.x < 1024) g_cta_tl[blockIdx.x * 8 + (k)] = gtimer_ns(); } while (0)
-#define TLG(idx) do { if (p.dbg != nullptr && blockIdx.x == 3 && blockIdx.y == 0 && threadIdx.x == 0 && (idx) < 64) p.dbg[idx] = clock64(); } while (0)
-#else
-#define TLG(idx) do { } while (0)
-#define CTL(k) do { } while (0)
-#endif
 
 __device__ __forceinline__ float4 ld_half4(const __half* p) {   // 4 consecutive halves (8 B) -> float4
   const uint2 v = __ldg(reinterpret_cast<const uint2*>(p));
@@ -120,7 +108,6 @@ __global__ void __launch_bounds__(kThreads, SPLIT ? 1 : 2) k_tc_gemm(TcParams p)
   float4* wB_s = wA_s + 256;                                                                  // {wz_a, wz_b, sw_a, sw_b}
   float2* wC_s = reinterpret_cast<float2*>(wB_s + 256);                                       // {c2f_a, c2f_b}
 
-  CTL(0);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   // MODE 2 (three N-tiles per M-tile): a 1-D grid with the N-tile index fastest, so that the three CTAs that read the
   // same 128 rows of the stream run next to each other and the second and third read hit the L2 (with the M-tile index
@@ -153,9 +140,7 @@ __global__ void __launch_bounds__(kThreads, SPLIT ? 1 : 2) k_tc_gemm(TcParams p)
     // has the shared-memory layout (consecutive c8 = consecutive 16 B: conflict-free LDS.128 across a warp)
     for (int i = threadIdx.x; i < kDconvWBytes / 16; i += kThreads) wA_s[i] = __ldg(p.wtab + i);
   }
-  CTL(1);
   pdl_wait();   // everything below reads what earlier kernels of the chain wrote
-  CTL(2);
   {
     const double inv_n = 1.0 / ((double)kC * p.T);
     for (int i = threadIdx.x; i < nseg; i += kThreads) {
@@ -175,8 +160,6 @@ __global__ void __launch_bounds__(kThreads, SPLIT ? 1 : 2) k_tc_gemm(TcParams p)
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  TLG(0);
-  CTL(3);
 
   if (warp == 8) {
     // ------------------------------------------------------------ weight loader (TMA bulk copies)
@@ -265,7 +248,6 @@ __global__ void __launch_bounds__(kThreads, SPLIT ? 1 : 2) k_tc_gemm(TcParams p)
         }
         fence_proxy_async();
         mbar_arrive(full_a + s);
-        TLG(1 + j);
       }
     } else if (MODE == 1) {
       // dconv + res_out: q channels 64j + 8*c8 .. +7  <-  in-channels g0 .. g0+3 (out-channel o reads in-channel o/2).
@@ -409,7 +391,6 @@ __global__ void __launch_bounds__(kThreads, SPLIT ? 1 : 2) k_tc_gemm(TcParams p)
         compute(j, 1, sb);
         fence_proxy_async();
         mbar_arrive(full_a + s);
-        TLG(1 + j);
       }
 #pragma unroll
       for (int it = 0; it < 4; ++it) {
@@ -487,17 +468,13 @@ __global__ void __launch_bounds__(kThreads, SPLIT ? 1 : 2) k_tc_gemm(TcParams p)
       }
       fence_proxy_async();
       mbar_arrive(full_a + s);
-      TLG(1 + j);
     }
     if (MODE == 1) qstat.flush_warp(slots, warp);
 
     // ------------------------------------------------------------ epilogue (warps 0-7)
     // warp w reads TMEM lanes 32*(w%4).. (rows) and columns (w/4)*NT/2 .. in chunks of 32.
-    TLG(10);
-    CTL(4);
     mbar_wait(acc_full, 0, 500);
     tc_fence_after();
-    TLG(11);
     const int lq = warp & 3, ch = warp >> 2;
     float* stg = reinterpret_cast<float*>(smem) + warp * (32 * kStgPitch);  // aliases the (now idle) stage buffers
     const int my_rl = lq * 32 + lane;       // the row this thread owns in TMEM
@@ -519,7 +496,6 @@ __global__ void __launch_bounds__(kThreads, SPLIT ? 1 : 2) k_tc_gemm(TcParams p)
         const int col0 = ch * (NT / 2) + cc * 32;
         float v[32];
         tmem_ld32(tmem_base + ((uint32_t)(lq * 32) << 16) + (uint32_t)col0, v);
-        TLG(12 + cc * 4);
         uint4* dst = reinterpret_cast<uint4*>(tile + my_rl * kRowPitch + col0 * 2);
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
@@ -542,7 +518,6 @@ __global__ void __launch_bounds__(kThreads, SPLIT ? 1 : 2) k_tc_gemm(TcParams p)
           }
           dst[i] = make_uint4(h[0], h[1], h[2], h[3]);
         }
-        TLG(14 + cc * 4);
       }
       if (valid) {
         const int sg = smap.seg(r0 + my_rl);
@@ -563,7 +538,6 @@ __global__ void __launch_bounds__(kThreads, SPLIT ? 1 : 2) k_tc_gemm(TcParams p)
       const int col0 = ch * (NT / 2) + cc * 32;
       float v[32];
       tmem_ld32(tmem_base + ((uint32_t)(lq * 32) << 16) + (uint32_t)col0, v);
-      TLG(12 + cc * 4);
       if (MODE == 1) {
 #pragma unroll
         for (int i = 0; i < 16; ++i) rowacc2 = __fadd2_rn(rowacc2, make_float2(v[2 * i], v[2 * i + 1]));
@@ -573,7 +547,6 @@ __global__ void __launch_bounds__(kThreads, SPLIT ? 1 : 2) k_tc_gemm(TcParams p)
       for (int i = 0; i < 8; ++i)
         *reinterpret_cast<float4*>(stg + lane * kStgPitch + i * 4) = make_float4(v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]);
       __syncwarp();
-      TLG(13 + cc * 4);
       // coalesced copy-out: 8 lanes x float4 = one 128 B row segment, 4 rows per instruction
       const int c4 = (lane & 7) * 4;
       const int gcol = (MODE == 2 ? by * NT : 0) + col0 + c4;
@@ -633,7 +606,6 @@ __global__ void __launch_bounds__(kThreads, SPLIT ? 1 : 2) k_tc_gemm(TcParams p)
       }
       };
       if (nrows == kTileM && nseg <= 2) copy_out(std::true_type{}); else copy_out(std::false_type{});
-      TLG(14 + cc * 4);
       if (MODE == 1) {
         // column sums: fold the 4 row groups of the warp, then one global atomic per column and utterance
 #pragma unroll
@@ -655,7 +627,6 @@ __global__ void __launch_bounds__(kThreads, SPLIT ? 1 : 2) k_tc_gemm(TcParams p)
         }
       }
     }
-    TLG(30);
     if (MODE == 0) ostat.flush_warp(slots, warp);
     if (MODE == 1) {
       // row sums: the two column halves (warps w and w+4) own the same rows
@@ -668,8 +639,6 @@ __global__ void __launch_bounds__(kThreads, SPLIT ? 1 : 2) k_tc_gemm(TcParams p)
 
   tc_fence_before();
   __syncthreads();
-  TLG(31);
-  CTL(5);
   if (warp == 9) tmem_dealloc(tmem_base, 256);
   Stat2* sdst = (MODE == 0) ? p.st_out : (MODE == 1 ? p.st_q : nullptr);
   if (sdst != nullptr && by == 0) seg_stats_commit(slots, 8, seg_acc, nseg, sdst + b_first);
@@ -685,26 +654,6 @@ void launch_mode(const TcParams& p, int ntiles_n, cudaStream_t st) {
 }
 
 }  // namespace
-
-#ifdef SEPTFA_TIMELINE
-long long* g_tl_conv1 = nullptr;  // bring-up timeline of one conv1 launch
-#endif
-
-#ifdef SEPTFA_TIMELINE
-void gemm_dump_cta_timeline(int ncta) {   // wall-clock phases of every CTA of the last dconv launch
-  static unsigned long long h[1024 * 8];
-  cudaDeviceSynchronize();
-  cudaMemcpyFromSymbol(h, g_cta_tl, sizeof(h));
-  unsigned long long t0 = ~0ull, t1 = 0;
-  for (int c = 0; c < ncta; ++c) { if (h[c * 8] < t0) t0 = h[c * 8]; if (h[c * 8 + 5] > t1) t1 = h[c * 8 + 5]; }
-  printf("dconv grid: %d CTAs, first start -> last end %llu ns\n", ncta, t1 - t0);
-  printf("cta start pre_pdl pdl_wait setup loop epilogue end\n");
-  for (int c = 0; c < ncta; c += (c < 8 || c > ncta - 9 || (c >= 296 && c < 304)) ? 1 : 37) {
-    const unsigned long long* t = h + c * 8;
-    printf("%4d %7llu %6llu %6llu %6llu %6llu %6llu %7llu\n", c, t[0] - t0, t[1] - t[0], t[2] - t[1], t[3] - t[2], t[4] - t[3], t[5] - t[4], t[5] - t0);
-  }
-}
-#endif
 
 template <int MODE, bool H16, bool AMAX = true, bool SPLIT = false>
 cudaError_t setup_one(int smem) {
@@ -735,15 +684,11 @@ cudaError_t tc_gemm_setup() {
 }
 
 void launch_tc_conv1(const Conv1Params& c, cudaStream_t st) {
-  if (!c.split && launch_conv1_persist(c, st)) return;   // persistent warp-specialised kernel (T >= 128, fp16 activations)
   TcParams p{};
   p.M = c.M; p.T = c.T; p.B = c.B;
   p.w_img = c.w_img; p.w_img_lo = c.w_img_lo; p.in = c.w_in; p.norm = c.norm;
   p.bias = c.bias_f; p.slope = c.slope;
   p.out = c.p_out; p.out_stride = kC; p.st_out = c.st_p;
-#ifdef SEPTFA_TIMELINE
-  p.dbg = g_tl_conv1;
-#endif
   if (c.split) {   // split-precision operands, fp32 p
     if (c.slope <= 1.f) launch_mode<0, false, true, true>(p, 1, st); else launch_mode<0, false, false, true>(p, 1, st);
   } else if (c.slope <= 1.f) {
@@ -760,7 +705,6 @@ void launch_tc_dconv(const DconvParams& c, cudaStream_t st) {
   p.st_p = c.st_p; p.wtab = c.wtab; p.bog = c.bog;
   p.slope2 = c.slope2; p.dil = c.dil; p.st_q = c.st_q;
   p.out = c.racc; p.out_stride = kC; p.rowsum = c.rowsum; p.colsum = c.colsum;
-  p.dbg = c.dbg;
   if (c.split) {   // split-precision operands, fp32 p and racc
     if (c.slope2 <= 1.f) launch_mode<1, false, true, true>(p, 1, st); else launch_mode<1, false, false, true>(p, 1, st);
   } else if (c.slope2 <= 1.f) {

@@ -57,7 +57,6 @@ struct DconvParams {
   float* rowsum;       // [M]
   double* colsum;      // [B,256] (pre-zeroed, accumulated with double atomics)
   Stat2* st_q;         // [B]
-  long long* dbg;      // optional timeline buffer (bring-up only), nullptr otherwise
   int half_io;         // p and racc are fp16
   const float4* wtab;  // tcgen05 engine: the folded taps in pair order, 640 float4 (septfa_abi.cu: dconv tap table)
   const float* bog;    // tcgen05 engine: [256] beta1 / gamma1 (zero-padding substitute, see gemm_tc.cu)
@@ -156,14 +155,13 @@ void launch_tf_gate(const GateParams& p, cudaStream_t st);
 void launch_resid_stats(const ResidParams& p, cudaStream_t st);
 void launch_resid_apply(const ResidParams& p, cudaStream_t st);
 void launch_out_stats(const float* w, StreamNorm norm, float slope, int M, int T, Stat2* st_o, cudaStream_t st);
-// resid_fused.cu
+// resid_fused.cu: gates + both residual GroupNorm steps in one cluster-resident kernel
 cudaError_t resid_fused_setup();
 int resid_fused_cluster_size(int T);   // 0: the utterance does not fit one cluster
-bool launch_resid_fused(const ResidParams& rp, const GateParams& gp, cudaStream_t st);
-#ifdef SEPTFA_TIMELINE
-void resid_fused_dump_timeline();
-void gemm_dump_cta_timeline(int ncta);
-#endif
+// clusters of the kernel variant (stream read / written as fp16) the device keeps resident at once (occupancy query)
+int resid_fused_resident_clusters(bool in_half, bool out_half, int T);
+// launches min(clusters, B) clusters of resid_fused_cluster_size(T) CTAs; racc is fp16
+void launch_resid_fused(const ResidParams& rp, const GateParams& gp, int clusters, cudaStream_t st);
 // preproc.cu
 void launch_minmax_normalize(const float* x, int B, int64_t L, const int64_t* lengths /*nullable*/, unsigned* ext /*[B][2] scratch*/,
                              float* out, cudaStream_t st);
@@ -200,7 +198,7 @@ cudaError_t conv1_pair_setup();
 void launch_conv1_pair(const Conv1PairParams& p, cudaStream_t st);
 // gemm_conv1_persist.cu
 cudaError_t conv1_persist_setup();
-bool launch_conv1_persist(const Conv1Params& p, cudaStream_t st);   // false: not applicable, use launch_tc_conv1's kernel
+void launch_conv1_persist(const Conv1Params& p, cudaStream_t st);   // fp16 p (half_io), T >= 128
 // dconv_mma2.cu: tensor-core depthwise + res_out kernel on CTA pairs (cta_group::2) with the weights resident in shared memory
 cudaError_t dconv_mma2_setup();
 void launch_dconv_mma2(const DconvMmaParams& p, cudaStream_t st);
@@ -208,9 +206,6 @@ void launch_dconv_mma2(const DconvMmaParams& p, cudaStream_t st);
 void launch_tc_conv1(const Conv1Params& p, cudaStream_t st);
 void launch_tc_dconv(const DconvParams& p, cudaStream_t st);
 void launch_tc_outconv(const OutConvParams& p, cudaStream_t st);
-#ifdef SEPTFA_TIMELINE
-extern long long* g_tl_conv1;
-#endif
 cudaError_t tc_gemm_setup();  // opt-in shared memory attributes; call once per device
 // backend.cu
 struct VadParams {
@@ -280,34 +275,44 @@ void launch_live_resample(const int32_t* slots, int n, const int32_t* hops_done,
                           cudaStream_t st);
 
 // Per-handle launch state (septfa_handle owns one; every C-ABI entry binds it to the calling thread before launching).
+// Which kernel runs at each stage of a forward is decided by plan_forward (septfa_abi.cu); the launchers only launch.
 struct LaunchCtx {
   int launches = 0;            // kernels launched since the last reset (host counter)
   int use_pdl = 1;             // launch with the programmatic-stream-serialization attribute
-  int conv1_persist = 1;       // persistent warp-specialised conv1 kernel (0: always the one-tile-per-CTA kernel)
-  int conv1_pair = 1;          // blocks 1 .. n-1, recursive-LN wiring, fast mode: TF32 CTA-pair conv1 fed by TMA from the fp32 stream
-                               // (1: from ~2.5 tiles per SM on, 2: always)
-  int stream_half = 0;         // opt-in: blocks 1 .. n-1 carry the residual stream as fp16 (recursive-LN wiring, fast precision
-                               // mode). 11 % faster, but the stream's rounding random-walks through all blocks: worst VAD
-                               // error on the shape sweep 9.5e-4 against 2.1e-4 - outside the default parity envelope
-  int dconv_mma = 1;           // tensor-core depthwise + res_out kernel on CTA pairs (dconv_mma2.cu) when applicable
-  int l2_discard = 1;          // consumed hand-off buffers (p in the pair dconv kernel, racc in the cluster residual kernel) are discarded from the L2
+  int sm_count = 0;            // SMs of the handle's device: the grids of the persistent and CTA-pair kernels
 };
 LaunchCtx& ctx();
 void bind_ctx(LaunchCtx* c);
 
+// Grid of a launch; cluster > 0 launches clusters of that many CTAs along x (for kernels without __cluster_dims__).
+struct Grid {
+  dim3 dim;
+  unsigned cluster;
+  Grid(dim3 d, unsigned cs = 0) : dim(d), cluster(cs) {}
+};
+
 // Kernel launch with (optional) programmatic dependent launch; counts the launch.
 template <typename... KArgs, typename... Args>
-inline void launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, bool pdl, Args&&... args) {
+inline void launch_k(void (*kern)(KArgs...), Grid grid, dim3 block, size_t smem, cudaStream_t st, bool pdl, Args&&... args) {
   cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
+  cfg.gridDim = grid.dim;
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchAttribute at[2];
+  int n = 0;
+  if (grid.cluster > 0) {
+    at[n].id = cudaLaunchAttributeClusterDimension;
+    at[n].val.clusterDim.x = grid.cluster; at[n].val.clusterDim.y = 1; at[n].val.clusterDim.z = 1;
+    ++n;
+  }
+  if (pdl && ctx().use_pdl) {
+    at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[n].val.programmaticStreamSerializationAllowed = 1;
+    ++n;
+  }
   cfg.attrs = at;
-  cfg.numAttrs = (pdl && ctx().use_pdl) ? 1 : 0;
+  cfg.numAttrs = n;
   cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
   ++ctx().launches;
 }

@@ -71,13 +71,6 @@ struct FusedParams {
 // The statistics of v cross the cluster with one push-style exchange (every CTA stores its partial into every peer's
 // shared memory, ONE cluster barrier, then only local reads); the statistics of the new stream go out as one double
 // atomic pair per CTA. A thread owns 4 channels (two packed pairs: FFMA2) of every 8th frame of the CTA's tile.
-#ifdef SEPTFA_TIMELINE
-__device__ unsigned long long g_fused_tl[32 * 128];
-__device__ __forceinline__ unsigned long long gtimer() { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
-#define FTL(k) do { if (threadIdx.x == 0 && blockIdx.x < 32 && (k) < 128) g_fused_tl[blockIdx.x * 128 + (k)] = gtimer(); } while (0)
-#else
-#define FTL(k) do { } while (0)
-#endif
 constexpr int kPersistThreads = 256;
 constexpr int kPersistWarps = kPersistThreads / 32;
 constexpr int kRowGroups = kPersistThreads / 64;   // a thread owns 4 channels of every kRowGroups-th frame of the tile
@@ -115,12 +108,10 @@ __global__ void __launch_bounds__(kPersistThreads, 4) k_resid_persist(FusedParam
     mbar_init(&xbar[1], 1);
     fence_mbar_init();
   }
-  FTL(0);
   cluster.barrier_arrive();   // "this CTA runs": peers wait for it before they store into our shared memory
   pdl_launch_dependents();
   __syncthreads();
   pdl_wait();
-  FTL(1);
 
   auto fetch = [&](int b) {   // one thread: two bulk copies onto the tile's mbarrier
     const int64_t row0 = (int64_t)b * p.T + t0;
@@ -234,7 +225,6 @@ __global__ void __launch_bounds__(kPersistThreads, 4) k_resid_persist(FusedParam
     };
     const int b_next = b + n_clusters;
     const bool has_next = b_next < p.B;
-    FTL(8 + it * 8 + 0);
     if (has_next) {
       fetch_small(b_next);                    // consumed by the gate stages further down
       if (tid == kPersistThreads - 1) scalars_for(b_next, buf ^ 1, 0);
@@ -257,7 +247,6 @@ __global__ void __launch_bounds__(kPersistThreads, 4) k_resid_persist(FusedParam
       G2[0] = __fmul2_rn(make_float2(rb4.x, rb4.y), make_float2(gf4.x, gf4.y));
       G2[1] = __fmul2_rn(make_float2(rb4.z, rb4.w), make_float2(gf4.z, gf4.w));
     }
-    FTL(8 + it * 8 + 1);
     mbar_wait(&full, it & 1, 700);   // the tile has landed (every thread observes the barrier itself)
     if (p.discard) {
       // racc is read exactly once, by this CTA, and it is in shared memory now: its lines in the L2 are dead but dirty (the
@@ -265,7 +254,6 @@ __global__ void __launch_bounds__(kPersistThreads, 4) k_resid_persist(FusedParam
       const uint8_t* rg = reinterpret_cast<const uint8_t*>(p.racc + ((int64_t)b * p.T + t0) * kC);
       for (int l = tid; l < nt * 4; l += kPersistThreads) asm volatile("discard.global.L2 [%0], 128;" ::"l"(rg + (size_t)l * 128) : "memory");
     }
-    FTL(8 + it * 8 + 2);
 
     // ---- statistics of v = y + gt (G1 r + G2)  (recursive)  |  gt (G1 r + G2)  (residual) over the whole utterance
     float2 mv = make_float2(0.f, 1.f);
@@ -293,7 +281,6 @@ __global__ void __launch_bounds__(kPersistThreads, 4) k_resid_persist(FusedParam
       }
       double ts = 0.0, tq = 0.0;
       block_total(s2.x + s2.y, q2.x + q2.y, ts, tq);
-      FTL(8 + it * 8 + 3);
       if (!peers_up) { cluster.barrier_wait(); peers_up = true; }   // every peer is running: its shared memory may be written
       // Push-style exchange without a cluster barrier: every CTA sends its 16-byte partial to every peer with st.async, which
       // counts the bytes on the RECEIVER's mbarrier; a CTA then waits for its own 8 x 16 bytes. (cluster.sync() is
@@ -311,7 +298,6 @@ __global__ void __launch_bounds__(kPersistThreads, 4) k_resid_persist(FusedParam
                        : "memory");
         }
       }
-      FTL(8 + it * 8 + 4);
       if (tid == 0) {
         mbar_wait(&xbar[buf], (it >> 1) & 1, 710);
         Stat2 tot{0.0, 0.0};
@@ -379,7 +365,6 @@ __global__ void __launch_bounds__(kPersistThreads, 4) k_resid_persist(FusedParam
       q2 = __ffma2_rn(o0, o0, q2);
       q2 = __ffma2_rn(o1, o1, q2);
     }
-    FTL(8 + it * 8 + 5);
     if (has_next) gate_stage1(buf ^ 1);
     {
       double ts = 0.0, tq = 0.0;
@@ -393,35 +378,11 @@ __global__ void __launch_bounds__(kPersistThreads, 4) k_resid_persist(FusedParam
     __syncthreads();   // every thread is done with this buffer and the scratch arrays: the next fetch may overwrite it
   }
   if (!peers_up) cluster.barrier_wait();
-  FTL(2);
 }
 
 }  // namespace
 
-// Programmatic early launch of the persistent cluster kernel: only safe because its predecessor (the dconv kernel)
-// does not trigger its dependents, so they launch as its CTAs exit. With the usual trigger at kernel entry the
-// persistent grid became resident while the dconv grid's second wave still needed the SM slots (5.86 vs 5.09 ms per
-// step); with the late trigger the early launch hides the launch latency instead (3.75 -> 3.70 ms).
-
-#ifdef SEPTFA_TIMELINE
-void resid_fused_dump_timeline() {   // bring-up: globaltimer stamps of the first 32 CTAs of the last launch
-  static unsigned long long h[32 * 128];
-  cudaDeviceSynchronize();
-  cudaMemcpyFromSymbol(h, g_fused_tl, sizeof(h));
-  for (int c = 0; c < 32; ++c) {
-    const unsigned long long* t = h + c * 128;
-    printf("cta %2d: start->pdl %6llu total %6llu |", c, t[1] - t[0], t[2] - t[0]);
-    for (int it = 0; it < 9; ++it) {
-      const unsigned long long* u = t + 8 + it * 8;
-      if (u[0] == 0) break;
-      printf(" [top@%llu gates %llu tile %llu ph1 %llu xchg %llu ph2 %llu]", u[0] - t[0], u[1] - u[0], u[2] - u[1], u[3] - u[2], u[4] - u[3], u[5] - u[4]);
-    }
-    printf("\n");
-  }
-}
-#endif
-
-int resid_fused_cluster_size(int T) {   // 0: the utterance does not fit one cluster (caller uses the streaming kernels)
+int resid_fused_cluster_size(int T) {   // 0: the utterance does not fit one cluster (the forward uses the streaming kernels)
   if (T > 16 * kMaxTc) return 0;
   if (T > 8 * kMaxTc) return 16;          // 18 .. 36 s: clusters of 16 CTAs (non-portable size, allowed per kernel in setup)
   return std::min(8, (T + 31) / 32);
@@ -447,49 +408,30 @@ cudaError_t resid_fused_setup() {
   return cudaSuccess;
 }
 
-// Clusters of `cs` CTAs of the persistent kernel the device keeps resident at once (cached per variant / cluster size / footprint).
-static int persist_clusters(int variant, int cs, size_t smem) {
-  static int cache[4][17] = {};
-  static size_t cache_smem[4][17] = {};
-  if (cache[variant][cs] != 0 && cache_smem[variant][cs] == smem) return cache[variant][cs];
+// Clusters of the persistent kernel the device keeps resident at once (0: none, or the query failed).
+int resid_fused_resident_clusters(bool in_half, bool out_half, int T) {
+  const int cs = resid_fused_cluster_size(T);
+  if (cs == 0) return 0;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(cs * 1024);
   cfg.blockDim = dim3(kPersistThreads);
-  cfg.dynamicSmemBytes = smem;
+  cfg.dynamicSmemBytes = (size_t)((T + cs - 1) / cs) * row_bytes(in_half);
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeClusterDimension;
   at[0].val.clusterDim.x = cs; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
   cfg.attrs = at;
   cfg.numAttrs = 1;
   int n = 0;
-  if (cudaOccupancyMaxActiveClusters(&n, resid_kernel(variant >> 1, variant & 1), &cfg) != cudaSuccess) { cudaGetLastError(); n = 0; }
-  cache[variant][cs] = n;
-  cache_smem[variant][cs] = smem;
+  if (cudaOccupancyMaxActiveClusters(&n, resid_kernel(in_half, out_half), &cfg) != cudaSuccess) { cudaGetLastError(); n = 0; }
   return n;
 }
 
-template <typename K>
-static void launch_cluster(K kernel, const FusedParams& p, int nclusters, int cs, int threads, size_t smem, cudaStream_t st) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(nclusters * cs);
-  cfg.blockDim = dim3(threads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute at[2];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = cs; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-  at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = ctx().use_pdl ? 2 : 1;
-  cudaLaunchKernelEx(&cfg, kernel, p);
-  ++ctx().launches;
-}
-
-// Returns false if the utterance does not fit a cluster (caller falls back to k_tf_gate + k_resid<0,1>).
-bool launch_resid_fused(const ResidParams& rp, const GateParams& gp, cudaStream_t st) {
+// Programmatic early launch of the persistent cluster kernel: only safe because its predecessor (the dconv kernel)
+// does not trigger its dependents, so they launch as its CTAs exit. With the usual trigger at kernel entry the
+// persistent grid became resident while the dconv grid's second wave still needed the SM slots (5.86 vs 5.09 ms per
+// step); with the late trigger the early launch hides the launch latency instead (3.75 -> 3.70 ms).
+void launch_resid_fused(const ResidParams& rp, const GateParams& gp, int clusters, cudaStream_t st) {
   const int cs = resid_fused_cluster_size(rp.T);
-  if (!rp.racc_half || cs == 0) return false;
   FusedParams p{};
   p.w_in = rp.w_half_in ? rp.w_half_in : static_cast<const void*>(rp.w);
   p.w_out = rp.w_half_out ? rp.w_half_out : static_cast<void*>(rp.w);
@@ -498,12 +440,10 @@ bool launch_resid_fused(const ResidParams& rp, const GateParams& gp, cudaStream_
   p.T = rp.T; p.B = rp.B; p.Tc = (rp.T + cs - 1) / cs; p.discard = rp.discard;
   p.inv_T = 1.0 / (double)rp.T; p.inv_HT = 1.0 / ((double)kH * rp.T); p.inv_CT = 1.0 / ((double)kC * rp.T);
   p.mode = rp.mode; p.g_a = rp.g_a; p.b_a = rp.b_a; p.st_w = rp.st_w;
-  const int in_half = rp.w_half_in ? 1 : 0, out_half = rp.w_half_out ? 1 : 0, variant = in_half * 2 + out_half;
+  const bool in_half = rp.w_half_in != nullptr;
   const size_t smem = (size_t)p.Tc * row_bytes(in_half);
-  const int n_clusters = persist_clusters(variant, cs, smem);
-  if (n_clusters <= 0) return false;
-  launch_cluster(resid_kernel(in_half, out_half), p, std::min(n_clusters, rp.B), cs, kPersistThreads, smem, st);
-  return true;
+  launch_k(resid_kernel(in_half, rp.w_half_out != nullptr), Grid(dim3(std::min(clusters, rp.B) * cs), cs), dim3(kPersistThreads),
+           smem, st, true, p);
 }
 
 }  // namespace septfa

@@ -62,8 +62,7 @@ struct septfa_handle {
   float act_k[9]{}; float act_b = 0.f; float act_a = 0.f;
   const float* win_fwd = nullptr; const float* win_inv = nullptr; const float2* twiddle = nullptr;
   int last_launches = 0;
-  int sm_count = 148;
-  LaunchCtx lctx;   // launch options and counter of this handle (bound to the calling thread by every entry point)
+  LaunchCtx lctx;   // launch options, device facts and counter of this handle (bound to the calling thread by every entry point)
   // forward_host resources
   cudaStream_t hstream = nullptr, hstream_in = nullptr, hstream_out = nullptr;
   cudaEvent_t hev_in[8] = {}, hev_done[8] = {};
@@ -78,8 +77,20 @@ struct septfa_handle {
     bool busy = false;
   } slots[SEPTFA_HOST_SLOTS];
   cudaStream_t slot_compute = nullptr;      // kernels of both slots, in submission order
-  int fused_resid = 1;  // cluster-resident gate + residual kernel when the utterance fits a cluster
-  int precision = SEPTFA_PRECISION_AUTO;   // option "precision"
+  // kernel options (septfa_set_option), read by plan_forward
+  int fused_resid = 1;    // cluster-resident gate + residual kernel when the utterance fits a cluster
+  int precision = SEPTFA_PRECISION_AUTO;
+  int conv1_persist = 1;  // persistent warp-specialised conv1 kernel (0: always the one-tile-per-CTA kernel)
+  int conv1_pair = 1;     // blocks 1 .. n-1, recursive-LN wiring, fast mode: TF32 CTA-pair conv1 fed by TMA from the fp32 stream
+                          // (1: from ~2.5 tiles per SM on, 2: always)
+  int stream_half = 0;    // opt-in: blocks 1 .. n-1 carry the residual stream as fp16 (recursive-LN wiring, fast precision
+                          // mode). 11 % faster, but the stream's rounding random-walks through all blocks: worst VAD
+                          // error on the shape sweep 9.5e-4 against 2.1e-4 - outside the default parity envelope
+  int dconv_mma = 1;      // tensor-core depthwise + res_out kernel on CTA pairs (dconv_mma2.cu) when applicable
+  int l2_discard = 1;     // consumed hand-off buffers (p in the pair dconv kernel, racc in the cluster residual kernel) are discarded from the L2
+  // resident clusters of the cluster residual kernel by (variant, frame count): an occupancy query of this handle's
+  // device, cached so that a forward does not repeat it (a cache: filling it changes no plan)
+  mutable std::map<std::pair<int, int>, int> resid_clusters;
   bool all_mma_ok = false;                 // every block's folded taps are representable for the tensor-core depthwise kernel
   float* hx_dev = nullptr; float* hout_dev = nullptr; float* hvad_dev = nullptr; void* hws = nullptr; void* hws_b = nullptr;
   float* hx_pin = nullptr; float* hout_pin = nullptr; float* hvad_pin = nullptr;
@@ -395,11 +406,85 @@ int check_forward_args(septfa_handle* h, int B, int64_t L) {
   return 0;
 }
 
-}  // namespace
+// Which kernel runs at each stage of a forward, and the storage modes that tie neighbouring kernels together.
+enum class Conv1Kernel { ref, tc_gemm, persist, pair, tma };
+enum class DconvKernel { ref, tc_gemm, mma2 };
+struct ForwardPlan {
+  bool split;             // split-precision operands of conv1 / dconv ("accurate" mode): fp32 p / racc
+  bool half_io;           // p and racc stored as fp16
+  bool planes;            // p stored as K-group planes of Mp slots (written by the persistent / pair / TMA conv1, read by mma2)
+  int Mp;
+  bool stream_half;       // blocks 1 .. n-1 carry the residual stream as fp16
+  Conv1Kernel conv1_first, conv1_rest;   // block 0, blocks 1 .. n-1
+  DconvKernel dconv;
+  int resid_clusters[2][2];   // [stream read as fp16][stream written as fp16]: resident clusters of the cluster residual
+                              // kernel for the variants the forward runs; all 0: k_tf_gate + the streaming kernels
+  bool tc_out;            // output conv on the tensor cores (else the fp32 CUDA-core kernel)
+  bool exports;           // back end: k_mask_istft_export (any est / mask / logits export), else k_mask_istft
+};
 
-#ifdef SEPTFA_TIMELINE
-long long* septfa_dbg_ptr = nullptr;   // bring-up timeline buffer (clock64 stamps of one CTA)
-#endif
+int resident_clusters(const septfa_handle& h, bool in_half, bool out_half, int T) {
+  const auto key = std::make_pair((in_half ? 2 : 0) + (out_half ? 1 : 0), T);
+  auto it = h.resid_clusters.find(key);
+  if (it == h.resid_clusters.end()) it = h.resid_clusters.emplace(key, resid_fused_resident_clusters(in_half, out_half, T)).first;
+  return it->second;
+}
+
+ForwardPlan plan_forward(const septfa_handle& h, int B, int64_t L, bool exports) {
+  ForwardPlan pl{};
+  const int T = (int)septfa_num_frames(L);
+  const int64_t M = (int64_t)B * T;
+  // engine is a bit mask of the contractions that run on the fp32 CUDA-core kernels
+  const bool tc_conv1 = !(h.engine & 1), tc_dconv = !(h.engine & 2);
+  pl.tc_out = !(h.engine & 4);
+  // p (conv1 -> dconv) and racc (dconv -> residual kernels) are stored as fp16 when both producers run on the tensor
+  // cores: their consumers round to fp16 operands anyway, and emulation on the oracle shows no change of the VAD /
+  // waveform error (DESIGN.md section 3); the fp32 CUDA-core engine keeps fp32 storage.
+  // Precision mode of the two block contractions: "accurate" = split-precision operands (three tensor-core passes) and
+  // fp32 p / racc. AUTO picks it for the residual-LN wiring (config_without_vad): its stream is never re-normalised, so
+  // the fp16 roundings of all 24 blocks accumulate to ~1e-3 in VAD probability, against ~1e-4 with the recursive-LN
+  // wiring of config_with_vad (measured: DESIGN.md, "Precision").
+  pl.split = tc_conv1 && tc_dconv &&
+             (h.precision == SEPTFA_PRECISION_ACCURATE || (h.precision == SEPTFA_PRECISION_AUTO && h.ln_mode == LN_RESIDUAL));
+  pl.half_io = tc_conv1 && tc_dconv && !pl.split;
+  // Tensor-core depthwise kernel (dconv_mma2.cu): p travels as K-group planes, which only the persistent conv1 (and
+  // the pair / TMA conv1 of blocks 1 .. n-1) write.
+  const bool persist = pl.half_io && T >= 128 && h.conv1_persist;
+  pl.planes = persist && h.dconv_mma && h.all_mma_ok;
+  pl.Mp = (int)((M + 255) / 256 * 256 + 2 * kPlaneHalo);   // whole tile PAIRS (dconv_mma2.cu walks its tiles in pairs)
+  // Gates + both residual GroupNorm steps in one cluster-resident kernel when an utterance fits a cluster and the
+  // device keeps clusters of it resident.
+  const bool fused = h.fused_resid && pl.half_io && resid_fused_cluster_size(T) > 0;
+  // Half-stream mode: between the blocks the residual stream is stored as fp16 (written by the cluster-resident residual
+  // kernel of block i, read by TMA as the A operand of conv1 of block i + 1 and by the residual kernel of block i + 1); the
+  // first block reads the front end's fp32 features, the last block writes fp32 for the output layer. Recursive-LN wiring
+  // in the fast precision mode only: the stream is re-normalised by every block, so its fp16 rounding is one more source of
+  // the size of the operand roundings (DESIGN.md, "Precision"), and the residual-LN wiring runs the accurate mode anyway.
+  // Only the cluster kernel reads and writes the fp16 stream, so every variant the blocks run must have resident clusters.
+  if (fused && pl.planes && h.stream_half && h.ln_mode == LN_RECURSIVE && h.nblk > 1) {
+    pl.resid_clusters[0][1] = resident_clusters(h, false, true, T);
+    pl.resid_clusters[1][0] = resident_clusters(h, true, false, T);
+    if (h.nblk > 2) pl.resid_clusters[1][1] = resident_clusters(h, true, true, T);
+    pl.stream_half = pl.resid_clusters[0][1] > 0 && pl.resid_clusters[1][0] > 0 && (h.nblk == 2 || pl.resid_clusters[1][1] > 0);
+    if (!pl.stream_half) pl.resid_clusters[0][1] = pl.resid_clusters[1][0] = pl.resid_clusters[1][1] = 0;
+  }
+  if (fused && !pl.stream_half) pl.resid_clusters[0][0] = resident_clusters(h, false, false, T);
+  // TF32 CTA-pair conv1 (gemm_conv1_pair.cu) for blocks 1 .. n-1: the fp32 stream is its A operand, fetched by TMA
+  // (from ~2.5 tiles per SM on: each of its CTAs first loads 128 KB of weights, which 1-2 tiles do not pay back - measured
+  // at 64 / 128 / 256 x 4 s: +0.06 / +0.03 / -0.055 ms per forward against the persistent producer kernel; option value 2
+  // forces it at any size)
+  const bool pair = pl.planes && !pl.stream_half && h.conv1_pair && h.ln_mode == LN_RECURSIVE && h.nblk > 1 &&
+                    (h.conv1_pair == 2 || (M + 127) / 128 * 2 >= (int64_t)h.lctx.sm_count * 5);
+  pl.conv1_first = !tc_conv1 ? Conv1Kernel::ref : (persist ? Conv1Kernel::persist : Conv1Kernel::tc_gemm);
+  pl.conv1_rest = pl.stream_half ? Conv1Kernel::tma : (pair ? Conv1Kernel::pair : pl.conv1_first);
+  pl.dconv = pl.planes ? DconvKernel::mma2 : (tc_dconv ? DconvKernel::tc_gemm : DconvKernel::ref);
+  // With any of the est / mask / logits exports, one kernel writes them and the waveform from one read of S and the logits;
+  // without them the register-prefetch kernel (3 CTAs per SM against 2) is slightly faster end to end (DESIGN.md section 3).
+  pl.exports = exports;
+  return pl;
+}
+
+}  // namespace
 
 extern "C" {
 
@@ -436,7 +521,7 @@ int septfa_create(septfa_handle** out, const septfa_config* cfg, int device) {
   h->ln_mode = c.apply_recursive_ln ? LN_RECURSIVE : (c.apply_residual_ln ? LN_RESIDUAL : LN_NONE);  // model.py:347-352
   build_keys(h);
   if (cudaSetDevice(device) != cudaSuccess) { delete h; return fail(nullptr, SEPTFA_E_CUDA, "cudaSetDevice failed"); }
-  cudaDeviceGetAttribute(&h->sm_count, cudaDevAttrMultiProcessorCount, device);
+  cudaDeviceGetAttribute(&h->lctx.sm_count, cudaDevAttrMultiProcessorCount, device);
   cudaError_t e = tc_gemm_setup();
   if (e == cudaSuccess) e = resid_fused_setup();
   if (e == cudaSuccess) e = conv1_persist_setup();
@@ -507,15 +592,15 @@ int septfa_set_option(septfa_handle* h, const char* name, int value) {
     return 0;
   }
   if (std::strcmp(name, "conv1_persist") == 0) {
-    h->lctx.conv1_persist = value ? 1 : 0;
+    h->conv1_persist = value ? 1 : 0;
     return 0;
   }
   if (std::strcmp(name, "conv1_pair") == 0) {
-    h->lctx.conv1_pair = value == 2 ? 2 : (value ? 1 : 0);
+    h->conv1_pair = value == 2 ? 2 : (value ? 1 : 0);
     return 0;
   }
   if (std::strcmp(name, "stream_half") == 0) {
-    h->lctx.stream_half = value ? 1 : 0;
+    h->stream_half = value ? 1 : 0;
     return 0;
   }
   if (std::strcmp(name, "fused_resid") == 0) {
@@ -527,11 +612,11 @@ int septfa_set_option(septfa_handle* h, const char* name, int value) {
     return 0;
   }
   if (std::strcmp(name, "dconv_mma") == 0) {
-    h->lctx.dconv_mma = value ? 1 : 0;
+    h->dconv_mma = value ? 1 : 0;
     return 0;
   }
   if (std::strcmp(name, "l2_discard") == 0) {
-    h->lctx.l2_discard = value ? 1 : 0;
+    h->l2_discard = value ? 1 : 0;
     return 0;
   }
   if (std::strcmp(name, "precision") == 0) {
@@ -864,20 +949,9 @@ int septfa_forward(septfa_handle* h, const float* x, int B, int64_t L, const sep
   const Workspace ws = carve(h, base, B, L);
   const int T = (int)septfa_num_frames(L);
   const int M = B * T;
-  // engine is a bit mask of the contractions that run on the fp32 CUDA-core kernels
-  const bool tc_conv1 = !(h->engine & 1), tc_dconv = !(h->engine & 2), tc_out = !(h->engine & 4);
-  // p (conv1 -> dconv) and racc (dconv -> residual kernels) are stored as fp16 when both producers run on the tensor
-  // cores: their consumers round to fp16 operands anyway, and emulation on the oracle shows no change of the VAD /
-  // waveform error (DESIGN.md section 3); the fp32 CUDA-core engine keeps fp32 storage.
-  // Precision mode of the two block contractions: "accurate" = split-precision operands (three tensor-core passes) and
-  // fp32 p / racc. AUTO picks it for the residual-LN wiring (config_without_vad): its stream is never re-normalised, so
-  // the fp16 roundings of all 24 blocks accumulate to ~1e-3 in VAD probability, against ~1e-4 with the recursive-LN
-  // wiring of config_with_vad (measured: DESIGN.md, "Precision").
-  const bool split = tc_conv1 && tc_dconv &&
-                     (h->precision == SEPTFA_PRECISION_ACCURATE || (h->precision == SEPTFA_PRECISION_AUTO && h->ln_mode == LN_RESIDUAL));
-  const int half_io = (tc_conv1 && tc_dconv && !split) ? 1 : 0;
   const auto& c = h->cfg;
   bind_ctx(&h->lctx);
+  const ForwardPlan pl = plan_forward(*h, B, L, est_stft != nullptr || mask != nullptr || logits_out != nullptr);
   ctx().launches = 0;
 
   prof_mark(h, SEPTFA_PROF_FRONTEND, st);
@@ -885,32 +959,21 @@ int septfa_forward(septfa_handle* h, const float* x, int B, int64_t L, const sep
   launch_frontend(x, B, L, T, h->win_fwd, h->twiddle, c.activity_input_bool, h->act_k, h->act_b, h->act_a, ws.S, ws.w,
                   ws.dcg, ws.st0, spectrum, st);   // (the optional spectrum export leaves from the front end's own rows)
 
-  // Tensor-core depthwise kernel (dconv_mma2.cu): p travels as K-group planes; its halo slots must read as zeros.
-  const bool planes = half_io && T >= 128 && h->lctx.conv1_persist && h->lctx.dconv_mma && h->all_mma_ok;
-  const int Mp = (M + 255) / 256 * 256 + 2 * kPlaneHalo;   // whole tile PAIRS (dconv_mma2.cu walks its tiles in pairs)
-  if (planes) {
+  const int Mp = pl.Mp;
+  if (pl.planes) {   // the halo slots of the plane layout must read as zeros
     uint8_t* pb = reinterpret_cast<uint8_t*>(ws.p);
     CUDA_TRY(h, cudaMemset2DAsync(pb, (size_t)Mp * 16, 0, (size_t)kPlaneHalo * 16, 32, st));
     CUDA_TRY(h, cudaMemset2DAsync(pb + (size_t)(M + kPlaneHalo) * 16, (size_t)Mp * 16, 0, (size_t)(Mp - M - kPlaneHalo) * 16, 32, st));
   }
-  // Half-stream mode: between the blocks the residual stream is stored as fp16 (written by the cluster-resident residual
-  // kernel of block i, read by TMA as the A operand of conv1 of block i + 1 and by the residual kernel of block i + 1); the
-  // first block reads the front end's fp32 features, the last block writes fp32 for the output layer. Recursive-LN wiring
-  // in the fast precision mode only: the stream is re-normalised by every block, so its fp16 rounding is one more source of
-  // the size of the operand roundings (DESIGN.md, "Precision"), and the residual-LN wiring runs the accurate mode anyway.
-  const bool stream_half = planes && h->lctx.stream_half && h->ln_mode == LN_RECURSIVE && h->fused_resid && resid_fused_cluster_size(T) > 0 && h->nblk > 1;
   alignas(64) CUtensorMap wh_tmap;
-  if (stream_half && !make_stream_tmap(&wh_tmap, ws.wh, M)) return fail(h, SEPTFA_E_CUDA, "cuTensorMapEncodeTiled failed for the fp16 stream");
-  // TF32 CTA-pair conv1 (gemm_conv1_pair.cu) for blocks 1 .. n-1: the fp32 stream is its A operand, fetched by TMA
-  // (from ~2.5 tiles per SM on: each of its CTAs first loads 128 KB of weights, which 1-2 tiles do not pay back - measured
-  // at 64 / 128 / 256 x 4 s: +0.06 / +0.03 / -0.055 ms per forward against the persistent producer kernel; option value 2
-  // forces it at any size)
-  const bool c1pair = planes && !stream_half && h->lctx.conv1_pair && h->ln_mode == LN_RECURSIVE && h->nblk > 1 &&
-                      (h->lctx.conv1_pair == 2 || (int64_t)((M + 127) / 128) * 2 >= (int64_t)h->sm_count * 5);
+  if (pl.conv1_rest == Conv1Kernel::tma && !make_stream_tmap(&wh_tmap, ws.wh, M))
+    return fail(h, SEPTFA_E_CUDA, "cuTensorMapEncodeTiled failed for the fp16 stream");
   alignas(64) CUtensorMap w32_tmap;
-  if (c1pair && !make_stream_tmap(&w32_tmap, ws.w, M, 128, true)) return fail(h, SEPTFA_E_CUDA, "cuTensorMapEncodeTiled failed for the fp32 stream");
+  if (pl.conv1_rest == Conv1Kernel::pair && !make_stream_tmap(&w32_tmap, ws.w, M, 128, true))
+    return fail(h, SEPTFA_E_CUDA, "cuTensorMapEncodeTiled failed for the fp32 stream");
   alignas(64) CUtensorMap racc_tmap;   // the pair kernel's epilogue stores racc with TMA tensor stores (boxes of 32 rows x 64 columns)
-  if (planes && !make_stream_tmap(&racc_tmap, ws.racc, M, 32)) return fail(h, SEPTFA_E_CUDA, "cuTensorMapEncodeTiled failed for racc");
+  if (pl.dconv == DconvKernel::mma2 && !make_stream_tmap(&racc_tmap, ws.racc, M, 32))
+    return fail(h, SEPTFA_E_CUDA, "cuTensorMapEncodeTiled failed for racc");
   const double inv_n = 1.0 / ((double)kC * T);
   StreamNorm norm{ws.st0, h->ln_g, h->ln_b, 1e-8f, inv_n};  // TCN.LN, model.py:333
   for (int i = 0; i < h->nblk; ++i) {
@@ -920,56 +983,49 @@ int septfa_forward(septfa_handle* h, const float* x, int B, int64_t L, const sep
     Stat2* st_v = ws.st_blk + (size_t)(i * 4 + 2) * B;
     Stat2* st_w = ws.st_blk + (size_t)(i * 4 + 3) * B;
     double* colsum = ws.colsum + (size_t)i * B * kC;
+    __half* p_planes = reinterpret_cast<__half*>(ws.p);
 
-    Conv1Params c1{ws.w, norm, M, T, B, d.b1, d.a1, d.w1_img, d.b1f, d.w1_t, ws.p, st_p, half_io, planes ? 1 : 0, Mp, d.w1_img_lo, split ? 1 : 0};
-#ifdef SEPTFA_TIMELINE
-    g_tl_conv1 = (i == 6 && getenv("SEPTFA_TIMELINE") && septfa_dbg_ptr) ? septfa_dbg_ptr + 1024 : nullptr;
-#endif
     prof_mark(h, SEPTFA_PROF_CONV1, st);
-    if (stream_half && i > 0) {
-      Conv1TmaParams ct{&wh_tmap, norm, M, T, B, d.w1_img, d.sb1, d.a1, reinterpret_cast<__half*>(ws.p), Mp, st_p};
-      launch_conv1_tma(ct, st);
-    } else if (c1pair && i > 0) {
-      Conv1PairParams cp{&w32_tmap, norm, M, T, B, d.w1_img32, d.sb1_32, d.a1, reinterpret_cast<__half*>(ws.p), Mp, st_p};
-      launch_conv1_pair(cp, st);
-    } else if (tc_conv1) {
-      launch_tc_conv1(c1, st);
-    } else {
-      launch_ref_conv1(c1, st);
+    const Conv1Params c1{ws.w, norm, M, T, B, d.b1, d.a1, d.w1_img, d.b1f, d.w1_t, ws.p, st_p, pl.half_io, pl.planes, Mp,
+                         d.w1_img_lo, pl.split};
+    switch (i == 0 ? pl.conv1_first : pl.conv1_rest) {
+      case Conv1Kernel::ref: launch_ref_conv1(c1, st); break;
+      case Conv1Kernel::tc_gemm: launch_tc_conv1(c1, st); break;
+      case Conv1Kernel::persist: launch_conv1_persist(c1, st); break;
+      case Conv1Kernel::pair:
+        launch_conv1_pair(Conv1PairParams{&w32_tmap, norm, M, T, B, d.w1_img32, d.sb1_32, d.a1, p_planes, Mp, st_p}, st);
+        break;
+      case Conv1Kernel::tma:
+        launch_conv1_tma(Conv1TmaParams{&wh_tmap, norm, M, T, B, d.w1_img, d.sb1, d.a1, p_planes, Mp, st_p}, st);
+        break;
     }
 
     prof_mark(h, SEPTFA_PROF_DCONV, st);
-    DconvParams dc{ws.p, st_p, d.g1, d.be1, d.w2b, d.w2f, d.c2f, d.a2, d.dil, M, T, B, d.w3_img, d.w3_t, ws.racc, ws.rowsum, colsum, st_q,
-                   nullptr, half_io, d.wtab, d.bog, d.w3_img_lo, split ? 1 : 0};
-#ifdef SEPTFA_TIMELINE
-    if (i == 5 && getenv("SEPTFA_TIMELINE")) {   // bring-up timeline of block 5's dconv launch
-      if (!septfa_dbg_ptr) { cudaMalloc(reinterpret_cast<void**>(&septfa_dbg_ptr), 8 * 256 * sizeof(long long)); }
-      cudaMemsetAsync(septfa_dbg_ptr, 0, 8 * 256 * sizeof(long long), st);
-      dc.dbg = septfa_dbg_ptr;
-    }
-#endif
-    if (planes) {
-      DconvMmaParams dm{reinterpret_cast<const __half*>(ws.p), Mp, st_p, d.tap_img2, d.swc, d.w16, d.bog, d.a2, d.dil, M, T, B, d.w3_img,
-                        reinterpret_cast<__half*>(ws.racc), ws.rowsum, colsum, st_q, &racc_tmap, h->lctx.l2_discard};
-      launch_dconv_mma2(dm, st);
-    } else if (tc_dconv) {
-      launch_tc_dconv(dc, st);
+    if (pl.dconv == DconvKernel::mma2) {
+      launch_dconv_mma2(DconvMmaParams{p_planes, Mp, st_p, d.tap_img2, d.swc, d.w16, d.bog, d.a2, d.dil, M, T, B, d.w3_img,
+                                       reinterpret_cast<__half*>(ws.racc), ws.rowsum, colsum, st_q, &racc_tmap, h->l2_discard},
+                        st);
     } else {
-      launch_ref_dconv(dc, st);
+      const DconvParams dc{ws.p, st_p, d.g1, d.be1, d.w2b, d.w2f, d.c2f, d.a2, d.dil, M, T, B, d.w3_img, d.w3_t, ws.racc,
+                           ws.rowsum, colsum, st_q, pl.half_io, d.wtab, d.bog, d.w3_img_lo, pl.split};
+      if (pl.dconv == DconvKernel::tc_gemm) launch_tc_dconv(dc, st); else launch_ref_dconv(dc, st);
     }
 
-    prof_mark(h, SEPTFA_PROF_GATE, st);
-    GateParams gp{st_q, (tc_dconv && !split) ? d.s3_tc : d.s3_ref, d.c03, ws.rowsum, colsum, d.tf, M, T, B, ws.ra, ws.rb, ws.gf, ws.gt, ws.mt};
+    const GateParams gp{st_q, (pl.dconv != DconvKernel::ref && !pl.split) ? d.s3_tc : d.s3_ref, d.c03, ws.rowsum, colsum, d.tf,
+                        M, T, B, ws.ra, ws.rb, ws.gf, ws.gt, ws.mt};
     ResidParams rp{};
-    rp.w = ws.w; rp.norm = norm; rp.racc = ws.racc; rp.racc_half = half_io; rp.ra = ws.ra; rp.rb = ws.rb; rp.gf = ws.gf; rp.gt = ws.gt;
-    rp.M = M; rp.T = T; rp.B = B; rp.mode = h->ln_mode; rp.st_v = st_v; rp.st_w = st_w; rp.discard = h->lctx.l2_discard;
-    if (stream_half) { rp.w_half_in = i > 0 ? ws.wh : nullptr; rp.w_half_out = i + 1 < h->nblk ? ws.wh : nullptr; }
+    rp.w = ws.w; rp.norm = norm; rp.racc = ws.racc; rp.racc_half = pl.half_io; rp.ra = ws.ra; rp.rb = ws.rb; rp.gf = ws.gf; rp.gt = ws.gt;
+    rp.M = M; rp.T = T; rp.B = B; rp.mode = h->ln_mode; rp.st_v = st_v; rp.st_w = st_w; rp.discard = h->l2_discard;
+    const bool in_half = pl.stream_half && i > 0, out_half = pl.stream_half && i + 1 < h->nblk;
+    if (in_half) rp.w_half_in = ws.wh;
+    if (out_half) rp.w_half_out = ws.wh;
     if (h->ln_mode == LN_RECURSIVE) { rp.g_a = d.lf_g; rp.b_a = d.lf_b; }        // model.py:347-348
     else if (h->ln_mode == LN_RESIDUAL) { rp.g_a = d.lm_g; rp.b_a = d.lm_b; }    // model.py:349-350
-    // gates + both residual GroupNorm steps in one cluster-resident kernel when an utterance fits a cluster
-    const bool fused = h->fused_resid && half_io && resid_fused_cluster_size(T) > 0;
-    prof_mark(h, fused ? SEPTFA_PROF_RESID : SEPTFA_PROF_GATE, st);
-    if (!(fused && launch_resid_fused(rp, gp, st))) {
+    if (const int clusters = pl.resid_clusters[in_half][out_half]) {
+      prof_mark(h, SEPTFA_PROF_RESID, st);
+      launch_resid_fused(rp, gp, clusters, st);
+    } else {
+      prof_mark(h, SEPTFA_PROF_GATE, st);
       launch_tf_gate(gp, st);
       prof_mark(h, SEPTFA_PROF_RESID, st);
       if (h->ln_mode != LN_NONE) launch_resid_stats(rp, st);
@@ -981,8 +1037,8 @@ int septfa_forward(septfa_handle* h, const float* x, int B, int64_t L, const sep
   // output layer: PReLU -> GroupNorm -> conv (model.py:322-325,357)
   prof_mark(h, SEPTFA_PROF_OUTCONV, st);
   launch_out_stats(ws.w, norm, h->out_a, M, T, ws.st_o, st);
-  OutConvParams oc{ws.w, norm, h->out_a, ws.st_o, h->out_g, h->out_be, M, T, B, h->out_bias, h->out_img, h->out_img_lo, h->out_wt, ws.logits};
-  if (tc_out) launch_tc_outconv(oc, st); else launch_ref_outconv(oc, st);
+  const OutConvParams oc{ws.w, norm, h->out_a, ws.st_o, h->out_g, h->out_be, M, T, B, h->out_bias, h->out_img, h->out_img_lo, h->out_wt, ws.logits};
+  if (pl.tc_out) launch_tc_outconv(oc, st); else launch_ref_outconv(oc, st);
 
   prof_mark(h, SEPTFA_PROF_VAD, st);
   const bool use_kw = kw != nullptr && c.final_vad;  // `if inference_kw and self.final_vad`, model.py:444
@@ -1002,28 +1058,12 @@ int septfa_forward(septfa_handle* h, const float* x, int B, int64_t L, const sep
     CUDA_TRY(h, cudaMemcpyAsync(out_vad, vsrc, (size_t)M * 2 * sizeof(float), cudaMemcpyDeviceToDevice, st));
   }
   prof_mark(h, SEPTFA_PROF_ISTFT, st);
-  // With any of the est / mask / logits exports, one kernel writes them and the waveform from one read of S and the logits;
-  // without them the register-prefetch kernel (3 CTAs per SM against 2) is slightly faster end to end (DESIGN.md section 3).
-  if (est_stft != nullptr || mask != nullptr || logits_out != nullptr)
+  if (pl.exports)
     launch_mask_istft_export(ws.S, ws.logits, gate, h->win_inv, h->twiddle, B, L, T, out_wav, reinterpret_cast<float2*>(est_stft),
                              mask, logits_out, st);
   else
     launch_mask_istft(ws.S, ws.logits, gate, h->win_inv, h->twiddle, B, L, T, out_wav, st);
   prof_mark(h, -1, st);
-#ifdef SEPTFA_TIMELINE
-  if (getenv("SEPTFA_FUSED_TL")) resid_fused_dump_timeline();
-  if (getenv("SEPTFA_GEMM_TL")) gemm_dump_cta_timeline((M + 127) / 128);
-  if (getenv("SEPTFA_TIMELINE") && septfa_dbg_ptr) {
-    std::vector<long long> hbuf(8 * 256);
-    cudaStreamSynchronize(st);
-    cudaMemcpy(hbuf.data(), septfa_dbg_ptr, hbuf.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-    fprintf(stderr, "TLG dconv:");
-    for (int i2 = 0; i2 < 64; ++i2) fprintf(stderr, " %lld", hbuf[i2] ? hbuf[i2] - hbuf[0] : -1);
-    fprintf(stderr, "\nTLG conv1:");
-    for (int i2 = 0; i2 < 64; ++i2) fprintf(stderr, " %lld", hbuf[1024 + i2] ? hbuf[1024 + i2] - hbuf[1024] : -1);
-    fprintf(stderr, "\n");
-  }
-#endif
   h->last_launches = ctx().launches;
   CUDA_TRY(h, cudaGetLastError());
   return 0;
