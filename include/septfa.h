@@ -267,8 +267,23 @@ int septfa_live_create_win(septfa_handle* h, int capacity, int window, int hop, 
  * input shifts by D. Per slot the session keeps 2 x (at most 2 width + orig) more floats; a new stream reads none of
  * them. At 16000 nothing is added and a push launches what it launched before. */
 int septfa_live_create_rate(septfa_handle* h, int capacity, int window, int hop, int rate, septfa_live** out);
+/* A session whose streams arrive at `rate` Hz and whose separated audio is returned at `out_rate` Hz (both in
+ * septfa_resample_geometry's range and independent of each other; septfa_live_create_rate is this with out_rate 16000).
+ * Let y_s be the 16 kHz stream of emitted channel s: the concatenated out of a 16 kHz-output session, after the PIT
+ * reordering. Push k returns out [n, 2, Ho], Ho = H out_rate / 16000 (septfa_live_output_hop):
+ *   out[s] = z_s[k Ho, (k + 1) Ho),   z_s = concat(D_out zeros, septfa_resample_to(y_s, out_rate)),
+ * bit for bit. D_out (0 at 16000) is the delay of the streaming output resampler in output samples: the outputs of a push
+ * before (k + 1) Ho - D_out need no 16 kHz sample after the hop (6 at 8 kHz, 18 at 48 kHz, 16 at 44.1 kHz; see
+ * septfa_resample_to_geometry). The hop must also be a multiple of the output rate's hop_multiple. perm and out_vad stay
+ * on the 16 kHz frame grid, unchanged. Per slot the session keeps 4 x (the output resampler's history) more floats
+ * (4 x 12 at 48 kHz, 4 x 24 at 8 kHz); a new stream reads none of them. At out_rate 16000 nothing is added and a push launches what it launched
+ * before; otherwise one more kernel runs after the emit. A refused create (bad rate, out rate, hop or geometry) returns
+ * SEPTFA_E_INVALID before anything is allocated and sets the launch count to 0. */
+int septfa_live_create_rates(septfa_handle* h, int capacity, int window, int hop, int rate, int out_rate, septfa_live** out);
 /* Hn, the native samples per push; *delay (nullable) receives D. */
 int septfa_live_input_hop(const septfa_live* lv, int* delay);
+/* Ho, the output samples per push and channel; *delay (nullable) receives D_out. */
+int septfa_live_output_hop(const septfa_live* lv, int* delay);
 void septfa_live_destroy(septfa_live* lv);
 /* F, the VAD frames per push; *first_frame (nullable) receives j0. */
 int septfa_live_vad_frames(const septfa_live* lv, int* first_frame);
@@ -304,6 +319,17 @@ int septfa_resample_geometry(int rate, int* delay, int* hop_multiple);
  * identity. The first call at a rate builds its bank, uploads it and waits for the upload; later calls at that rate are
  * stream-ordered and do not synchronise the host. */
 int septfa_resample(septfa_handle* h, const void* x, int x_fmt, int B, int64_t L, int rate, float* out, void* stream);
+
+/* Resampling the model's 16 kHz output to `rate`: torchaudio.functional.resample(y, 16000, rate) with the same defaults
+ * and the same bank construction with source and destination swapped (orig = 16000 / g, new = rate / g), within ~1e-6
+ * of float64 torchaudio. Accepted rates are those of septfa_resample, refused the same way.
+ * septfa_resample_to_geometry needs no handle and no device: *delay (nullable) receives D_out, the delay in output
+ * samples of a streaming output resampler (septfa_live_create_rates), and *hop_multiple (nullable) receives 16000 / g,
+ * which a live hop must be a multiple of. */
+int septfa_resample_to_geometry(int rate, int* delay, int* hop_multiple);
+/* y: device float32 [B, L] at 16 kHz; out: device float32 [B, ceil(rate L / 16000)]. Rate 16000 copies. The bank cache,
+ * the first-call upload and the stream ordering are those of septfa_resample. */
+int septfa_resample_to(septfa_handle* h, const float* y, int B, int64_t L, int rate, float* out, void* stream);
 
 /* calc_sisdr (model/combined_loss.py:16-56): SI-SDR in dB of `rows` pairs preds[rows, n] / target[rows, n] (device,
  * float32, contiguous) in one pass; out_db device [rows]; scratch: device, rows * 5 doubles; rows <= 65535. Runs on the

@@ -248,17 +248,20 @@ void launch_live_pit_emit(const int32_t* slots, int n, int32_t* hops_done, const
                           float* out_vad /*[n,2,F] or null*/, int32_t* perm /*[n,2]*/, LiveGeom g, cudaStream_t st);
 void launch_live_release(const int32_t* slots_host, int n, int32_t* hops_done, cudaStream_t st);
 
-// ---- resampling to 16 kHz (resample.cu)
+// ---- resampling between 16 kHz and another rate (resample.cu)
 constexpr int kResampleRate = 16000;
 constexpr int kResampleMinRate = 8000, kResampleMaxRate = 192000;
 constexpr int kResampleTile = 512;   // outputs per CTA
-// What a rate needs, computed on the host from the bank's effective support.
+// Direction of a bank: a rate's input to the model's 16 kHz, or the model's 16 kHz output to a rate.
+enum ResampleDir { kToModel = 0, kFromModel = 1 };
+// What a rate needs, computed on the host from the bank's effective support. "Source" is the side the bank reads
+// (the native rate for kToModel, 16 kHz for kFromModel), "destination" the side it writes.
 struct ResamplePlan {
-  int orig, nw;        // rate / g, 16000 / g with g = gcd(rate, 16000)
+  int orig, nw;        // source / g, destination / g with g = gcd(rate, 16000)
   int ntaps;           // taps stored per phase (the longest effective run; shorter ones are zero-padded)
-  int delay;           // D: 16 kHz samples a live stream lags by
-  int hist;            // native samples a live push reads from before its hop
-  int tile_span;       // native samples one tile of kResampleTile outputs reads (shared memory floats)
+  int delay;           // D: destination samples a live stream lags by
+  int hist;            // source samples a live push reads from before its hop
+  int tile_span;       // source samples one tile of kResampleTile outputs reads (shared memory floats)
 };
 struct ResampleBank {
   const float* taps;   // [ntaps][nw] fp32, tap i of phase p at i * nw + p
@@ -266,13 +269,16 @@ struct ResampleBank {
   int orig, nw, delay, hist, tile_span;
 };
 // false for a rate outside [8000, 192000]; taps / spans (nullable) receive the bank
-bool resample_plan(int rate, ResamplePlan* plan, std::vector<float>* taps, std::vector<int2>* spans);
-int64_t resample_out_len(int rate, int64_t L);
+bool resample_plan(int rate, ResampleDir dir, ResamplePlan* plan, std::vector<float>* taps, std::vector<int2>* spans);
+int64_t resample_out_len(const ResamplePlan& plan, int64_t L);   // ceil(nw L / orig)
 void launch_resample(const void* x, bool pcm16, int B, int64_t L, int64_t L16, float* out, const ResampleBank& bk,
                      cudaStream_t st);
 void launch_live_resample(const int32_t* slots, int n, const int32_t* hops_done, float* hist /*[cap][2][hist]*/,
                           const float* hops /*[n,Hn]*/, float* u /*[n,H]*/, const ResampleBank& bk, int H, int Hn,
                           cudaStream_t st);
+// after launch_live_pit_emit (hops_done already advanced): y [n,2,H] at 16 kHz -> out [n,2,Ho] at the output rate
+void launch_live_out_resample(const int32_t* slots, int n, const int32_t* hops_done, float* hist /*[cap][2][2][hist]*/,
+                              const float* y, float* out, const ResampleBank& bk, int H, int Ho, cudaStream_t st);
 
 // Per-handle launch state (septfa_handle owns one; every C-ABI entry binds it to the calling thread before launching).
 // Which kernel runs at each stage of a forward is decided by plan_forward (septfa_abi.cu); the launchers only launch.

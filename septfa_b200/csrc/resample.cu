@@ -1,7 +1,9 @@
-// Resampling to 16 kHz on the device: torchaudio.functional.resample(x, rate, 16000) with its defaults
-// (sinc_interp_hann, lowpass_filter_width = 6, rolloff = 0.99), as read_mixture applies it through transforms.Resample.
+// Resampling on the device: torchaudio.functional.resample(x, rate, 16000) with its defaults (sinc_interp_hann,
+// lowpass_filter_width = 6, rolloff = 0.99), as read_mixture applies it through transforms.Resample, and the output
+// direction resample(y, 16000, rate) with the same defaults. The two differ only in which side is the source: below,
+// "native" samples are the source's (the rate's for kToModel, 16 kHz for kFromModel).
 //
-// With g = gcd(rate, 16000), orig = rate / g and new = 16000 / g, output sample m = b new + p (phase p) is
+// With g = gcd(rate, 16000), orig = source / g and new = destination / g, output sample m = b new + p (phase p) is
 //   y[m] = sum_j x[b orig + j - width] k[p][j],   j = 0 .. 2 width + orig - 1,   x = 0 outside [0, L),
 // width = ceil(6 orig / base), base = 0.99 min(orig, new), and k[p][j] the Hann-windowed sinc at the scaled time
 // t = base ((j - width) / orig - p / new). The bank keeps only the taps with |t| < 6 (beyond that torchaudio clamps t to
@@ -29,7 +31,7 @@ int64_t ceil_div(int64_t a, int64_t b) { return -floor_div(-a, b); }
 
 }  // namespace
 
-bool resample_plan(int rate, ResamplePlan* pl, std::vector<float>* taps, std::vector<int2>* spans) {
+bool resample_plan(int rate, ResampleDir dir, ResamplePlan* pl, std::vector<float>* taps, std::vector<int2>* spans) {
   if (rate < kResampleMinRate || rate > kResampleMaxRate) return false;
   ResamplePlan P{};
   if (rate == kResampleRate) {
@@ -43,7 +45,8 @@ bool resample_plan(int rate, ResamplePlan* pl, std::vector<float>* taps, std::ve
     return true;
   }
   const int g = std::gcd(rate, kResampleRate);
-  const int64_t orig = rate / g, nw = kResampleRate / g, mn = std::min(orig, nw);
+  const int src = dir == kToModel ? rate : kResampleRate, dst = dir == kToModel ? kResampleRate : rate;
+  const int64_t orig = src / g, nw = dst / g, mn = std::min(orig, nw);
   const double base = (double)mn * 0.99;
   const int64_t width = (int64_t)std::ceil(6.0 * (double)orig / base);
   // |t| < 6  <=>  (p orig 99 mn - 600 orig new) < c (99 mn new) < (p orig 99 mn + 600 orig new), c = j - width
@@ -208,12 +211,49 @@ __global__ void __launch_bounds__(256) k_live_resample(const int32_t* __restrict
   }
 }
 
+// Live sessions at an output rate: grid row 2 e + c resamples channel c of entry e's emitted 16 kHz hop y[e][c] (stream
+// samples [k H, (k + 1) H) of the channel, in the emitted speaker order) into out[e][c] = z[k Ho, (k + 1) Ho) of
+// z = concat(D zeros, resample(y, 16000, rate)). It runs after k_live_pit_emit, which has advanced the slot's counter,
+// so this push is k = hops_done - 1. The history [slot][parity][channel][hist] holds the channel's last `hist` 16 kHz
+// samples, double-buffered by the parity of k as in k_live_resample; a stream at k = 0 reads none of it.
+__global__ void __launch_bounds__(256) k_live_out_resample(const int32_t* __restrict__ slots,
+                                                           const int32_t* __restrict__ hops_done, float* __restrict__ hist,
+                                                           const float* __restrict__ y, float* __restrict__ out,
+                                                           ResampleBank bk, int H, int Ho) {
+  extern __shared__ float xs[];
+  const int e = blockIdx.y >> 1, c = blockIdx.y & 1;
+  const int slot = slots[e];
+  const int k = hops_done[slot] - 1;
+  const int Hr = bk.hist;
+  const int t0 = blockIdx.x * kResampleTile;
+  const int nout = min(kResampleTile, Ho - t0);
+  const int64_t m0 = (int64_t)k * Ho + t0 - bk.delay;      // z index of the tile's first output (< 0: before D)
+  const int64_t kh = (int64_t)k * H;                         // stream index of the hop's first sample
+  const float* x = y + (size_t)blockIdx.y * H;
+  const float* hr = hist + (((size_t)slot * 2 + (k & 1)) * 2 + c) * Hr;
+  int p0;
+  const int64_t lo = tile_first_input(bk, m0, &p0);
+  const int n = tile_inputs(bk, p0, nout);
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    const int64_t gi = lo + i;
+    xs[i] = gi < 0 ? 0.f : gi >= kh ? x[gi - kh] : hr[gi - (kh - Hr)];
+  }
+  __syncthreads();
+  float* o = out + (size_t)blockIdx.y * Ho + t0;
+  for (int t = threadIdx.x; t < nout; t += blockDim.x) {
+    int p;
+    const int off = tile_offset(bk, p0, t, &p);
+    o[t] = m0 + t < 0 ? 0.f : resample_one(bk, p, xs + off);
+  }
+  if (blockIdx.x == 0) {
+    float* hw = hist + (((size_t)slot * 2 + ((k + 1) & 1)) * 2 + c) * Hr;
+    for (int i = threadIdx.x; i < Hr; i += blockDim.x) hw[i] = x[H - Hr + i];
+  }
+}
+
 }  // namespace
 
-int64_t resample_out_len(int rate, int64_t L) {   // ceil(16000 L / rate)
-  const int g = std::gcd(rate, kResampleRate);
-  return ceil_div(L * (kResampleRate / g), rate / g);
-}
+int64_t resample_out_len(const ResamplePlan& pl, int64_t L) { return ceil_div(L * pl.nw, pl.orig); }
 
 void launch_resample(const void* x, bool pcm16, int B, int64_t L, int64_t L16, float* out, const ResampleBank& bk,
                      cudaStream_t st) {
@@ -230,6 +270,13 @@ void launch_live_resample(const int32_t* slots, int n, const int32_t* hops_done,
                           const ResampleBank& bk, int H, int Hn, cudaStream_t st) {
   const dim3 grid((H + kResampleTile - 1) / kResampleTile, n);
   k_live_resample<<<grid, 256, (size_t)bk.tile_span * sizeof(float), st>>>(slots, hops_done, hist, hops, u, bk, H, Hn);
+  ++ctx().launches;
+}
+
+void launch_live_out_resample(const int32_t* slots, int n, const int32_t* hops_done, float* hist, const float* y, float* out,
+                              const ResampleBank& bk, int H, int Ho, cudaStream_t st) {
+  const dim3 grid((Ho + kResampleTile - 1) / kResampleTile, 2 * n);
+  k_live_out_resample<<<grid, 256, (size_t)bk.tile_span * sizeof(float), st>>>(slots, hops_done, hist, y, out, bk, H, Ho);
   ++ctx().launches;
 }
 

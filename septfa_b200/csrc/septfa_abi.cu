@@ -104,9 +104,9 @@ struct septfa_handle {
   int ev_used = 0;
   double prof_ms[SEPTFA_PROF_NCAT] = {0};
   int prof_launches[SEPTFA_PROF_NCAT] = {0};
-  // resampling filter banks by input rate, and their device memory: kept apart from `allocs`, which a weight commit
-  // frees, since live sessions and later calls hold the bank pointers until septfa_destroy
-  std::map<int, ResampleBank> banks;
+  // resampling filter banks by (direction, rate), and their device memory: kept apart from `allocs`, which a weight
+  // commit frees, since live sessions and later calls hold the bank pointers until septfa_destroy
+  std::map<std::pair<int, int>, ResampleBank> banks;
   std::vector<void*> bank_allocs;
 };
 
@@ -139,6 +139,10 @@ struct septfa_live {
   int in_hop = 0;                 // Hn = H rate / 16000 native samples per push
   ResampleBank bank{};            // the handle's bank for `rate`
   float* hist = nullptr;          // [capacity][2][bank.hist] native history, double-buffered by hop parity
+  int out_rate = kResampleRate;   // output rate; other than 16000: each emitted hop is resampled last
+  int out_hop = 0;                // Ho = H out_rate / 16000 output samples per push
+  ResampleBank out_bank{};        // the handle's 16000 -> out_rate bank
+  float* hist_out = nullptr;      // [capacity][2 parity][2 channels][out_bank.hist] 16 kHz history of the emitted channels
 };
 
 namespace {
@@ -163,10 +167,12 @@ int check_geometry(septfa_handle* h, int W, int H) {
   return 0;
 }
 
-// An input rate the resampler accepts: an integer in [8000, 192000] Hz.
-int check_rate(septfa_handle* h, int rate, ResamplePlan* plan) {
-  if (!resample_plan(rate, plan, nullptr, nullptr))
-    return fail(h, SEPTFA_E_INVALID, "rate " + std::to_string(rate) + ": the input rate must lie in 8000 .. 192000 Hz");
+// An input or output rate the resampler accepts: an integer in [8000, 192000] Hz.
+int check_rate(septfa_handle* h, int rate, ResampleDir dir, ResamplePlan* plan) {
+  if (!resample_plan(rate, dir, plan, nullptr, nullptr))
+    return fail(h, SEPTFA_E_INVALID, dir == kToModel
+                    ? "rate " + std::to_string(rate) + ": the input rate must lie in 8000 .. 192000 Hz"
+                    : "out rate " + std::to_string(rate) + ": the output rate must lie in 8000 .. 192000 Hz");
   return 0;
 }
 
@@ -261,15 +267,16 @@ int upload(septfa_handle* h, const std::vector<T>& src, const T** dst) {
   return 0;
 }
 
-// The handle's bank for `rate` (checked by the caller), built and uploaded at the first call for that rate. The upload
-// is waited for, so the bank can be used on any stream afterwards; later calls find it in the cache.
-int get_bank(septfa_handle* h, int rate, cudaStream_t st, ResampleBank* out) {
-  auto it = h->banks.find(rate);
+// The handle's bank for `rate` in direction `dir` (checked by the caller), built and uploaded at the first call for
+// them. The upload is waited for, so the bank can be used on any stream afterwards; later calls find it in the cache.
+int get_bank(septfa_handle* h, int rate, ResampleDir dir, cudaStream_t st, ResampleBank* out) {
+  const std::pair<int, int> key{(int)dir, rate};
+  auto it = h->banks.find(key);
   if (it != h->banks.end()) { *out = it->second; return 0; }
   ResamplePlan pl{};
   std::vector<float> taps;
   std::vector<int2> spans;
-  resample_plan(rate, &pl, &taps, &spans);
+  resample_plan(rate, dir, &pl, &taps, &spans);
   float* dt = nullptr;
   int2* ds = nullptr;
   CUDA_TRY(h, cudaMalloc(reinterpret_cast<void**>(&dt), taps.size() * sizeof(float)));
@@ -280,7 +287,7 @@ int get_bank(septfa_handle* h, int rate, cudaStream_t st, ResampleBank* out) {
   CUDA_TRY(h, cudaMemcpyAsync(ds, spans.data(), spans.size() * sizeof(int2), cudaMemcpyHostToDevice, st));
   CUDA_TRY(h, cudaStreamSynchronize(st));
   const ResampleBank bk{dt, ds, pl.orig, pl.nw, pl.delay, pl.hist, pl.tile_span};
-  h->banks[rate] = bk;
+  h->banks[key] = bk;
   *out = bk;
   return 0;
 }
@@ -1430,6 +1437,7 @@ struct LiveWorkspace {
   float* pred;      // [n, 2, W]
   float* vad;       // [n, 2, T(W)]
   float* u;         // [n, H] the resampled hops (sessions at a rate other than 16000)
+  float* y;         // [n, 2, H] the emitted 16 kHz hops (sessions at an output rate other than 16000)
   void* fws;        // the forward's workspace
   size_t fws_bytes;
   size_t total;
@@ -1445,6 +1453,10 @@ LiveWorkspace live_carve(const septfa_live* lv, uintptr_t base, int n) {
   w.pred = reinterpret_cast<float*>(base + off);    off += al((size_t)n * 2 * W * sizeof(float));
   w.vad = reinterpret_cast<float*>(base + off);     off += al((size_t)n * 2 * septfa_num_frames(W) * sizeof(float));
   if (lv->rate != kResampleRate) { w.u = reinterpret_cast<float*>(base + off); off += al((size_t)n * lv->g.hop * sizeof(float)); }
+  if (lv->out_rate != kResampleRate) {
+    w.y = reinterpret_cast<float*>(base + off);
+    off += al((size_t)n * 2 * lv->g.hop * sizeof(float));
+  }
   w.fws = reinterpret_cast<void*>(base + off);
   w.fws_bytes = septfa_workspace_bytes(lv->h, n, W);
   w.total = off + w.fws_bytes;
@@ -1484,12 +1496,16 @@ int septfa_live_create_win(septfa_handle* h, int capacity, int window, int hop, 
 }
 
 int septfa_live_create_rate(septfa_handle* h, int capacity, int window, int hop, int rate, septfa_live** out) {
+  return septfa_live_create_rates(h, capacity, window, hop, rate, kResampleRate, out);
+}
+
+int septfa_live_create_rates(septfa_handle* h, int capacity, int window, int hop, int rate, int out_rate, septfa_live** out) {
   if (!h || !out || capacity < 1 || capacity > 32767)
     return fail(h, SEPTFA_E_INVALID, "bad arguments (1 <= capacity <= 32767 slots per live session)");
   *out = nullptr;
   if (int rc = check_geometry(h, window, hop)) { h->last_launches = 0; return rc; }
   ResamplePlan pl{};
-  if (int rc = check_rate(h, rate, &pl)) { h->last_launches = 0; return rc; }
+  if (int rc = check_rate(h, rate, kToModel, &pl)) { h->last_launches = 0; return rc; }
   if (hop % pl.nw) {   // a push must carry a whole number of native samples
     h->last_launches = 0;
     return fail(h, SEPTFA_E_INVALID, "rate " + std::to_string(rate) + ", hop " + std::to_string(hop) +
@@ -1501,27 +1517,47 @@ int septfa_live_create_rate(septfa_handle* h, int capacity, int window, int hop,
     return fail(h, SEPTFA_E_INVALID, "rate " + std::to_string(rate) + ", hop " + std::to_string(hop) +
                                          ": the resampler's history exceeds one hop");
   }
+  ResamplePlan opl{};
+  if (int rc = check_rate(h, out_rate, kFromModel, &opl)) { h->last_launches = 0; return rc; }
+  if (hop % opl.orig) {   // a push must return a whole number of output samples
+    h->last_launches = 0;
+    return fail(h, SEPTFA_E_INVALID, "out rate " + std::to_string(out_rate) + ", hop " + std::to_string(hop) +
+                                         ": the hop must be a multiple of " + std::to_string(opl.orig) +
+                                         " samples at this output rate");
+  }
+  if (opl.hist > hop) {
+    h->last_launches = 0;
+    return fail(h, SEPTFA_E_INVALID, "out rate " + std::to_string(out_rate) + ", hop " + std::to_string(hop) +
+                                         ": the output resampler's history exceeds one hop");
+  }
   if (!h->committed) return fail(h, SEPTFA_E_STATE, "weights not committed");
   CUDA_TRY(h, cudaSetDevice(h->device));
-  ResampleBank bank{};
+  ResampleBank bank{}, out_bank{};
   if (rate != kResampleRate)
-    if (int rc = get_bank(h, rate, nullptr, &bank)) return rc;
+    if (int rc = get_bank(h, rate, kToModel, nullptr, &bank)) return rc;
+  if (out_rate != kResampleRate)
+    if (int rc = get_bank(h, out_rate, kFromModel, nullptr, &out_bank)) return rc;
   auto* lv = new septfa_live();
   lv->h = h;
   lv->capacity = capacity;
   lv->rate = rate;
   lv->in_hop = in_hop;
   lv->bank = bank;
+  lv->out_rate = out_rate;
+  lv->out_hop = (int)((int64_t)hop * opl.nw / opl.orig);
+  lv->out_bank = out_bank;
   const int first = (window - hop + 255) / 256;   // the first window frame whose centre 256 j lies in [W - H, W)
   lv->g = LiveGeom{window, hop, first, (window + 255) / 256 - first};
   const size_t ring_b = (size_t)(window - hop) * sizeof(float);
   const size_t hist_b = (size_t)capacity * 2 * std::max(bank.hist, 1) * sizeof(float);
+  const size_t hist_out_b = (size_t)capacity * 4 * std::max(out_bank.hist, 1) * sizeof(float);
   if (cudaMalloc(reinterpret_cast<void**>(&lv->hops_done), (size_t)capacity * sizeof(int32_t)) != cudaSuccess ||
       cudaMalloc(reinterpret_cast<void**>(&lv->in_ring), (size_t)capacity * ring_b) != cudaSuccess ||
       cudaMalloc(reinterpret_cast<void**>(&lv->tail_ring), (size_t)capacity * 2 * ring_b) != cudaSuccess ||
       (rate != kResampleRate && cudaMalloc(reinterpret_cast<void**>(&lv->hist), hist_b) != cudaSuccess) ||
+      (out_rate != kResampleRate && cudaMalloc(reinterpret_cast<void**>(&lv->hist_out), hist_out_b) != cudaSuccess) ||
       cudaMemset(lv->hops_done, 0, (size_t)capacity * sizeof(int32_t)) != cudaSuccess) {
-    cudaFree(lv->hops_done); cudaFree(lv->in_ring); cudaFree(lv->tail_ring); cudaFree(lv->hist);
+    cudaFree(lv->hops_done); cudaFree(lv->in_ring); cudaFree(lv->tail_ring); cudaFree(lv->hist); cudaFree(lv->hist_out);
     delete lv;
     return fail(h, SEPTFA_E_CUDA, "live session allocation failed");
   }
@@ -1532,7 +1568,7 @@ int septfa_live_create_rate(septfa_handle* h, int capacity, int window, int hop,
 void septfa_live_destroy(septfa_live* lv) {
   if (!lv) return;
   cudaSetDevice(lv->h->device);
-  cudaFree(lv->hops_done); cudaFree(lv->in_ring); cudaFree(lv->tail_ring); cudaFree(lv->hist);
+  cudaFree(lv->hops_done); cudaFree(lv->in_ring); cudaFree(lv->tail_ring); cudaFree(lv->hist); cudaFree(lv->hist_out);
   delete lv;
 }
 
@@ -1540,6 +1576,12 @@ int septfa_live_input_hop(const septfa_live* lv, int* delay) {
   if (!lv) return SEPTFA_E_INVALID;
   if (delay) *delay = lv->rate == kResampleRate ? 0 : lv->bank.delay;
   return lv->in_hop;
+}
+
+int septfa_live_output_hop(const septfa_live* lv, int* delay) {
+  if (!lv) return SEPTFA_E_INVALID;
+  if (delay) *delay = lv->out_rate == kResampleRate ? 0 : lv->out_bank.delay;
+  return lv->out_hop;
 }
 
 size_t septfa_live_workspace_bytes(const septfa_live* lv, int n) {
@@ -1593,8 +1635,11 @@ int septfa_live_push(septfa_live* lv, const int32_t* slots_host, int n, const fl
   const int launches = before + h->last_launches;
   bind_ctx(&h->lctx);
   ctx().launches = 0;
-  launch_live_pit_emit(ws.slots, n, lv->hops_done, ws.pred, ws.vad, (int)septfa_num_frames(lv->g.win), lv->tail_ring, out,
-                       out_vad, perm, lv->g, st);
+  const bool out_resample = lv->out_rate != kResampleRate;
+  launch_live_pit_emit(ws.slots, n, lv->hops_done, ws.pred, ws.vad, (int)septfa_num_frames(lv->g.win), lv->tail_ring,
+                       out_resample ? ws.y : out, out_vad, perm, lv->g, st);
+  if (out_resample)
+    launch_live_out_resample(ws.slots, n, lv->hops_done, lv->hist_out, ws.y, out, lv->out_bank, lv->g.hop, lv->out_hop, st);
   h->last_launches = launches + ctx().launches;
   CUDA_TRY(h, cudaGetLastError());
   return 0;
@@ -1634,35 +1679,61 @@ int septfa_minmax_normalize(septfa_handle* h, const float* x, int B, int64_t L, 
 
 int septfa_resample_geometry(int rate, int* delay, int* hop_multiple) {
   ResamplePlan pl{};
-  if (int rc = check_rate(nullptr, rate, &pl)) return rc;
+  if (int rc = check_rate(nullptr, rate, kToModel, &pl)) return rc;
   if (delay) *delay = pl.delay;
   if (hop_multiple) *hop_multiple = pl.nw;
   return 0;
 }
 
-int septfa_resample(septfa_handle* h, const void* x, int x_fmt, int B, int64_t L, int rate, float* out, void* stream) {
+int septfa_resample_to_geometry(int rate, int* delay, int* hop_multiple) {
+  ResamplePlan pl{};
+  if (int rc = check_rate(nullptr, rate, kFromModel, &pl)) return rc;
+  if (delay) *delay = pl.delay;
+  if (hop_multiple) *hop_multiple = pl.orig;   // the 16 kHz side is the source here
+  return 0;
+}
+
+}  // extern "C"
+
+namespace {
+
+// The batch resampler of both directions: x [B, L] (float32, or int16 PCM to 16 kHz) -> out [B, ceil(nw L / orig)].
+int resample_batch(septfa_handle* h, const void* x, int x_fmt, int B, int64_t L, int rate, ResampleDir dir, float* out,
+                   void* stream) {
   if (!h) return SEPTFA_E_INVALID;
   h->last_launches = 0;
   if (!x || !out || B < 1 || B > 65535 || L < 1) return fail(h, SEPTFA_E_INVALID, "bad arguments (1 <= B <= 65535, L >= 1)");
   if (x_fmt != SEPTFA_FMT_F32 && x_fmt != SEPTFA_FMT_PCM16)
     return fail(h, SEPTFA_E_INVALID, "x_fmt must be SEPTFA_FMT_F32 or SEPTFA_FMT_PCM16");
   ResamplePlan pl{};
-  if (int rc = check_rate(h, rate, &pl)) return rc;
+  if (int rc = check_rate(h, rate, dir, &pl)) return rc;
   CUDA_TRY(h, cudaSetDevice(h->device));
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const int64_t L16 = resample_out_len(rate, L);
+  const int64_t Lo = resample_out_len(pl, L);
   if (rate == kResampleRate && x_fmt == SEPTFA_FMT_F32) {
     CUDA_TRY(h, cudaMemcpyAsync(out, x, (size_t)B * L * sizeof(float), cudaMemcpyDeviceToDevice, st));
     return 0;
   }
   ResampleBank bk{};
-  if (int rc = get_bank(h, rate, st, &bk)) return rc;
+  if (int rc = get_bank(h, rate, dir, st, &bk)) return rc;
   bind_ctx(&h->lctx);
   ctx().launches = 0;
-  launch_resample(x, x_fmt == SEPTFA_FMT_PCM16, B, L, L16, out, bk, st);
+  launch_resample(x, x_fmt == SEPTFA_FMT_PCM16, B, L, Lo, out, bk, st);
   h->last_launches = ctx().launches;
   CUDA_TRY(h, cudaGetLastError());
   return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int septfa_resample(septfa_handle* h, const void* x, int x_fmt, int B, int64_t L, int rate, float* out, void* stream) {
+  return resample_batch(h, x, x_fmt, B, L, rate, kToModel, out, stream);
+}
+
+int septfa_resample_to(septfa_handle* h, const float* y, int B, int64_t L, int rate, float* out, void* stream) {
+  return resample_batch(h, y, SEPTFA_FMT_F32, B, L, rate, kFromModel, out, stream);
 }
 
 int septfa_sisdr(const float* preds, const float* target, int64_t rows, int64_t n, int zero_mean, float* out_db, double* scratch,

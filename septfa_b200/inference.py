@@ -133,7 +133,7 @@ def _first_channel(audio):
     return audio[0] if audio.shape[1] > audio.shape[0] else audio[:, 0]
 
 
-def separate_files(model, paths, save_dir, inference_kw=None, precision_save=32, device=0, batch=64):
+def separate_files(model, paths, save_dir, inference_kw=None, precision_save=32, device=0, batch=64, out_rate=None):
     """The file loop either side of the forward (SURVEY.md section 8(f) rank 1), batched: 16-bit wav files of EQUAL
     length and rate are grouped into batches. 16 kHz mono batches travel to the device as int16 PCM, are converted and
     min-max normalised there (only_inference.py:69,81, bit-identical to numpy), separated, and come back as float32 or -
@@ -143,16 +143,36 @@ def separate_files(model, paths, save_dir, inference_kw=None, precision_save=32,
     channel as read_mixture does. These files do not go through read_mixture, so its notes on stereo and resampled input
     are not printed for them. Other files (float wav, rates outside that range) take the single-file path of
     :func:`read_mixture`. Writes ``<stem>_Speaker_{0,1}.wav`` into ``save_dir`` (float32 wav, or 16-bit PCM for precision
-    16) and returns ``{path: vad [2, T]}``."""
+    16) and returns ``{path: vad [2, T]}``.
+
+    ``out_rate`` sets the rate of the written files. ``None`` writes the model's 16 kHz output. ``"input"`` writes each
+    file at its own rate with exactly its input length: ``SeparationModel.resample_to(out, rate)[..., :L]`` on the device
+    (the round trip is zero-phase, so the output stays aligned with the input); every file's rate must then lie in
+    8 .. 192 kHz, or ``ValueError`` is raised before any file is written. An integer in 8 .. 192 kHz writes every file at
+    that rate, ``ceil(out_rate L16 / 16000)`` samples for a 16 kHz output of L16 samples. When a group's output rate is not
+    16 kHz, 16 kHz mono files take the batched device path of the other rates."""
     from .lib import RESAMPLE_MAX_RATE, RESAMPLE_MIN_RATE
     from scipy.io.wavfile import read, write
+    if out_rate is not None and out_rate != "input" and (
+            isinstance(out_rate, bool) or not isinstance(out_rate, (int, np.integer))
+            or not RESAMPLE_MIN_RATE <= out_rate <= RESAMPLE_MAX_RATE):
+        raise ValueError(f"out_rate must be None, 'input' or an integer in {RESAMPLE_MIN_RATE} .. {RESAMPLE_MAX_RATE} Hz, "
+                         f"got {out_rate!r}")
+
+    def target(sr):   # the rate a file at sr is written at
+        return 16000 if out_rate is None else int(sr) if out_rate == "input" else int(out_rate)
+
     Path(save_dir).mkdir(parents=True, exist_ok=True)
     kw = copy.deepcopy(DEFAULT_INFERENCE_KW)
     kw.update(inference_kw or {})
     groups, rate_groups, singles = {}, {}, []
     for pth in paths:
         sr, audio = read(pth)
-        if sr == 16000 and audio.ndim == 1 and audio.dtype == np.int16 and len(audio) >= 257:
+        if out_rate == "input" and not RESAMPLE_MIN_RATE <= sr <= RESAMPLE_MAX_RATE:
+            raise ValueError(f"{pth}: out_rate='input' needs a rate in {RESAMPLE_MIN_RATE} .. {RESAMPLE_MAX_RATE} Hz, "
+                             f"the file is at {sr} Hz")
+        if (sr == 16000 and audio.ndim == 1 and audio.dtype == np.int16 and len(audio) >= 257
+                and target(sr) == 16000):
             groups.setdefault(len(audio), []).append((pth, audio))
         elif (RESAMPLE_MIN_RATE <= sr <= RESAMPLE_MAX_RATE and audio.dtype == np.int16 and audio.ndim in (1, 2)
               and audio.size):
@@ -160,19 +180,27 @@ def separate_files(model, paths, save_dir, inference_kw=None, precision_save=32,
             if -(-16000 * len(a) // sr) >= 257:
                 rate_groups.setdefault((sr, len(a)), []).append((pth, a))
             else:
-                singles.append(pth)
+                singles.append((pth, sr, len(a)))
         else:
-            singles.append(pth)
+            singles.append((pth, sr, len(audio) if audio.ndim == 1 or not audio.size else len(_first_channel(audio))))
     out_dtype = torch.float16 if precision_save == 16 else torch.float32
     vads = {}
 
-    def emit(pth, out, vad):
+    def to_rate(out, sr, n):
+        """The 16 kHz outputs [..., L16] (device) at the file's output rate; n: the file's input length."""
+        r = target(sr)
+        if r == 16000:
+            return out
+        out = model.resample_to(out, r)
+        return out[..., :n] if out_rate == "input" else out
+
+    def emit(pth, out, vad, rate=16000):
         stem = Path(pth).stem
         for s in range(2):
             a = out[s].float().numpy()
             if precision_save == 16:
                 a = np.clip(np.round(a * 32767.0), -32768, 32767).astype(np.int16)
-            write(os.path.join(save_dir, f"{stem}_Speaker_{s}.wav"), 16000, a)
+            write(os.path.join(save_dir, f"{stem}_Speaker_{s}.wav"), rate, a)
         vads[pth] = vad
 
     for _, items in sorted(groups.items()):
@@ -182,21 +210,25 @@ def separate_files(model, paths, save_dir, inference_kw=None, precision_save=32,
             for i, (pth, _) in enumerate(ch):
                 emit(pth, out[i], vad[i].clone() if torch.is_tensor(vad) else None)
     dev = torch.device("cuda", device)
-    for (sr, _), items in sorted(rate_groups.items()):
+    for (sr, n), items in sorted(rate_groups.items()):
         for i in range(0, len(items), batch):
             ch = items[i:i + batch]
             x = torch.from_numpy(np.stack([a for _, a in ch])).to(dev)
             with torch.no_grad():
                 out, vad, _ = model(model.minmax_normalize(model.resample(x, sr)), kw)
-            out = out.to(out_dtype).cpu()
+            out = to_rate(out, sr, n).to(out_dtype).cpu()
             vad = vad.cpu() if torch.is_tensor(vad) else None
             for j, (pth, _) in enumerate(ch):
-                emit(pth, out[j], vad[j].clone() if vad is not None else None)
-    for pth in singles:
+                emit(pth, out[j], vad[j].clone() if vad is not None else None, target(sr))
+    for pth, sr, n in singles:
         x = read_mixture(pth).to(torch.device("cuda", device))
         with torch.no_grad():
             out, vad, _ = model(x, kw)
-        emit(pth, out[0].cpu(), vad[0].cpu() if torch.is_tensor(vad) else None)
+        if RESAMPLE_MIN_RATE <= sr <= RESAMPLE_MAX_RATE:
+            out, rate = to_rate(out, sr, n), target(sr)
+        else:
+            rate = 16000
+        emit(pth, out[0].cpu(), vad[0].cpu() if torch.is_tensor(vad) else None, rate)
     return vads
 
 

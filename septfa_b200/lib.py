@@ -101,7 +101,9 @@ _PROTOS = {
     "septfa_live_create": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]),
     "septfa_live_create_win": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "septfa_live_create_rate": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
+    "septfa_live_create_rates": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "septfa_live_input_hop": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
+    "septfa_live_output_hop": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "septfa_live_destroy": (None, [C.c_void_p]),
     "septfa_live_vad_frames": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "septfa_live_workspace_bytes": (C.c_size_t, [C.c_void_p, C.c_int]),
@@ -110,6 +112,8 @@ _PROTOS = {
                                    C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "septfa_resample_geometry": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "septfa_resample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_void_p, C.c_void_p]),
+    "septfa_resample_to_geometry": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "septfa_resample_to": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int, C.c_void_p, C.c_void_p]),
     "septfa_minmax_normalize": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "septfa_sisdr": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "septfa_pit_l1": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p,
@@ -149,7 +153,7 @@ def num_frames(L):
     return 1 + int(L) // 256
 
 
-RESAMPLE_MIN_RATE, RESAMPLE_MAX_RATE = 8000, 192000   # input rates septfa_resample accepts
+RESAMPLE_MIN_RATE, RESAMPLE_MAX_RATE = 8000, 192000   # rates septfa_resample and septfa_resample_to accept
 
 
 def resample_geometry(rate):
@@ -159,5 +163,16 @@ def resample_geometry(rate):
     lib = load()
     d, m = C.c_int(), C.c_int()
     rc = lib.septfa_resample_geometry(int(rate), C.byref(d), C.byref(m))
+    check(None, rc)
+    return d.value, m.value
+
+
+def resample_to_geometry(rate):
+    """``(delay, hop_multiple)`` of the output ``rate`` from septfa_resample_to_geometry (no device needed): the delay
+    D_out in output samples of a streaming 16000 -> ``rate`` resampler, and the number a live hop (16 kHz samples) must
+    be a multiple of for that output rate. Raises SeptfaError for a rate the library refuses."""
+    lib = load()
+    d, m = C.c_int(), C.c_int()
+    rc = lib.septfa_resample_to_geometry(int(rate), C.byref(d), C.byref(m))
     check(None, rc)
     return d.value, m.value

@@ -14,6 +14,11 @@ A session at another input ``rate`` (8 .. 192 kHz) takes ``input_hop = hop * rat
 resamples each stream on the device (``septfa_live_create_rate``), carrying the resampler's history from push to push.
 It then serves the 16 kHz stream ``u = concat(delay zeros, resample(x))``: the output lags the input by ``delay``
 samples (6 .. 12, see ``septfa_resample_geometry``) on top of the hop.
+
+A session with another ``out_rate`` (8 .. 192 kHz, independent of ``rate``) returns ``output_hop = hop * out_rate /
+16000`` samples per channel and push: the 16 kHz output resampled on the device (``septfa_live_create_rates``), i.e.
+``concat(out_delay zeros, model.resample_to(y))`` of the 16 kHz output stream y, cut into hops. ``out_delay`` (0 at
+16000, 18 at 48 kHz, see ``septfa_resample_to_geometry``) is in output samples. VAD and permutations are unchanged.
 """
 from __future__ import annotations
 
@@ -32,19 +37,20 @@ FRAMES_PER_HOP = 63      # VAD frames per push at the default geometry
 MAX_WINDOW = 160000      # 10 s
 
 
-def check_geometry(window, hop, rate=RATE):
+def check_geometry(window, hop, rate=RATE, out_rate=RATE):
     """``(window, hop)`` as ints if the library accepts them: 256 <= hop, 2 hop <= window <= 160000, both multiples of 16
-    samples (1 ms); ``rate`` an integer in 8000 .. 192000 Hz, and the hop a multiple of ``16000 / gcd(rate, 16000)`` so
-    that a push carries a whole number of native samples (160 at 44.1 kHz, any hop at 48 kHz). ``ValueError``
-    otherwise."""
-    if not all(isinstance(v, (int, np.integer)) and not isinstance(v, bool) for v in (window, hop, rate)):
-        raise ValueError(f"window, hop and rate are integers, got {window!r}, {hop!r}, {rate!r}")
-    window, hop, rate = int(window), int(hop), int(rate)
-    if not _lib.RESAMPLE_MIN_RATE <= rate <= _lib.RESAMPLE_MAX_RATE:
-        raise ValueError(f"rate = {rate}: must lie in {_lib.RESAMPLE_MIN_RATE} .. {_lib.RESAMPLE_MAX_RATE} Hz")
-    step = RATE // math.gcd(rate, RATE)
-    if hop % step:
-        raise ValueError(f"rate = {rate}, hop = {hop}: the hop must be a multiple of {step} samples at this rate")
+    samples (1 ms); ``rate`` and ``out_rate`` integers in 8000 .. 192000 Hz, and the hop a multiple of
+    ``16000 / gcd(r, 16000)`` for both, so that a push carries a whole number of native samples and returns a whole
+    number of output samples (160 at 44.1 kHz, any hop at 48 kHz). ``ValueError`` otherwise."""
+    if not all(isinstance(v, (int, np.integer)) and not isinstance(v, bool) for v in (window, hop, rate, out_rate)):
+        raise ValueError(f"window, hop, rate and out_rate are integers, got {window!r}, {hop!r}, {rate!r}, {out_rate!r}")
+    window, hop, rate, out_rate = int(window), int(hop), int(rate), int(out_rate)
+    for name, r in (("rate", rate), ("out_rate", out_rate)):
+        if not _lib.RESAMPLE_MIN_RATE <= r <= _lib.RESAMPLE_MAX_RATE:
+            raise ValueError(f"{name} = {r}: must lie in {_lib.RESAMPLE_MIN_RATE} .. {_lib.RESAMPLE_MAX_RATE} Hz")
+        step = RATE // math.gcd(r, RATE)
+        if hop % step:
+            raise ValueError(f"{name} = {r}, hop = {hop}: the hop must be a multiple of {step} samples at this rate")
     if hop < 256:
         raise ValueError(f"hop = {hop}: must be >= 256 samples")
     if window < 2 * hop:
@@ -83,16 +89,19 @@ class LiveSession:
     speakers in the emitted order; it is None for a model without a VAD head or with ``vad=False``. ``release(slots)``
     ends the streams in those slots: the next push into one starts a new stream. ``inference_kw`` is the forward's
     (gating, smoothed VAD), fixed for the session. At a rate other than 16000 the outputs are those of a 16 kHz session
-    fed ``concat(delay zeros, model.resample(stream))``; ``delay`` is 0 at 16000.
+    fed ``concat(delay zeros, model.resample(stream))``; ``delay`` is 0 at 16000. At an ``out_rate`` other than 16000,
+    ``out`` is ``[n, 2, output_hop]``: hop k of ``concat(out_delay zeros, model.resample_to(y, out_rate))`` per channel,
+    y the channel's 16 kHz output stream; ``out_delay`` is 0 at 16000.
     """
 
-    def __init__(self, model, capacity, inference_kw=None, device=None, window=WINDOW, hop=HOP, rate=RATE):
+    def __init__(self, model, capacity, inference_kw=None, device=None, window=WINDOW, hop=HOP, rate=RATE,
+                 out_rate=RATE):
         self.model = model
         self.capacity = int(capacity)
         if not 1 <= self.capacity <= 32767:
             raise ValueError("capacity must lie in 1 .. 32767")
-        self.window, self.hop = check_geometry(window, hop, rate)
-        self.rate = int(rate)
+        self.window, self.hop = check_geometry(window, hop, rate, out_rate)
+        self.rate, self.out_rate = int(rate), int(out_rate)
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         if self.device.type != "cuda":
             raise RuntimeError("septfa_b200.LiveSession runs on CUDA only (no CPU fallback)")
@@ -100,11 +109,13 @@ class LiveSession:
         self._lv = C.c_void_p()
         with torch.cuda.device(self.device):
             self._h = model._handle(self.device)
-            _lib.check(self._h.ptr, self._h.lib.septfa_live_create_rate(self._h.ptr, self.capacity, self.window, self.hop,
-                                                                        self.rate, C.byref(self._lv)))
+            _lib.check(self._h.ptr, self._h.lib.septfa_live_create_rates(self._h.ptr, self.capacity, self.window, self.hop,
+                                                                         self.rate, self.out_rate, C.byref(self._lv)))
             delay = C.c_int()
             self.input_hop = self._h.lib.septfa_live_input_hop(self._lv, C.byref(delay))
             self.delay = delay.value
+            self.output_hop = self._h.lib.septfa_live_output_hop(self._lv, C.byref(delay))
+            self.out_delay = delay.value
             j0 = C.c_int()
             self.frames_per_hop = self._h.lib.septfa_live_vad_frames(self._lv, C.byref(j0))
             self.first_frame = j0.value
@@ -127,7 +138,7 @@ class LiveSession:
         hops = hops.contiguous()
         with torch.cuda.device(self.device):
             h = self.model._handle(self.device)
-            out = torch.empty((n, 2, self.hop), dtype=torch.float32, device=self.device)
+            out = torch.empty((n, 2, self.output_hop), dtype=torch.float32, device=self.device)
             v = torch.empty((n, 2, self.frames_per_hop), dtype=torch.float32, device=self.device) \
                 if (vad and self.model.final_vad) else None
             perm = torch.empty((n, 2), dtype=torch.int32, device=self.device)

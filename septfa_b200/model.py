@@ -292,6 +292,28 @@ class SeparationModel(nn.Module):
             self.last_launch_count = h.lib.septfa_last_launch_count(h.ptr)
         return out
 
+    def resample_to(self, y: torch.Tensor, rate):
+        """torchaudio.functional.resample(y, 16000, rate) on the device (septfa_resample_to): the model's 16 kHz output
+        back at ``rate``. ``y [..., L]`` is a CUDA float32 tensor whose leading dimensions are resampled as rows (a
+        forward's ``[B, 2, L]`` goes in directly); returns float32 ``[..., ceil(rate L / 16000)]``. ``rate``: an integer
+        in 8000 .. 192000 Hz; 16000 returns the input values."""
+        assert y.ndim >= 1 and y.is_cuda and y.dtype == torch.float32
+        if isinstance(rate, bool) or int(rate) != rate:
+            raise ValueError(f"rate must be an integer number of Hz, got {rate!r}")
+        rate = int(rate)
+        y = y.contiguous()
+        L = y.shape[-1]
+        rows = y.numel() // L if L else 0
+        out = torch.empty((*y.shape[:-1], max(-(-rate * L // 16000), 0) if rate > 0 else 0), dtype=torch.float32,
+                          device=y.device)
+        with torch.cuda.device(y.device):
+            h = self._handle(y.device)
+            rc = h.lib.septfa_resample_to(h.ptr, C.c_void_p(y.data_ptr()), rows, L, rate, C.c_void_p(out.data_ptr()),
+                                          C.c_void_p(torch.cuda.current_stream(y.device).cuda_stream))
+            _lib.check(h.ptr, rc)
+            self.last_launch_count = h.lib.septfa_last_launch_count(h.ptr)
+        return out
+
     def forward_host_submit(self, x_host: torch.Tensor, inference_kw={}, device=0, slot=0, out=None, vad=None,
                             out_dtype=torch.float32):
         """Asynchronous half of :meth:`forward_host` (septfa_forward_host_submit_fmt): enqueue copy-in, forward and

@@ -15,7 +15,12 @@ every hop carries hop * R / 16000 native samples of seeded mixtures, which the s
 the same window / forward / emit. The three legs alternate step by step; the record adds the rate leg's push times and
 its overhead over the 16 kHz push.
 
-    python tools/live_bench.py [--capacity 1024 --steps 60 --warmup 10c --window 48000 --hop 16000 --rate 48000] --out FILE.json
+With --out-rate R (other than 16000) one more leg pushes the same schedule into a session at --rate in and R out
+(septfa_live_create_rates), alternated step by step with the same session at 16 kHz out (the rate leg, or the 16 kHz
+push when --rate is 16000); the record adds its push times and its overhead over that session.
+
+    python tools/live_bench.py [--capacity 1024 --steps 60 --warmup 10c --window 48000 --hop 16000 --rate 48000
+                                --out-rate 48000] --out FILE.json
 """
 import argparse
 import contextlib
@@ -57,6 +62,7 @@ def main():
     ap.add_argument("--window", type=int, default=48000, help="window W in samples")
     ap.add_argument("--hop", type=int, default=16000, help="hop H in samples")
     ap.add_argument("--rate", type=int, default=16000, help="input rate of a third leg (16000: no third leg)")
+    ap.add_argument("--out-rate", type=int, default=16000, help="output rate of one more leg (16000: no such leg)")
     ap.add_argument("--out", default=None, help="write the JSON record here too")
     a = ap.parse_args()
     W, H = a.window, a.hop
@@ -103,6 +109,14 @@ def main():
         ws_r = torch.empty(lib.septfa_live_workspace_bytes(lv_r, n), dtype=torch.uint8, device=dev)
         mixes_r = torch.from_numpy(synth.make_mixtures(32, max_hops * Hn, 4322)).to(dev).view(32, max_hops, Hn)
 
+    lv_o = C.c_void_p()
+    if a.out_rate != FS:
+        _lib.check(h.ptr, lib.septfa_live_create_rates(h.ptr, n, W, H, a.rate, a.out_rate, C.byref(lv_o)))
+        out_delay = C.c_int()
+        Ho = lib.septfa_live_output_hop(lv_o, C.byref(out_delay))
+        ws_o = torch.empty(lib.septfa_live_workspace_bytes(lv_o, n), dtype=torch.uint8, device=dev)
+        out_o = torch.empty((n, 2, Ho), device=dev)
+
     st = C.c_void_p()
     _lib.check(h.ptr, lib.septfa_online_create_win(h.ptr, n, W, H, C.byref(st)))
     ws_on = torch.empty(lib.septfa_online_workspace_bytes(st), dtype=torch.uint8, device=dev)
@@ -121,13 +135,15 @@ def main():
 
     push_ms, step_ms, ns, restarts, launches = [], [], [], [], 0
     push_r_ms, launches_r = [], 0
+    push_o_ms, launches_o = [], 0
     for t in range(a.warmup + a.steps):
         length = np.round((3 + (np.arange(n) + gen) % 8) * c).astype(np.int64)
         ended = np.nonzero((k == length) & (start <= t))[0].astype(np.int32)
         if ended.size:
             _lib.check(h.ptr, lib.septfa_live_release(lv, ended.ctypes.data_as(C.c_void_p), ended.size, stream))
-            if lv_r:
-                _lib.check(h.ptr, lib.septfa_live_release(lv_r, ended.ctypes.data_as(C.c_void_p), ended.size, stream))
+            for other in (lv_r, lv_o):
+                if other:
+                    _lib.check(h.ptr, lib.septfa_live_release(other, ended.ctypes.data_as(C.c_void_p), ended.size, stream))
             gen[ended] += 1
             k[ended] = 0
         slots = np.nonzero(start <= t)[0].astype(np.int32)
@@ -158,6 +174,16 @@ def main():
                                                        stream))
             tr = timed(push_r)
             launches_r = lib.septfa_last_launch_count(h.ptr)
+        if lv_o:
+            hops_o = hops_r if lv_r else hops
+
+            def push_o():
+                _lib.check(h.ptr, lib.septfa_live_push(lv_o, sl, slots.size, C.c_void_p(hops_o.data_ptr()), C.byref(ikw),
+                                                       C.c_void_p(out_o.data_ptr()), C.c_void_p(vad.data_ptr()),
+                                                       C.c_void_p(perm.data_ptr()), C.c_void_p(ws_o.data_ptr()), ws_o.numel(),
+                                                       stream))
+            to = timed(push_o)
+            launches_o = lib.septfa_last_launch_count(h.ptr)
         ts = timed(step)
         k[slots] += 1
         if t >= a.warmup:
@@ -165,12 +191,15 @@ def main():
             push_ms.append(tp)
             if lv_r:
                 push_r_ms.append(tr)
+            if lv_o:
+                push_o_ms.append(to)
             step_ms.append(ts)
             ns.append(int(slots.size))
             restarts.append(int(ended.size))
     lib.septfa_live_destroy(lv)
-    if lv_r:
-        lib.septfa_live_destroy(lv_r)
+    for other in (lv_r, lv_o):
+        if other:
+            lib.septfa_live_destroy(other)
     lib.septfa_online_destroy(st)
 
     p50p, p50s, p99p = pct(push_ms, 0.5), pct(step_ms, 0.5), pct(push_ms, 0.99)
@@ -192,6 +221,14 @@ def main():
                            "push": {"p50_ms": p50r, "p99_ms": p99r, "min_ms": min(push_r_ms), "launches": launches_r},
                            "overhead_p50_ms": p50r - p50p, "overhead_p99_ms": p99r - p99p,
                            "realtime_streams_at_push_p99": n * (H / FS) / (p99r / 1000.0)}
+    if lv_o:
+        p50o, p99o = pct(push_o_ms, 0.5), pct(push_o_ms, 0.99)
+        b50, b99 = (p50r, p99r) if lv_r else (p50p, p99p)
+        rec["out_rate_leg"] = {"rate": a.rate, "out_rate": a.out_rate, "output_hop": Ho, "out_delay_samples": out_delay.value,
+                               "push": {"p50_ms": p50o, "p99_ms": p99o, "min_ms": min(push_o_ms), "launches": launches_o},
+                               "same_session_16k_out": {"p50_ms": b50, "p99_ms": b99},
+                               "overhead_p50_ms": p50o - b50, "overhead_p99_ms": p99o - b99,
+                               "realtime_streams_at_push_p99": n * (H / FS) / (p99o / 1000.0)}
     line = json.dumps(rec)
     print(line, flush=True)
     if a.out:

@@ -9,7 +9,10 @@ data-sheet rate (7.7 TB/s) and of the rate this project measured for a plain cop
 HBM is the bound that applies; the record says so when the time is within 2x of the HBM floor, and "not at the HBM
 bound" otherwise.
 
-    python tools/resample_bench.py [--iters 50 --warmup 5] --out FILE.json
+With --to it times the output direction instead (septfa_resample_to): the separated output of a 256 x 4 s forward,
+[512, 64000] float32 at 16 kHz, to 44.1 and 48 kHz (131 MB in, 360 / 393 MB out), with the same fields.
+
+    python tools/resample_bench.py [--iters 50 --warmup 5] [--to] --out FILE.json
 """
 import argparse
 import contextlib
@@ -45,6 +48,7 @@ def main():
     ap.add_argument("--seconds", type=float, default=4.0)
     ap.add_argument("--iters", type=int, default=50)
     ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--to", action="store_true", help="time septfa_resample_to on the output of a --batch x --seconds forward")
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
     if not torch.cuda.is_available():
@@ -56,7 +60,36 @@ def main():
     h = model._handle(dev)
     stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
     cases = []
-    for rate in (44100, 48000):
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+
+    def timed(call):
+        for _ in range(a.warmup):
+            call()
+        torch.cuda.synchronize()
+        e0.record()
+        for _ in range(a.iters):
+            call()
+        e1.record()
+        torch.cuda.synchronize()
+        return e0.elapsed_time(e1) / a.iters / 1e3
+
+    for rate in (44100, 48000) if a.to else ():
+        rows, L16 = 2 * a.batch, int(round(a.seconds * 16000))   # both speakers of every mixture
+        L = -(-rate * L16 // 16000)
+        y = torch.rand((rows, L16), generator=torch.Generator(device=dev).manual_seed(rate), device=dev) * 1.8 - 0.9
+        out = torch.empty((rows, L), device=dev)
+        t = timed(lambda: _lib.check(h.ptr, h.lib.septfa_resample_to(h.ptr, C.c_void_p(y.data_ptr()), rows, L16, rate,
+                                                                     C.c_void_p(out.data_ptr()), stream)))
+        nbytes = y.numel() * 4 + out.numel() * 4
+        floor = nbytes / HBM_DATASHEET
+        gcd = math.gcd(rate, 16000)
+        cases.append({"rate": rate, "direction": "16000 -> rate", "rows": rows, "L16": L16, "L": L,
+                      "orig": 16000 // gcd, "new": rate // gcd, "delay": _lib.resample_to_geometry(rate)[0],
+                      "kernel_us": t * 1e6, "bytes": nbytes, "achieved_TBps": nbytes / t / 1e12,
+                      "of_hbm_datasheet": floor / t, "of_hbm_measured": (nbytes / HBM_MEASURED) / t,
+                      "hbm_floor_measured_us": nbytes / HBM_MEASURED * 1e6,
+                      "bound": "HBM" if t < 2 * floor else "not at the HBM bound"})
+    for rate in () if a.to else (44100, 48000):
         L = int(round(a.seconds * rate))
         L16 = -(-16000 * L // rate)
         g = torch.Generator(device=dev).manual_seed(rate)
@@ -68,16 +101,7 @@ def main():
             def call():
                 _lib.check(h.ptr, h.lib.septfa_resample(h.ptr, C.c_void_p(x.data_ptr()), x_fmt, a.batch, L, rate,
                                                          C.c_void_p(out.data_ptr()), stream))
-            for _ in range(a.warmup):
-                call()
-            torch.cuda.synchronize()
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            for _ in range(a.iters):
-                call()
-            e1.record()
-            torch.cuda.synchronize()
-            t = e0.elapsed_time(e1) / a.iters / 1e3
+            t = timed(call)
             nbytes = x.numel() * x.element_size() + out.numel() * 4
             floor = nbytes / HBM_DATASHEET
             gcd = math.gcd(rate, 16000)
@@ -86,7 +110,7 @@ def main():
                           "kernel_us": t * 1e6, "bytes": nbytes, "achieved_TBps": nbytes / t / 1e12,
                           "of_hbm_datasheet": floor / t, "of_hbm_measured": (nbytes / HBM_MEASURED) / t,
                           "bound": "HBM" if t < 2 * floor else "not at the HBM bound"})
-    rec = {"bench": "septfa_resample", **gpu_info(0),
+    rec = {"bench": "septfa_resample_to" if a.to else "septfa_resample", **gpu_info(0),
            "timing": f"CUDA events over {a.iters} back-to-back calls after {a.warmup} warm-up calls",
            "hbm_datasheet_TBps": HBM_DATASHEET / 1e12, "hbm_measured_copy_TBps": HBM_MEASURED / 1e12, "cases": cases}
     print(json.dumps(rec), flush=True)
